@@ -61,7 +61,34 @@ def parse_args():
                     help="reads per sample file of the host command-line leg (0 = skip)")
     ap.add_argument("--ref-reads", type=int, default=int(os.environ.get("TB_BENCH_REF_READS", 50_000)),
                     help="--impl reference: reads per sample file written as SAM for the reference binary")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step returned (collapse groups, tiecov runs / junctions) as "
+                         "DIR/<name>.npy: a fixed, seeded sample of rows, at most 64 MB in all, so that two builds can be compared")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_ROWS = 1 << 18   # rows sampled per output table: the three tables stay under 64 MB as float64
+
+
+def dump_table(out_dir, prefix, count, columns):
+    """Writes a fixed, seeded sample of `count` rows of `columns` [(name, array, np dtype)] as out_dir/<prefix>_<name>.npy, the
+    sampled row numbers as <prefix>_row.npy and the row count as <prefix>_count.npy. The sample depends on `count` alone, so
+    two builds that return the same rows write the same files. Integer columns go out as float64 (exact below 2^53)."""
+    os.makedirs(out_dir, exist_ok=True)
+    rows = np.arange(count, dtype=np.int64) if count <= DUMP_ROWS else \
+        np.sort(np.random.default_rng(12345).choice(count, DUMP_ROWS, replace=False))
+    np.save(os.path.join(out_dir, f"{prefix}_count.npy"), np.asarray([count], np.float64))
+    np.save(os.path.join(out_dir, f"{prefix}_row.npy"), rows.astype(np.float64))
+    for name, a, dt in columns:
+        if hasattr(a, "cpu"):   # device tensor: gather the sample there, copy only it
+            import torch
+            a = a[torch.from_numpy(rows).to(a.device)].cpu().numpy()
+        else:
+            a = np.asarray(a)[rows]
+        np.save(os.path.join(out_dir, f"{prefix}_{name}.npy"), a.astype(dt))
 
 
 class ClockSampler(threading.Thread):
@@ -464,6 +491,12 @@ def run_tiecov_leg(args, rank, world, local, dev, stream, peak, barrier, dist):
     barrier()
     launches = cctx.launch_count() - l0
     cov_ms = c0.elapsed_time(c1) / args.steps
+    if args.dump_outputs and rank == 0:   # the rows of the whole stream, gathered on rank 0 by the last step
+        f64, f32 = np.float64, np.float32
+        dump_table(args.dump_outputs, "tiecov_runs", loc["total_runs"],
+                   list(zip(("tid", "start", "end", "value"), loc["gathered_runs"](), (f64, f64, f64, f64))))
+        dump_table(args.dump_outputs, "tiecov_juncs", loc["total_juncs"],
+                   list(zip(("tid", "start", "end", "strand", "value"), loc["gathered_juncs"](), (f64, f64, f64, f32, f64))))
     tot = torch.tensor([float(mbases), float(loc["n_runs"]), float(loc["n_juncs"]), float(loc["stats"]["halo_bytes_sent"]),
                         float(loc["stats"]["lead_sent"]), float(g["gather_bytes"]) if rank else 0.0], device=dev, dtype=torch.float64)
     tmax = torch.tensor([cov_ms, ms[3]], device=dev, dtype=torch.float64)
@@ -512,7 +545,7 @@ def run_tiecov_leg(args, rank, world, local, dev, stream, peak, barrier, dist):
         del out_local, all_out
         torch.cuda.empty_cache()
         r2 = cctx.coverage_stream(host, args.cov_window, hout)
-        es = max(1, min(args.steps, 3))
+        es = args.steps
         g0, g1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         barrier()
         with torch.cuda.stream(stream):
@@ -689,6 +722,13 @@ def main():
     launches = ctx.launch_count() - l0
     ms_total = e0.elapsed_time(e1)
     G = res["n_groups"]
+    if args.dump_outputs and rank == 0:   # the groups of the last step (of every rank when the cohort is sharded)
+        # no name may keep `out` alive here: the e2e leg below frees it to make room for its own buffers
+        g_all = res["groups_all_ranks"] if strong else G
+        dump_table(args.dump_outputs, "collapse", g_all, [(kk, (gat if strong else out)[kk][:g_all], np.float32 if kk == "yc" else np.float64)
+                                                          for kk in ("rep_index", "yc", "yx", "yd")])
+        if not strong:
+            np.save(os.path.join(args.dump_outputs, "collapse_n_kept.npy"), np.asarray([res["n_kept"]], np.float64))
     if world > 1:
         t = torch.tensor([ms_total], device=dev, dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -799,7 +839,7 @@ def main():
             del cols, out, res, wire_cols
             torch.cuda.empty_cache()
             hout = {kk: v.numpy().view(np.uint32) if kk in ("rep_index", "yx") else v.numpy() for kk, v in hout_t.items()}
-            es = max(1, min(args.steps, 3))
+            es = args.steps
             ctx.collapse_window(host, run_off, pos_range=pr, out=hout)  # warm the staging buffers
             barrier()
             t0 = time.perf_counter()

@@ -75,6 +75,129 @@ def assert_collapse_equal(got, exp, what=""):
     assert len(bad) == 0, f"{what}: yc differs at {bad[:5]} got {got['yc'][bad[:5]]} exp {exp['yc'][bad[:5]]}"
 
 
+_AUX_INT = {"c": "<b", "C": "<B", "s": "<h", "S": "<H", "i": "<i", "I": "<I"}
+_SEQ2 = [a + b for a in "=ACMGRSVTWYHKDBN" for b in "=ACMGRSVTWYHKDBN"]   # one byte of BAM SEQ = two bases
+_QUAL33 = bytes((q + 33) & 0xFF for q in range(256))
+
+
+def bam_sam_text(path):
+    """A BAM file as the SAM text htslib prints for it (`htsfile -c`): header, then one line per record. BGZF is a series of
+    gzip members, so the gzip module reads it; the record layout is the one of the SAM/BAM specification, section 4.2."""
+    import gzip
+    import struct
+    b = gzip.open(path, "rb").read()
+    assert b[:4] == b"BAM\1", f"{path}: not a BAM file"
+    l_text = struct.unpack_from("<i", b, 4)[0]
+    lines = [b[8:8 + l_text].rstrip(b"\0").decode().rstrip("\n")]
+    o = 8 + l_text
+    n_ref = struct.unpack_from("<i", b, o)[0]
+    o += 4
+    names = []
+    for _ in range(n_ref):
+        ln = struct.unpack_from("<i", b, o)[0]
+        names.append(b[o + 4:o + 3 + ln].decode())
+        o += 8 + ln
+    while o < len(b):
+        bs, tid, pos, l_qn, mapq, _bin, n_cig, flag, l_seq, ntid, npos, tlen = struct.unpack_from("<iiiBBHHHiiii", b, o)
+        end, o = o + 4 + bs, o + 36
+        qname = b[o:o + l_qn - 1].decode()
+        o += l_qn
+        cig = sam.cigar_str(struct.unpack_from(f"<{n_cig}I", b, o))
+        o += 4 * n_cig
+        seq = "".join([_SEQ2[x] for x in b[o:o + (l_seq + 1) // 2]])[:l_seq] if l_seq else "*"
+        o += (l_seq + 1) // 2
+        qual = "*" if (l_seq == 0 or b[o] == 0xFF) else b[o:o + l_seq].translate(_QUAL33).decode("latin-1")
+        o += l_seq
+        f = [qname, str(flag), names[tid] if tid >= 0 else "*", str(pos + 1), str(mapq), cig,
+             "*" if ntid < 0 else ("=" if ntid == tid else names[ntid]), str(npos + 1), str(tlen), seq, qual]
+        while o < end:
+            tag, t = b[o:o + 2].decode(), chr(b[o + 2])
+            o += 3
+            if t == "A":
+                f.append(f"{tag}:A:{chr(b[o])}"); o += 1
+            elif t in _AUX_INT:
+                v = struct.unpack_from(_AUX_INT[t], b, o)[0]
+                f.append(f"{tag}:i:{v}"); o += struct.calcsize(_AUX_INT[t])
+            elif t == "f":
+                f.append(f"{tag}:f:{struct.unpack_from('<f', b, o)[0]:g}"); o += 4
+            elif t == "d":
+                f.append(f"{tag}:d:{struct.unpack_from('<d', b, o)[0]:g}"); o += 8
+            elif t in "ZH":
+                z = b.index(b"\0", o)
+                f.append(f"{tag}:{t}:{b[o:z].decode()}"); o = z + 1
+            elif t == "B":
+                st, cnt = chr(b[o]), struct.unpack_from("<i", b, o + 1)[0]
+                fmt = "<f" if st == "f" else _AUX_INT[st]
+                w = struct.calcsize(fmt)
+                vals = [struct.unpack_from(fmt, b, o + 5 + w * k)[0] for k in range(cnt)]
+                f.append(f"{tag}:B:{st}" + "".join(f",{v:g}" if st == "f" else f",{v}" for v in vals)); o += 5 + w * cnt
+            else:
+                raise ValueError(f"{path}: aux type {t!r}")
+        lines.append("\t".join(f))
+    return "\n".join(lines) + "\n"
+
+
+# The reference's own test data (test/t1/t1s[0-9].bam, test/t2/t2s[0-9].bam) and what the compiled, unmodified reference
+# makes of it: md5 of the record text of `tiebrush -o o.bam <files>` (`htsfile -c o.bam | grep -v '^@' | md5sum`), of the
+# bedGraph and junction BED of `tiecov -c -j` on the t1+t2 output, and the counts of its summary line.
+FIXTURES = os.path.join(GOLDEN, "fixtures")
+REF_MD5 = {"t1": "db674977026be7f2832fe9869ed40376", "t2": "27f7b93a789a9cddb06dca63449d32af", "t12": "50320443e9d380da6bc6c46b1fa90d85",
+           "cov": "8d1b0c70113a233095742cec61bb8129", "junc": "61427ff301f9ea70d48d5fbff20db7e2"}
+REF_COUNTS = {"t1": (416922, 3479), "t2": (242910, 8179), "t12": (659832, 9491)}   # (input records kept, records written)
+
+
+def fixture_inputs(which):
+    """The sample BAMs of the fixture sets `which` (e.g. ["t1", "t2"]): (per-file columns, SAM header lines, input line by
+    line hash). Decoded once per process."""
+    key = ("fixtures",) + tuple(which)
+    if key not in _cache:
+        paths = [os.path.join(FIXTURES, t, f"{t}s{i}.bam") for t in which for i in range(10)]
+        for p in paths:
+            if p not in _cache:
+                _cache[p] = bam_sam_text(p)
+        texts = [_cache[p] for p in paths]
+        header = [ln for ln in texts[0].split("\n") if ln.startswith("@")]
+        ids = sam.parse_sam("\n".join(header))[1]
+        files = [sam.to_columns(sam.parse_sam(t, ids)[0]) for t in texts]
+        lines = {}
+        for t in texts:
+            for ln in t.split("\n"):
+                if ln and ln[0] != "@":
+                    lines.setdefault(sam.line_hash(ln.split("\t")), ln)
+        _cache[key] = (files, header, lines)
+    return _cache[key]
+
+
+def collapsed_records(got, lines):
+    """The SAM record lines tiebrush writes for the groups of run_collapse(): the representative's line with YC (float),
+    YX and, when non-zero, YD appended, as htslib prints them."""
+    return ["\t".join([lines[int(lh)], f"YC:f:{float(yc):g}", f"YX:i:{int(yx)}"] + ([f"YD:i:{int(yd)}"] if int(yd) > 0 else []))
+            for lh, yc, yx, yd in zip(got["lhash"], got["yc"], got["yx"], got["yd"])]
+
+
+def md5_text(lines):
+    import hashlib
+    return hashlib.md5(("\n".join(lines) + "\n").encode()).hexdigest()
+
+
+def coverage_input(header, records):
+    """tiecov's view of a collapsed file: columns of its mapped records, weight YC (1 where the tag is absent)."""
+    R, ids = sam.parse_sam("\n".join(header + records) + "\n")
+    cols = sam.to_columns(R)
+    keep = np.nonzero((cols["flag"] & 4) == 0)[0]
+    sub = sam.take(cols, keep)
+    sub["yc"] = np.where(cols["has_yc"], cols["yc_in"], np.float32(1)).astype(np.float32)[keep]
+    return sub, {v: k for k, v in ids.items()}
+
+
+def coverage_files(got, names):
+    """The bytes of tiecov's -c bedGraph and -j junction BED for coverage rows `got` (the formats of tiecov.cpp)."""
+    bg = "track type=bedGraph\n" + "".join(f"{names[int(t)]}\t{int(s)}\t{int(e)}\t{float(v):.3f}\n" for t, s, e, v in zip(*got["runs"]))
+    bed = "track name=junctions\n" + "".join(f"{names[int(t)]}\t{int(s) - 1}\t{int(e)}\tJUNC{i + 1:08d}\t{float(v):.3f}\t{chr(int(c))}\n"
+                                             for i, (t, s, e, c, v) in enumerate(zip(*got["juncs"])))
+    return bg, bed
+
+
 def load_coverage_case(case):
     z = _npz("coverage.npz")
     pre = f"{case}/"

@@ -33,6 +33,25 @@ def test_collapse_merged(case):
     H.assert_collapse_equal(H.run_collapse(gpu_collapse, files, opts, fm), exp, case)
 
 
+@pytest.mark.parametrize("name,which", [("t1", ["t1"]), ("t2", ["t2"]), ("t12", ["t1", "t2"])])
+def test_fixture_bams_against_reference_md5(name, which):
+    """The reference's own sample BAMs (tests/golden/fixtures) through the GPU collapse: the records tiebrush would write
+    from its groups have the md5 of the compiled reference's output; for t1+t2 also the bytes of tiecov -c -j on them."""
+    from tiebrush_b200 import api
+    files, header, lines = H.fixture_inputs(which)
+    got = H.run_collapse(gpu_collapse, files, {})
+    assert (got["n_kept"], len(got["lhash"])) == H.REF_COUNTS[name]
+    records = H.collapsed_records(got, lines)
+    assert H.md5_text(records) == H.REF_MD5[name]
+    if name == "t12":
+        import hashlib
+        cols, names = H.coverage_input(header, records)
+        with api.Context(device=0) as ctx:
+            bg, bed = H.coverage_files(ctx.coverage_window(cols), names)
+        assert hashlib.md5(bg.encode()).hexdigest() == H.REF_MD5["cov"]
+        assert hashlib.md5(bed.encode()).hexdigest() == H.REF_MD5["junc"]
+
+
 @pytest.fixture(params=[1, 2])
 def tile_gen(request, monkeypatch):
     """Both tile kernels: generation 1 (default) and generation 2 (slices staged by cp.async.bulk + mbarrier, opt-in)."""

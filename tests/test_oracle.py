@@ -1,7 +1,7 @@
 """CPU tests: the C restatement (oracle/tb_oracle.c) against golden vectors produced by the UNMODIFIED
 compiled reference (tests/golden/make_golden.py). This is what pins the oracle."""
+import hashlib
 import os
-import subprocess
 
 import numpy as np
 import pytest
@@ -43,37 +43,20 @@ def test_coverage_rejects_unsupported_ops():
         oracle.coverage(cols)
 
 
-REF_TEST = "/root/reference/test"
-
-
-@pytest.mark.skipif(not (os.path.isdir(REF_TEST) and os.path.exists(os.path.join(oracle.REF_DIR, "tiebrush"))),
-                    reason="needs /root/reference and oracle/_ref (build container only)")
-def test_full_fixtures_against_live_reference(tmp_path):
-    """All 20 sample BAMs of the reference's own tests: oracle vs the compiled reference run live."""
-    paths = [f"{REF_TEST}/t1/t1s{i}.bam" for i in range(10)] + [f"{REF_TEST}/t2/t2s{i}.bam" for i in range(10)]
-    out = str(tmp_path / "o.bam")
-    r = subprocess.run([os.path.join(oracle.REF_DIR, "tiebrush"), "-o", out] + paths, check=True, capture_output=True, text=True)
-    assert r.stderr.startswith("659832 input records written as 9491")
-    hts = os.path.join(oracle.REF_DIR, "htsfile")
-    exp_txt = subprocess.run([hts, "-c", out], check=True, capture_output=True, text=True).stdout
-    expR, ids = sam.parse_sam(exp_txt)
-    expc = sam.to_columns(expR)
-    files = [sam.to_columns(sam.parse_sam(subprocess.run([hts, "-c", p], check=True, capture_output=True, text=True).stdout, ids)[0])
-             for p in paths]
+def test_full_fixtures_against_reference_md5():
+    """All 20 sample BAMs of the reference's own tests (tests/golden/fixtures): the oracle's collapsed records, and its
+    tiecov -c -j files on them, byte for byte what the compiled reference wrote (md5 of its outputs, helpers.REF_MD5)."""
+    files, header, lines = H.fixture_inputs(["t1", "t2"])
     got = H.run_collapse(oracle.collapse, files, {})
-    H.assert_collapse_equal(got, dict(tid=expc["tid"], lhash=expc["lhash"], yc=expc["yc_in"], yx=expc["yx_in"],
-                                      yd=expc["yd_in"], n_kept=659832), "t1+t2")
-    # tiecov on the collapsed output
-    subprocess.run([os.path.join(oracle.REF_DIR, "tiecov"), "-c", str(tmp_path / "k.cov"), "-j", str(tmp_path / "k.j"), out], check=True)
-    import sys
-    sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
-    import make_golden as mg
-    runs = mg.parse_bedgraph(open(tmp_path / "k.cov.bedgraph").read(), ids)
-    juncs = mg.parse_bed(open(tmp_path / "k.j.bed").read(), ids)
-    assert len(runs[0]) == 9043 and len(juncs[0]) == 18
-    cols = dict(expc)
-    cols["yc"] = np.where(expc["has_yc"], expc["yc_in"], np.float32(1)).astype(np.float32)
-    H.assert_coverage_equal(oracle.coverage(cols), runs, juncs, "t1+t2 tiecov")
+    assert (got["n_kept"], len(got["lhash"])) == H.REF_COUNTS["t12"]
+    records = H.collapsed_records(got, lines)
+    assert H.md5_text(records) == H.REF_MD5["t12"]
+    cols, names = H.coverage_input(header, records)
+    cov = oracle.coverage(cols)
+    assert len(cov["runs"][0]) == 9043 and len(cov["juncs"][0]) == 18
+    bg, bed = H.coverage_files(cov, names)
+    assert hashlib.md5(bg.encode()).hexdigest() == H.REF_MD5["cov"]
+    assert hashlib.md5(bed.encode()).hexdigest() == H.REF_MD5["junc"]
 
 
 def test_sample_heatmap_oracle_matches_the_reference_binary(tmp_path):
