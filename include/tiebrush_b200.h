@@ -125,6 +125,24 @@ typedef struct {
   int32_t   on_device;  /* 0: host arrays; 1: device arrays                                      */
 } tb_groups_out;
 
+/* The YD segment lists (GSegList, tiebrush.cpp:122-253) carried from one collapse window to the next, so that a window
+ * may begin at any start position instead of only at a coverage gap. One list per chain: chain c = side * n_samples +
+ * sample, side 0 = the '+' list (fsegs), side 1 = the '-' list (rsegs). All arrays are HOST memory.
+ * Canonical form, with B = pos_hi + 1 (the smallest 1-based start the next window can hold): the nodes [s, e] (1-based,
+ * inclusive, in list order) with e >= B that cover at least two positions or are the list's last node. Nothing else of
+ * the lists can change a later distance (merge order, groups, filters and the processRead cache never cross a cut
+ * between two start positions). */
+typedef struct {
+  int32_t  tid;        /* reference id of the lists; -1 = none                                    */
+  int32_t  pos_hi;     /* pos_hi of the window that produced them                                 */
+  int32_t  n_chains;   /* 2 * n_samples, chain c = side * n_samples + sample                      */
+  int64_t  capacity;   /* entries seg_start / seg_end can hold (carry_out)                        */
+  int64_t  n_segs;     /* segments; on a capacity error: the number needed                        */
+  int64_t* chain_off;  /* [n_chains + 1] segments of chain c: [chain_off[c], chain_off[c+1])      */
+  int32_t* seg_start;  /* 1-based, inclusive; canonical form above                                */
+  int32_t* seg_end;
+} tb_yd_carry;
+
 /* One coverage window: records of a coordinate-sorted (collapsed or raw) stream, unmapped records
  * already dropped (tiecov.cpp:436-438). A window must hold whole bundles (tiecov.cpp:443). */
 typedef struct {
@@ -183,6 +201,23 @@ int   tb_sync(tb_ctx*);
 /* ---- tiebrush: merge + collapse of one window --------------------------------------------- */
 /* replaces TInputFiles::next + passes_options + addPData + flushPData for the window */
 int tb_collapse_window(tb_ctx*, const tb_soa_in* in, tb_groups_out* out);
+
+/* tb_collapse_window for a window cut at any start position: the YD lists start from carry_in (NULL = empty, as in
+ * tb_collapse_window) and the lists this window leaves behind are written to carry_out (NULL = not wanted) in the
+ * canonical form for B = in->pos_hi + 1. Feeding each window the carry_out of the window before it gives the groups of
+ * one call over their union. Rules (a violation returns non-zero with a message and writes nothing):
+ *   - carry_in->tid != in->tid: the lists start empty (the reference resets them at a tid change, tiebrush.cpp:586-589);
+ *   - on the same tid, in->pos_lo < carry_in->pos_hi is an error (the windows would overlap);
+ *   - n_chains != 2 * in->n_files is an error (carry_in and carry_out alike);
+ *   - chain_off must be non-decreasing from 0 to n_segs; within a chain the segments must have end >= start, be sorted
+ *     and must not overlap (touching segments are allowed);
+ *   - carry_out->capacity too small: error, and carry_out->n_segs is set to the number of segments needed (the groups
+ *     of `out` are valid; call again with a larger carry_out).
+ * A window with no records or no groups returns carry_in re-filtered against its own pos_hi. Host or device columns
+ * and the compact / packed wire formats work as in tb_collapse_window. Both YD implementations seed the lists and
+ * extract them on the device; without a carry nothing is added to tb_collapse_window's work. */
+int tb_collapse_window_carry(tb_ctx*, const tb_soa_in* in, const tb_yd_carry* carry_in, tb_groups_out* out,
+                             tb_yd_carry* carry_out);
 
 /* ---- tiecov: coverage, junctions, bedgraph runs of one window ------------------------------ */
 /* replaces addCov + flushCoverage + addJunction + flushJuncs; runs / juncs may each be NULL

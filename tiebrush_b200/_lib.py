@@ -11,7 +11,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libtiebrush_b200.so")
 
 SYMBOLS = ["tb_create", "tb_destroy", "tb_last_error", "tb_set_stream", "tb_get_stream", "tb_sync",
-           "tb_collapse_window", "tc_coverage_window", "tc_sample_window", "tb_launch_count", "tb_set_profiling",
+           "tb_collapse_window", "tb_collapse_window_carry", "tc_coverage_window", "tc_sample_window", "tb_launch_count", "tb_set_profiling",
            "tb_last_kernel_ms", "tb_version", "tb_last_path", "tb_last_yd_path", "tb_last_heavy_slots", "tb_last_tile_gen", "tb_last_tile_stat",
            "tc_coverage_stream", "tb_comm_unique_id", "tb_comm_init", "tb_comm_destroy", "tb_comm_rank", "tb_comm_world",
            "tc_shard_coverage", "tc_shard_coverage_gather", "tc_shard_gather", "tc_shard_stat", "tc_stream_windows", "tc_last_exact"]
@@ -32,6 +32,11 @@ class SoaIn(C.Structure):
 class GroupsOut(C.Structure):
     _fields_ = [("capacity", C.c_int64), ("n_groups", C.c_int64), ("n_kept", C.c_int64), ("rep_index", C.c_void_p),
                 ("yc", C.c_void_p), ("yx", C.c_void_p), ("yd", C.c_void_p), ("on_device", C.c_int32)]
+
+
+class YdCarry(C.Structure):
+    _fields_ = [("tid", C.c_int32), ("pos_hi", C.c_int32), ("n_chains", C.c_int32), ("capacity", C.c_int64), ("n_segs", C.c_int64),
+                ("chain_off", C.c_void_p), ("seg_start", C.c_void_p), ("seg_end", C.c_void_p)]
 
 
 class CovIn(C.Structure):
@@ -72,6 +77,7 @@ def load():
     lib.tb_get_stream.restype = C.c_void_p
     lib.tb_sync.argtypes = [C.c_void_p]
     lib.tb_collapse_window.argtypes = [C.c_void_p, C.POINTER(SoaIn), C.POINTER(GroupsOut)]
+    lib.tb_collapse_window_carry.argtypes = [C.c_void_p, C.POINTER(SoaIn), C.POINTER(YdCarry), C.POINTER(GroupsOut), C.POINTER(YdCarry)]
     lib.tc_coverage_window.argtypes = [C.c_void_p, C.POINTER(CovIn), C.POINTER(RunsOut), C.POINTER(JuncsOut)]
     lib.tc_sample_window.argtypes = [C.c_void_p, C.POINTER(CovIn), C.c_void_p, C.POINTER(RunsOut)]
     lib.tb_launch_count.argtypes = [C.c_void_p]

@@ -123,6 +123,13 @@ def pack_fixed_columns(cols, run_off, max_dict=255):
     return dict(pos_d8=d8, pos_ext=ext, meta8=m8, meta_ext=tup[~hit].astype(np.uint64), meta_dict=dict_sorted.astype(np.uint64))
 
 
+def empty_yd_carry(n_samples):
+    """The YD carry a stream starts from: no lists (what tb_collapse_window assumes). Pass it, or the yd_carry of the
+    previous window's result, as collapse_window(..., yd_carry=)."""
+    return dict(tid=-1, pos_hi=0, chain_off=np.zeros(2 * n_samples + 1, np.int64), seg_start=np.zeros(0, np.int32),
+                seg_end=np.zeros(0, np.int32))
+
+
 class Context:
     def __init__(self, device=0, n_samples=1, mode=0, flag_mask=0, max_nh=NO_MAX_NH, min_qual=-1, keep_bits=0, collapse_same=0):
         self.lib = _lib.load()
@@ -179,8 +186,12 @@ class Context:
         return int(self.lib.tb_last_path(self.h))
 
     # ------------------------------------------------------------------------------------------
-    def collapse_window(self, cols, run_off, tid=0, file_merged=None, pos_range=None, out=None):
-        """One window of tiebrush. Returns dict(rep_index, yc, yx, yd, n_kept, n_groups)."""
+    def collapse_window(self, cols, run_off, tid=0, file_merged=None, pos_range=None, out=None, yd_carry=None):
+        """One window of tiebrush. Returns dict(rep_index, yc, yx, yd, n_kept, n_groups).
+        yd_carry: the YD lists carried in from the window before (empty_yd_carry(k), or the "yd_carry" of the previous
+        result); the window may then start at any start position, not only at a coverage gap. The result then holds the
+        lists this window leaves behind under "yd_carry" (dict of numpy arrays: tid, pos_hi, chain_off, seg_start,
+        seg_end; chain c = side * k + sample). Without it the call is tb_collapse_window, unchanged."""
         first = cols["pos"] if cols.get("pos") is not None else cols["pos_d8"]
         dev = _is_torch(first)
         n = int(first.shape[0])
@@ -238,11 +249,31 @@ class Context:
                 out = dict(rep_index=np.empty(cap, np.uint32), yc=np.empty(cap, np.float32), yx=np.empty(cap, np.uint32), yd=np.empty(cap, np.int32))
         o = _lib.GroupsOut(int(out["rep_index"].shape[0]), 0, 0, _ptr(out["rep_index"]), _ptr(out["yc"]), _ptr(out["yx"]), _ptr(out["yd"]),
                            1 if _is_torch(out["rep_index"]) else 0)
-        rc = self.lib.tb_collapse_window(self.h, C.byref(sin), C.byref(o))
-        if rc != 0:
-            raise TieBrushError(self._err())
+        if yd_carry is None:
+            rc = self.lib.tb_collapse_window(self.h, C.byref(sin), C.byref(o))
+            if rc != 0:
+                raise TieBrushError(self._err())
+        else:
+            ci = {key: _host(yd_carry[key], dt) for key, dt in (("chain_off", np.int64), ("seg_start", np.int32), ("seg_end", np.int32))}
+            cin = _lib.YdCarry(int(yd_carry["tid"]), int(yd_carry["pos_hi"]), len(ci["chain_off"]) - 1, len(ci["seg_start"]),
+                               int(ci["chain_off"][-1]), _ptr(ci["chain_off"]), _ptr(ci["seg_start"]), _ptr(ci["seg_end"]))
+            cap = max(4096, 2 * len(ci["seg_start"]) + 8 * k)
+            while True:   # a carry_out too small for the lists: the call says how many there are
+                co = dict(chain_off=np.zeros(2 * k + 1, np.int64), seg_start=np.zeros(cap, np.int32), seg_end=np.zeros(cap, np.int32))
+                cout = _lib.YdCarry(0, 0, 2 * k, cap, 0, _ptr(co["chain_off"]), _ptr(co["seg_start"]), _ptr(co["seg_end"]))
+                rc = self.lib.tb_collapse_window_carry(self.h, C.byref(sin), C.byref(cin), C.byref(o), C.byref(cout))
+                if rc == 0 or int(cout.n_segs) <= cap:
+                    break
+                cap = int(cout.n_segs)
+            if rc != 0:
+                raise TieBrushError(self._err())
+            m = int(cout.n_segs)
+            carry = dict(tid=int(cout.tid), pos_hi=int(cout.pos_hi), chain_off=co["chain_off"], seg_start=co["seg_start"][:m], seg_end=co["seg_end"][:m])
         g = int(o.n_groups)
-        return dict(rep_index=out["rep_index"][:g], yc=out["yc"][:g], yx=out["yx"][:g], yd=out["yd"][:g], n_kept=int(o.n_kept), n_groups=g)
+        res = dict(rep_index=out["rep_index"][:g], yc=out["yc"][:g], yx=out["yx"][:g], yd=out["yd"][:g], n_kept=int(o.n_kept), n_groups=g)
+        if yd_carry is not None:
+            res["yd_carry"] = carry
+        return res
 
     # ------------------------------------------------------------------------------------------
     def sample_window(self, cols, cap_rows=None):

@@ -13,7 +13,15 @@ void tb_ctx::set_error(const char* fmt, ...) {
 }
 
 int tc_coverage_impl(tb_ctx* ctx, const tc_soa_in* in, tc_runs_out* runs, tc_juncs_out* juncs, const int32_t* yx, CovExt* ext);
-int tb_collapse_impl(tb_ctx* ctx, const tb_soa_in* in, tb_groups_out* out);
+int tb_collapse_impl(tb_ctx* ctx, const tb_soa_in* in, tb_groups_out* out, const tb_yd_carry* cin, tb_yd_carry* cout);
+
+// the rules of tb_collapse_window_carry (include/tiebrush_b200.h) for one carry; nonzero = error set
+static int yd_carry_invalid(tb_ctx* ctx, const tb_soa_in* in, const tb_yd_carry* c, const char* what) {
+  const int nchains = 2 * in->n_files;
+  if (c->n_chains != nchains) { ctx->set_error("tb_collapse_window_carry: %s has n_chains %d, the window has %d (2 * n_files)", what, c->n_chains, nchains); return 1; }
+  if (!c->chain_off) { ctx->set_error("tb_collapse_window_carry: %s has no chain_off", what); return 1; }
+  return 0;
+}
 
 static void global_error(const char* fmt, ...) {
   char buf[1024];
@@ -98,7 +106,40 @@ int tb_collapse_window(tb_ctx* ctx, const tb_soa_in* in, tb_groups_out* out) {
   if (!ctx) return 1;
   if (!in || !out) { ctx->set_error("tb_collapse_window: null argument"); return 1; }
   ctx->err.clear();
-  return tb_collapse_impl(ctx, in, out);
+  return tb_collapse_impl(ctx, in, out, nullptr, nullptr);
+}
+
+int tb_collapse_window_carry(tb_ctx* ctx, const tb_soa_in* in, const tb_yd_carry* cin, tb_groups_out* out, tb_yd_carry* cout) {
+  if (!ctx) return 1;
+  if (!in || !out) { ctx->set_error("tb_collapse_window_carry: null argument"); return 1; }
+  ctx->err.clear();
+  if (in->n_files < 1) { ctx->set_error("tb_collapse_window_carry: n_files=%d", in->n_files); return 1; }
+  if ((cin || cout) && in->pos_hi <= in->pos_lo) { ctx->set_error("tb_collapse_window_carry: pos_lo/pos_hi not set"); return 1; }
+  if (cin) {
+    if (yd_carry_invalid(ctx, in, cin, "carry_in")) return 1;
+    const int nchains = 2 * in->n_files;
+    if (cin->n_segs < 0 || cin->chain_off[0] != 0 || cin->chain_off[nchains] != cin->n_segs) {
+      ctx->set_error("tb_collapse_window_carry: carry_in chain_off must run from 0 to n_segs (%lld)", (long long)cin->n_segs); return 1;
+    }
+    if (cin->n_segs > 0 && (!cin->seg_start || !cin->seg_end)) { ctx->set_error("tb_collapse_window_carry: carry_in has no segments"); return 1; }
+    for (int c = 0; c < nchains; ++c) {
+      if (cin->chain_off[c + 1] < cin->chain_off[c]) { ctx->set_error("tb_collapse_window_carry: carry_in chain_off decreases at chain %d", c); return 1; }
+      for (int64_t q = cin->chain_off[c]; q < cin->chain_off[c + 1]; ++q) {
+        if (cin->seg_end[q] < cin->seg_start[q]) { ctx->set_error("tb_collapse_window_carry: carry_in segment %lld has end < start", (long long)q); return 1; }
+        if (q > cin->chain_off[c] && cin->seg_start[q] <= cin->seg_end[q - 1]) {
+          ctx->set_error("tb_collapse_window_carry: carry_in segments %lld and %lld of chain %d overlap or are unsorted", (long long)q - 1, (long long)q, c); return 1;
+        }
+      }
+    }
+    if (cin->tid == in->tid && in->pos_lo < cin->pos_hi) {
+      ctx->set_error("tb_collapse_window_carry: pos_lo %d lies before the carried lists' pos_hi %d", in->pos_lo, cin->pos_hi); return 1;
+    }
+  }
+  if (cout) {
+    if (yd_carry_invalid(ctx, in, cout, "carry_out")) return 1;
+    if (cout->capacity < 0 || (cout->capacity > 0 && (!cout->seg_start || !cout->seg_end))) { ctx->set_error("tb_collapse_window_carry: carry_out has no room"); return 1; }
+  }
+  return tb_collapse_impl(ctx, in, out, cin, cout);
 }
 
 int tc_coverage_window(tb_ctx* ctx, const tc_soa_in* in, tc_runs_out* runs, tc_juncs_out* juncs) {

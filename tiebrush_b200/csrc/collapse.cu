@@ -87,14 +87,39 @@ struct MetaOut {
 struct HistIn { const uint32_t* c; __device__ uint32_t operator()(int64_t i) const { return c[i]; } };
 struct HistOut { uint32_t* p; __device__ void operator()(int64_t i, uint32_t exc, uint32_t) const { p[i] = exc; } };
 
+// ---- YD carry (tb_collapse_window_carry), host side -----------------------------------------------------------------------
+// carry_in re-filtered against B without any device work (a window with no records or no groups)
+int yd_carry_pass_host(tb_ctx* ctx, const tb_soa_in* hin, const tb_yd_carry* cin, tb_yd_carry* cout) {
+  const int nchains = 2 * hin->n_files;
+  const int32_t B = hin->pos_hi + 1;
+  auto keep = [&](int64_t q, int64_t b) { return cin->seg_end[q] >= B && (cin->seg_end[q] > cin->seg_start[q] || q == b - 1); };
+  int64_t tot = 0;
+  if (cin)
+    for (int c = 0; c < nchains; ++c)
+      for (int64_t q = cin->chain_off[c], b = cin->chain_off[c + 1]; q < b; ++q) tot += keep(q, b);
+  cout->n_segs = tot;
+  if (tot > cout->capacity) { ctx->set_error("tb_collapse_window_carry: carry_out capacity %lld < %lld segments", (long long)cout->capacity, (long long)tot); return 1; }
+  cout->tid = hin->tid; cout->pos_hi = hin->pos_hi;
+  int64_t j = 0;
+  for (int c = 0; c < nchains; ++c) {
+    cout->chain_off[c] = j;
+    if (cin)
+      for (int64_t q = cin->chain_off[c], b = cin->chain_off[c + 1]; q < b; ++q)
+        if (keep(q, b)) { cout->seg_start[j] = cin->seg_start[q]; cout->seg_end[j] = cin->seg_end[q]; ++j; }
+  }
+  cout->chain_off[nchains] = j;
+  return 0;
+}
+
 }  // namespace
 
-int tb_collapse_impl(tb_ctx* ctx, const tb_soa_in* hin, tb_groups_out* out) {
+int tb_collapse_impl(tb_ctx* ctx, const tb_soa_in* hin, tb_groups_out* out, const tb_yd_carry* cin, tb_yd_carry* cout) {
   TB_CUDA(cudaSetDevice(ctx->device));
   const int64_t n = hin->n;
   const int k = hin->n_files;
   out->n_groups = 0; out->n_kept = 0;
-  if (n == 0) return 0;
+  if (cin && cin->tid != hin->tid) cin = nullptr;   // the reference empties the lists at a tid change (tiebrush.cpp:586-589)
+  if (n == 0) return cout ? yd_carry_pass_host(ctx, hin, cin, cout) : 0;
   if (n >= (1LL << 31)) { ctx->set_error("tb_collapse_window: n=%lld too large for one window (< 2^31)", (long long)n); return 1; }
   if (k < 1 || k > ctx->n_samples) { ctx->set_error("tb_collapse_window: n_files=%d but the context was created for %d samples", k, ctx->n_samples); return 1; }
   bool any_merged = false;
@@ -212,6 +237,31 @@ int tb_collapse_impl(tb_ctx* ctx, const tb_soa_in* hin, tb_groups_out* out) {
     TB_CUDA(cudaMemcpyAsync(B[XB_MERGED].p, hin->file_merged, (size_t)k, cudaMemcpyHostToDevice, st));
     d_merged = B[XB_MERGED].as<uint8_t>();
   }
+  YdCarry cy;
+  const int nchains = 2 * k;
+  if (cin || cout) {   // device copy of carry_in; areas for the seeds and for carry_out
+    cy.in = cin != nullptr; cy.out = cout != nullptr;
+    cy.nin = cin ? cin->n_segs : 0;
+    cy.bout = hin->pos_hi + 1;
+    cy.cap = cout ? cout->capacity : 0;
+    TB_CUDA(B[XB_YDCARRY].ensure(sizeof(int64_t) * (nchains + 1) + sizeof(int32_t) * (3 * (size_t)nchains + 2 * (size_t)cy.nin) + 64));
+    long long* coff = B[XB_YDCARRY].as<long long>();
+    cy.seed = (int32_t*)(coff + nchains + 1); cy.ext = cy.seed + nchains; cy.efin = cy.ext + nchains;
+    if (cin) {
+      int32_t* cs = cy.efin + nchains; int32_t* ce = cs + cy.nin;
+      TB_CUDA(cudaMemcpyAsync(coff, cin->chain_off, sizeof(int64_t) * (nchains + 1), cudaMemcpyHostToDevice, st));
+      if (cy.nin > 0) {
+        TB_CUDA(cudaMemcpyAsync(cs, cin->seg_start, sizeof(int32_t) * (size_t)cy.nin, cudaMemcpyHostToDevice, st));
+        TB_CUDA(cudaMemcpyAsync(ce, cin->seg_end, sizeof(int32_t) * (size_t)cy.nin, cudaMemcpyHostToDevice, st));
+      }
+      cy.coff = coff; cy.cs = cs; cy.ce = ce;
+    }
+    if (cout) {
+      TB_CUDA(B[XB_YDCOUT].ensure(sizeof(int64_t) * (2 * (size_t)nchains + 1) + sizeof(int32_t) * 2 * (size_t)cy.cap + 64));
+      cy.ometa = B[XB_YDCOUT].as<long long>();
+      cy.os = (int32_t*)(cy.ometa + 2 * nchains + 1); cy.oe = cy.os + cy.cap;
+    }
+  }
   TB_CUDA(cudaStreamSynchronize(st));  // h_status and the caller's small host arrays may be reused from here on
   {
     int64_t mx = (int64_t)S + 2; if (n > mx) mx = n;
@@ -264,10 +314,10 @@ int tb_collapse_impl(tb_ctx* ctx, const tb_soa_in* hin, tb_groups_out* out) {
   if (G > out->capacity) { ctx->set_error("tb_collapse_window: output capacity %lld < %lld groups", (long long)out->capacity, (long long)G); return 1; }
   out->n_kept = kept;
   out->n_groups = G;
-  if (G == 0) return 0;
+  if (G == 0) return cout ? yd_carry_pass_host(ctx, hin, cin, cout) : 0;
   // ---- C7: YD ----
   if (ctx->profiling) TB_CUDA(cudaEventRecord(ctx->ev[2], st));
-  if (col_yd(ctx, in, g, grp, G)) return 1;
+  if (col_yd(ctx, in, g, grp, G, cy)) return 1;
   if (ctx->profiling) TB_CUDA(cudaEventRecord(ctx->ev[3], st));
   if (!out->on_device) {
     TB_CUDA(cudaMemcpyAsync(out->rep_index, grp.rep, sizeof(uint32_t) * G, cudaMemcpyDeviceToHost, st));
@@ -275,7 +325,32 @@ int tb_collapse_impl(tb_ctx* ctx, const tb_soa_in* hin, tb_groups_out* out) {
     TB_CUDA(cudaMemcpyAsync(out->yx, grp.yx, sizeof(uint32_t) * G, cudaMemcpyDeviceToHost, st));
     TB_CUDA(cudaMemcpyAsync(out->yd, grp.yd, sizeof(int32_t) * G, cudaMemcpyDeviceToHost, st));
   }
+  std::vector<long long> ometa;
+  std::vector<int32_t> oseg;
+  if (cout) {   // the carried lists come back in the order the chains reserved their slots
+    ometa.resize(2 * (size_t)nchains + 1);
+    TB_CUDA(cudaMemcpyAsync(ometa.data(), cy.ometa, sizeof(int64_t) * ometa.size(), cudaMemcpyDeviceToHost, st));
+    TB_CUDA(cudaStreamSynchronize(st));
+    const int64_t tot = ometa[2 * nchains];
+    cout->n_segs = tot;
+    if (tot > cout->capacity) { ctx->set_error("tb_collapse_window_carry: carry_out capacity %lld < %lld segments", (long long)cout->capacity, (long long)tot); return 1; }
+    oseg.resize(2 * (size_t)tot + 2);
+    if (tot > 0) {
+      TB_CUDA(cudaMemcpyAsync(oseg.data(), cy.os, sizeof(int32_t) * (size_t)tot, cudaMemcpyDeviceToHost, st));
+      TB_CUDA(cudaMemcpyAsync(oseg.data() + tot, cy.oe, sizeof(int32_t) * (size_t)tot, cudaMemcpyDeviceToHost, st));
+    }
+  }
   TB_CUDA(cudaStreamSynchronize(st));
+  if (cout) {
+    const int64_t tot = ometa[2 * nchains];
+    int64_t j = 0;
+    for (int c = 0; c < nchains; ++c) {
+      cout->chain_off[c] = j;
+      for (int64_t q = ometa[2 * c], e = q + ometa[2 * c + 1]; q < e; ++q, ++j) { cout->seg_start[j] = oseg[q]; cout->seg_end[j] = oseg[tot + q]; }
+    }
+    cout->chain_off[nchains] = j;
+    cout->tid = hin->tid; cout->pos_hi = hin->pos_hi;
+  }
   if (ctx->profiling) {
     float ms = 0;
     if (cudaEventElapsedTime(&ms, ctx->ev[6], ctx->ev[7]) == cudaSuccess) ctx->last_ms[4] = ms;

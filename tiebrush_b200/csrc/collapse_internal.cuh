@@ -19,9 +19,28 @@ struct ColGroups {
   uint32_t* bits;                                        // [G*W] direct-sample bitsets (XB_BITS)
 };
 
+// YD lists carried across a window cut (tb_collapse_window_carry), device side; a default-constructed value = no carry.
+// Chains are c = side * k + sample. The output area is filled in the order the chains reserve their slots; the host
+// puts it into chain order.
+struct YdCarry {
+  bool in = false;                 // lists seeded from carry_in (same tid)
+  bool out = false;                // lists wanted back
+  int64_t nin = 0;                 // carried segments
+  const long long* coff = nullptr; // [nchains+1] carry_in offsets
+  const int32_t* cs = nullptr;     // [nin] carry_in segments, 1-based inclusive
+  const int32_t* ce = nullptr;
+  int32_t* seed = nullptr;         // [nchains] frontier the chain starts from (compact on the parallel path), -1 = none
+  int32_t* ext = nullptr;          // [nchains] parallel path: how far the first live carried node reaches below the window
+  int32_t* efin = nullptr;         // [nchains] parallel path: frontier after the chain's last member
+  int32_t bout = 0;                // B of carry_out = pos_hi + 1
+  int64_t cap = 0;                 // entries of os / oe
+  int32_t* os = nullptr; int32_t* oe = nullptr;
+  long long* ometa = nullptr;      // [2*nchains] first slot and count per chain, then the slot cursor
+};
+
 // Fast path: shared-memory hash tiles. Returns 0 ok, 1 error, 2 = group table overflow (caller falls back to the ordered path).
 int col_front_tile(tb_ctx* ctx, const ColIn& in, const ColGeom& g, ColGroups& out, int64_t* n_groups, int64_t* n_kept);
 // Exact path: sequential emulation of the reference's per-position sorted list, in merge order.
 int col_front_ordered(tb_ctx* ctx, const ColIn& in, const ColGeom& g, ColGroups& out, int64_t* n_groups, int64_t* n_kept);
 // YD chains over the dense groups.
-int col_yd(tb_ctx* ctx, const ColIn& in, const ColGeom& g, const ColGroups& grp, int64_t G);
+int col_yd(tb_ctx* ctx, const ColIn& in, const ColGeom& g, const ColGroups& grp, int64_t G, const YdCarry& cy);

@@ -207,7 +207,7 @@ __global__ void __launch_bounds__(YDH_THREADS, 4) yd_heads_kernel(const uint32_t
                                                                  unsigned long long* __restrict__ st_max, unsigned long long* __restrict__ st_cnt,
                                                                  unsigned long long* __restrict__ ticket, uint32_t* __restrict__ flag,
                                                                  uint32_t* __restrict__ heads, uint32_t* __restrict__ nsub_out, unsigned long long* work,
-                                                                 long long* __restrict__ status) {
+                                                                 long long* __restrict__ status, const int32_t* __restrict__ seed) {
   __shared__ unsigned long long s_scan64[33];
   __shared__ uint32_t s_scan32[33];
   __shared__ unsigned long long s_tile, s_pa, s_pb;
@@ -223,7 +223,9 @@ __global__ void __launch_bounds__(YDH_THREADS, 4) yd_heads_kernel(const uint32_t
     key[k] = 0; gs[k] = 0;
     if (i < n_members) {
       const uint32_t g = chain[i];
-      key[k] = ((unsigned long long)mchain[i] << 32) | gend[g];
+      uint32_t ge = gend[g];
+      if (seed) { const int32_t sd = seed[mchain[i]]; if (sd >= 0 && (uint32_t)sd > ge) ge = (uint32_t)sd; }   // carried frontier
+      key[k] = ((unsigned long long)mchain[i] << 32) | ge;
       gs[k] = gstart[g];
       tm = key[k] > tm ? key[k] : tm;
     }
@@ -364,12 +366,21 @@ __device__ __forceinline__ void yd_cp_async16(void* smem_dst, const void* gsrc) 
 __device__ __forceinline__ void yd_cp_commit() { asm volatile("cp.async.commit_group;\n" ::: "memory"); }
 template <int N> __device__ __forceinline__ void yd_cp_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N) : "memory"); }
 
+// frontier after member i, kept when i is the last member of chain c (the carry_out of the parallel path needs it)
+__device__ __forceinline__ void yd_note_frontier(const uint32_t* headflag, uint32_t i, uint32_t c, uint32_t n_members, int E, int32_t* efin) {
+  if (i + 1 == n_members || (headflag[i + 1] >> 1) != c) efin[c] = E;
+}
+
 constexpr int YD_FWARPS = 4;   // warps per CTA of the frontier kernel (6 KB of shared-memory rings each)
+// CARRY: lists carried into the window (seed) and / or the final frontiers wanted (efin); the instantiation without
+// them is the kernel of a plain tb_collapse_window call
+template <bool CARRY>
 __global__ void __launch_bounds__(YD_FWARPS * 32) yd_frontier_kernel(ColIn in, const GDesc* __restrict__ cdesc, const uint32_t* __restrict__ rep,
                                                                     const uint32_t* __restrict__ chain, const uint32_t* __restrict__ headflag,
                                                                     const uint32_t* __restrict__ ustart, uint32_t nunits, unsigned long long* work,
                                                                     const uint32_t* __restrict__ U, const uint32_t* __restrict__ rankpre,
-                                                                    unsigned long long* __restrict__ bm, int64_t lpad, int32_t* __restrict__ mstart) {
+                                                                    unsigned long long* __restrict__ bm, int64_t lpad, int32_t* __restrict__ mstart,
+                                                                    const int32_t* __restrict__ seed, int32_t* __restrict__ efin, uint32_t n_members) {
   // two-stage pipeline per warp: member ids (group, head flag) are fetched 2*YD_PF steps ahead, descriptors YD_PF steps
   // ahead, so each of the two dependent gathers has YD_PF steps to land. A lane only ever reads ring entries it
   // requested itself (except in the replay, which synchronises the warp first).
@@ -421,7 +432,18 @@ __global__ void __launch_bounds__(YD_FWARPS * 32) yd_frontier_kernel(ColIn in, c
       // until nothing changes: a fixed point satisfies the recurrence member by member, hence is the exact result.
       int jx = 0; bool bulk = head != 0;
       int contrib = live ? (bulk ? dm.zend : dm.e0) : -1;
-      int e_after = F.E;
+      if (CARRY && seed && live && head) {   // a chain's first member after a cut: its step starts from the carried frontier
+        const int E0 = seed[s_flg[wl][islot][lane] >> 1];
+        if (E0 >= dm.start) {
+          bulk = false;
+          if (ne <= YD_INLINE_EX) {
+            jx = (ne >= 3 && E0 >= dm.s2) ? 2 : ((ne >= 2 && E0 >= dm.s1) ? 1 : 0);
+            contrib = jx == 2 ? dm.e2 : (jx == 1 ? dm.e1 : dm.e0);
+          } else jx = yd_reach(in, rep[g], E0, U, rankpre, &contrib);
+          contrib = max(contrib, E0);
+        }
+      }
+      int e_after = F.E, e_lane = -1;
       bool replay = false;
 #pragma unroll 1
       for (int iter = 0;; ++iter) {
@@ -445,7 +467,7 @@ __global__ void __launch_bounds__(YD_FWARPS * 32) yd_frontier_kernel(ColIn in, c
         }
         const bool changed = nb != bulk || nj != jx;
         bulk = nb; jx = nj; contrib = nc;
-        if (!__any_sync(0xffffffffu, changed)) { e_after = __shfl_sync(0xffffffffu, v, cnt - 1); break; }
+        if (!__any_sync(0xffffffffu, changed)) { e_after = __shfl_sync(0xffffffffu, v, cnt - 1); e_lane = v; break; }
         if (iter >= 8) { replay = true; break; }
       }
       uint32_t r = bulk ? (uint32_t)ne : (uint32_t)jx + 1u;
@@ -454,16 +476,21 @@ __global__ void __launch_bounds__(YD_FWARPS * 32) yd_frontier_kernel(ColIn in, c
         if (lane == 0) {
           for (int t = 0; t < cnt; ++t) {
             const GDesc& d = s_ring[wl][slot][t];
-            if (s_flg[wl][islot][t] & 1u) F.reset();
+            const uint32_t fl = s_flg[wl][islot][t];
+            if (fl & 1u) { F.reset(); if (CARRY && seed) F.E = seed[fl >> 1]; }
             const uint32_t rr = ((d.meta & 0xffffu) > (uint32_t)YD_INLINE_EX) ? rep[s_gid[wl][islot][t]] : 0u;
             s_r[wl][t] = (uint8_t)F.step(in, d, rr, U, rankpre);
+            if (CARRY && efin) yd_note_frontier(headflag, cb + (uint32_t)t, fl >> 1, n_members, F.E, efin);
           }
         }
         F.E = __shfl_sync(0xffffffffu, F.E, 0);
         __syncwarp();
         r = s_r[wl][lane];
         __syncwarp();
-      } else F.E = e_after;
+      } else {
+        F.E = e_after;
+        if (CARRY && efin && live) yd_note_frontier(headflag, cb + lane, s_flg[wl][islot][lane] >> 1, n_members, e_lane, efin);
+      }
       // Y7 fused: the kept exons OR their links into the chain's bitmap; compact start per member for the lookup
       if (live) {
         const int64_t base = (int64_t)(s_flg[wl][islot][lane] >> 1) * lpad;
@@ -501,32 +528,174 @@ struct LastZeroIn {   // highest clear bit of block b (global bit index), -1 if 
 struct LastZeroOut { long long* lz; __device__ void operator()(int64_t b, long long exc, long long) const { lz[b] = exc; } };
 
 // ---- Y9: d = number of consecutive set links ending at start-1 --------------------------------------------------------
+// last clear bit below bit q (global index) of the link bitmaps: the block's words, then the prefix over earlier blocks
+__device__ __forceinline__ long long yd_clear_below(const unsigned long long* __restrict__ bm, const long long* __restrict__ lz, int64_t q) {
+  int64_t w = q >> 6; const int b = (int)(q & 63);
+  unsigned long long zeros = ~bm[w] & ((1ULL << b) - 1ULL);
+  const int64_t wb = w & ~7LL;   // first word of the 512-bit block
+  for (;;) {
+    if (zeros) return w * 64 + (63 - __clzll((long long)zeros));
+    if (w == wb) return lz[wb >> 3];
+    --w; zeros = ~bm[w];
+  }
+}
+// ext (carried lists only): a run of links that reaches the chain's first bit continues the carried node that began before
+// the window, ext[chain] positions further down
 __global__ void __launch_bounds__(256) yd_lookup_kernel(const int32_t* __restrict__ mstart, const uint32_t* __restrict__ chain, int64_t n_members,
                                                         const uint32_t* __restrict__ flag, const unsigned long long* __restrict__ bm,
-                                                        const long long* __restrict__ lz, int64_t lpad, int32_t* __restrict__ yd) {
+                                                        const long long* __restrict__ lz, int64_t lpad, int32_t* __restrict__ yd,
+                                                        const int32_t* __restrict__ ext) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n_members) return;
   const int x = mstart[i];
-  if (x <= 0) return;
+  if (x <= 0) {
+    if (ext && x == 0) { const int32_t d = ext[flag[i] >> 1]; if (d > 0) atomicMax(&yd[chain[i]], d); }
+    return;
+  }
   const uint32_t g = chain[i];
   const int64_t base = (int64_t)(flag[i] >> 1) * lpad;
   const int64_t q = base + x - 1;
-  int64_t w = q >> 6; const int b = (int)(q & 63);
-  const unsigned long long word = bm[w];
-  if (!((word >> b) & 1ULL)) return;
-  unsigned long long zeros = ~word & ((1ULL << b) - 1ULL);
-  long long z = -2;
-  const int64_t wb = w & ~7LL;   // first word of the 512-bit block
-  for (;;) {
-    if (zeros) { z = w * 64 + (63 - __clzll((long long)zeros)); break; }
-    if (w == wb) break;
-    --w; zeros = ~bm[w];
-  }
-  if (z == -2) z = lz[wb >> 3];
+  if (!((bm[q >> 6] >> (q & 63)) & 1ULL)) return;
+  long long z = yd_clear_below(bm, lz, q);
   if (z < base - 1) z = base - 1;   // cannot happen (every chain's region ends with clear padding); keeps d bounded
-  const long long d = q - z;
+  long long d = q - z;
+  if (ext && z == base - 1) d += ext[flag[i] >> 1];
   if (d > 0) atomicMax(&yd[g], (int32_t)d);
 }
+
+// ---- carried lists (tb_collapse_window_carry) ---------------------------------------------------------------------------
+// Carry-in: chain c's list starts as the carried nodes that are still alive (end >= ubase, the window's first start). On
+// the parallel path that is what a first member of the chain made of those nodes would leave behind (all appended to an
+// empty list, links only inside a node): their positions enter U, their links enter the chain's bitmap, the chain's
+// frontier starts at the last node's end, and the one node that may begin below ubase is cut at ubase with the cut-off
+// length kept in ext[c]. On the sequential path the nodes are loaded into the list itself.
+__device__ __forceinline__ int yd_seg_chain(const long long* __restrict__ coff, int nchains, long long q) {   // last c with coff[c] <= q
+  int lo = 0, hi = nchains;
+  while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (coff[mid] <= q) lo = mid; else hi = mid; }
+  return lo;
+}
+__global__ void __launch_bounds__(256) yd_carry_u_kernel(const int32_t* __restrict__ cs, const int32_t* __restrict__ ce, int64_t nin, int ubase,
+                                                         uint32_t* __restrict__ U, int64_t ubits, long long* __restrict__ status) {
+  const int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= nin || ce[q] < ubase) return;
+  const int s = max(cs[q], ubase), e = ce[q];
+  if ((int64_t)e - ubase >= ubits) { status[YS_FALLBACK] = 1; return; }
+  yd_set_bits32(U, (int64_t)s - ubase, (int64_t)e - ubase);
+}
+// U == nullptr: sequential path, genomic seeds
+__global__ void __launch_bounds__(128) yd_carry_seed_kernel(const long long* __restrict__ coff, const int32_t* __restrict__ cs, const int32_t* __restrict__ ce,
+                                                            int nchains, int ubase, const uint32_t* __restrict__ U, const uint32_t* __restrict__ rankpre,
+                                                            int32_t* __restrict__ seed, int32_t* __restrict__ ext, int32_t* __restrict__ efin) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= nchains) return;
+  const long long a = coff[c], b = coff[c + 1];
+  int32_t sd = -1, x = 0;
+  if (b > a && ce[b - 1] >= ubase) {
+    sd = U ? yd_rank(U, rankpre, (int64_t)ce[b - 1] - ubase) : ce[b - 1];
+    for (long long q = a; q < b; ++q)
+      if (ce[q] >= ubase) { if (cs[q] < ubase) x = ubase - cs[q]; break; }
+  }
+  seed[c] = sd; ext[c] = x;
+  if (efin) efin[c] = sd;
+}
+__global__ void __launch_bounds__(256) yd_carry_links_kernel(const long long* __restrict__ coff, const int32_t* __restrict__ cs, const int32_t* __restrict__ ce,
+                                                             int64_t nin, int nchains, int ubase, const uint32_t* __restrict__ U,
+                                                             const uint32_t* __restrict__ rankpre, unsigned long long* __restrict__ bm, int64_t lpad) {
+  const int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= nin || ce[q] < ubase) return;
+  const int64_t base = (int64_t)yd_seg_chain(coff, nchains, q) * lpad;
+  const int64_t a = yd_rank(U, rankpre, (int64_t)max(cs[q], ubase) - ubase), b = yd_rank(U, rankpre, (int64_t)ce[q] - ubase);
+  if (b > a) yd_set_bits64(bm, base + a, base + b - 1);
+}
+
+// Carry-out, canonical form for B = pos_hi + 1: nodes with end >= B that cover two positions or more, and the last node
+// when its end >= B. A chain reserves its slots with one atomicAdd; past the capacity only the count is kept.
+__device__ __forceinline__ bool yd_keep_node(int32_t s, int32_t e, bool last, int32_t B) { return e >= B && (e > s || last); }
+__device__ __forceinline__ long long yd_reserve(long long* ometa, int nchains, int c, long long cnt) {
+  const long long slot = (long long)atomicAdd((unsigned long long*)&ometa[2 * nchains], (unsigned long long)cnt);
+  ometa[2 * c] = slot; ometa[2 * c + 1] = cnt;
+  return slot;
+}
+__device__ __forceinline__ void yd_put(int32_t* os, int32_t* oe, int64_t cap, long long at, int32_t s, int32_t e) {
+  if (at < cap) { os[at] = s; oe[at] = e; }
+}
+// compact coordinate -> genomic offset from ubase: the a-th set bit of U
+__device__ int64_t yd_select(const uint32_t* __restrict__ U, const uint32_t* __restrict__ rankpre, int64_t nuw, int64_t a) {
+  int64_t lo = 0, hi = nuw - 1;
+  while (lo < hi) { const int64_t mid = (lo + hi + 1) >> 1; if ((int64_t)rankpre[mid] <= a) lo = mid; else hi = mid - 1; }
+  uint32_t w = U[lo];
+  for (int64_t r = a - (int64_t)rankpre[lo]; r > 0; --r) w &= w - 1;
+  return lo * 32 + __ffs((int)w) - 1;
+}
+// first bit >= p (chain-relative) that is set (want = true) or clear, or lim
+__device__ int64_t yd_next_bit(const unsigned long long* __restrict__ bm, int64_t base, int64_t p, int64_t lim, bool want) {
+  while (p < lim) {
+    const int64_t gq = base + p, w = gq >> 6;
+    const unsigned long long word = (want ? bm[w] : ~bm[w]) & (~0ULL << (gq & 63));
+    if (word) { const int64_t r = w * 64 + __ffsll((long long)word) - 1 - base; return r < lim ? r : lim; }
+    p = (w + 1) * 64 - base;
+  }
+  return lim;
+}
+struct YdParOut {   // what the extraction on the parallel path reads
+  const unsigned long long* bm; const long long* lz; int64_t lpad;
+  const uint32_t* U; const uint32_t* rankpre; int64_t nuw; int ubase; int64_t bbit;   // bbit = B - ubase (< the bits of U)
+  const int32_t* ext; const int32_t* efin;
+};
+// nodes of chain c on the parallel path: the maximal runs of links ending at or beyond cB - 1, then the last node [E, E]
+// when the link below the frontier E is clear; written from slot `at` when write is set. Returns the node count.
+__device__ long long yd_par_nodes(const YdParOut& P, int c, bool write, long long at, int32_t* os, int32_t* oe, int64_t cap) {
+  const int64_t E = P.efin[c], cB = yd_rank(P.U, P.rankpre, P.bbit);   // cB: compact coordinate of the first covered position >= B
+  if (E < cB) return 0;
+  const int64_t base = (int64_t)c * P.lpad, p0 = cB > 0 ? cB - 1 : 0;
+  long long cnt = 0;
+  auto gend = [&](int64_t a) -> int32_t { return (int32_t)(P.ubase + yd_select(P.U, P.rankpre, P.nuw, a)); };
+  auto gstart = [&](int64_t a) -> int32_t { return (a == 0 && P.ext[c] > 0) ? P.ubase - P.ext[c] : gend(a); };
+  int64_t p = p0;
+  bool last_linked = false;
+  while (p < E) {
+    p = yd_next_bit(P.bm, base, p, E, true);
+    if (p >= E) break;
+    int64_t r0 = p;
+    if (p == p0 && p > 0 && ((P.bm[(base + p - 1) >> 6] >> ((base + p - 1) & 63)) & 1ULL)) {   // the run began before the scan
+      long long z = yd_clear_below(P.bm, P.lz, base + p);
+      r0 = z < base ? 0 : z + 1 - base;
+    }
+    const int64_t q = yd_next_bit(P.bm, base, p, E, false);   // links r0..q-1: node [r0, q]
+    if (write) yd_put(os, oe, cap, at + cnt, gstart(r0), gend(q));
+    ++cnt;
+    last_linked = q == E;
+    p = q;
+  }
+  if (!last_linked) { if (write) yd_put(os, oe, cap, at + cnt, gstart(E), gend(E)); ++cnt; }
+  return cnt;
+}
+// one thread per chain: chains without members in this window pass their carried nodes on (re-filtered against B);
+// on the parallel path the others are read from the link bitmaps (the sequential path wrote them from its lists)
+__global__ void __launch_bounds__(128) yd_carry_out_kernel(int nchains, const unsigned long long* __restrict__ colbase, const long long* __restrict__ coff,
+                                                           const int32_t* __restrict__ cs, const int32_t* __restrict__ ce, int32_t B, bool parallel,
+                                                           YdParOut P, int32_t* __restrict__ os, int32_t* __restrict__ oe, int64_t cap,
+                                                           long long* __restrict__ ometa) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= nchains) return;
+  if (colbase[c + 1] == colbase[c]) {
+    long long cnt = 0;
+    const long long a = coff ? coff[c] : 0, b = coff ? coff[c + 1] : 0;
+    for (long long q = a; q < b; ++q) cnt += yd_keep_node(cs[q], ce[q], q == b - 1, B);
+    const long long at = yd_reserve(ometa, nchains, c, cnt);
+    long long j = 0;
+    for (long long q = a; q < b; ++q) if (yd_keep_node(cs[q], ce[q], q == b - 1, B)) yd_put(os, oe, cap, at + j++, cs[q], ce[q]);
+  } else if (parallel) {
+    const long long cnt = yd_par_nodes(P, c, false, 0, os, oe, cap);
+    yd_par_nodes(P, c, true, yd_reserve(ometa, nchains, c, cnt), os, oe, cap);
+  }
+}
+// everything the sequential kernel needs for the carry
+struct YdSeqCarry {
+  const long long* coff; const int32_t* cs; const int32_t* ce;   // carry_in, nullptr = lists start empty
+  const unsigned long long* colbase; const uint32_t* flag; int nchains; int ubase;
+  int32_t B; int32_t* os; int32_t* oe; int64_t cap; long long* ometa;   // os == nullptr: no carry_out
+};
 
 // ---- sequential fallback: the literal list ------------------------------------------------------------------------------
 // one segment list; node q lives at st[q*32], en[q*32] (the lane offset is folded into the pointers)
@@ -576,6 +745,23 @@ struct SegArr {
     }
     return true;
   }
+  // the carried nodes of one chain that are still alive; false on capacity overflow
+  __device__ __noinline__ bool seed(const int32_t* cs, const int32_t* ce, long long a, long long b, int ubase) {
+    for (long long q = a; q < b; ++q) {
+      if (ce[q] < ubase) continue;
+      if (n >= cap) return false;
+      S(n) = (uint32_t)cs[q]; E(n) = (uint32_t)ce[q]; ++n;
+    }
+    return true;
+  }
+  // the list in canonical carry form
+  __device__ __noinline__ void export_carry(uint32_t c, const YdSeqCarry& k) {
+    long long cnt = 0;
+    for (int q = 0; q < n; ++q) cnt += yd_keep_node((int32_t)S(q), (int32_t)E(q), q == n - 1, k.B);
+    const long long at = yd_reserve(k.ometa, k.nchains, (int)c, cnt);
+    long long j = 0;
+    for (int q = 0; q < n; ++q) if (yd_keep_node((int32_t)S(q), (int32_t)E(q), q == n - 1, k.B)) yd_put(k.os, k.oe, k.cap, at + j++, (int32_t)S(q), (int32_t)E(q));
+  }
   // processRead :221-250
   template <class Src>
   __device__ int process(Src& src, uint32_t rstart, bool& ok) {
@@ -612,10 +798,11 @@ __device__ __forceinline__ int yd_step(const ColIn& in, SegArr& L, const GDesc& 
 constexpr int YD_CAP_SMEM = 24;      // live nodes per list in shared memory
 constexpr int YD_CAP_GLOBAL = 4096;  // live nodes per list in the global-memory repeat
 
-template <bool SMEM>
+template <bool SMEM, bool CARRY>   // CARRY: lists seeded from / exported to a carry (ca); false = plain tb_collapse_window
 __global__ void __launch_bounds__(YD_WARPS * 32) yd_chain_kernel(ColIn in, const GDesc* __restrict__ desc, const uint32_t* __restrict__ rep,
                                                                 const uint32_t* __restrict__ chain, const uint32_t* __restrict__ heads,
-                                                                unsigned long long* work, int32_t* __restrict__ yd, uint32_t* gscratch, long long* status) {
+                                                                unsigned long long* work, int32_t* __restrict__ yd, uint32_t* gscratch, long long* status,
+                                                                YdSeqCarry ca) {
   extern __shared__ __align__(16) uint32_t s_dyn[];   // SMEM: YD_WARPS * 2 * YD_CAP_SMEM * 32 words of lists
   __shared__ GDesc s_desc[YD_WARPS][32];
   __shared__ uint32_t s_g[YD_WARPS][32];
@@ -636,19 +823,24 @@ __global__ void __launch_bounds__(YD_WARPS * 32) yd_chain_kernel(ColIn in, const
     uint32_t c0 = 0, c1 = 0;
     if (j < nsub) { c0 = heads[j]; c1 = heads[j + 1]; }
     const uint32_t len = c1 - c0;
+    const uint32_t ch = (CARRY && len > 0) ? ca.flag[c0] >> 1 : 0u;
     if (len > 0 && len <= YD_LONG) {   // short sub-chains: one per lane
       L.reset();
+      if (CARRY && ca.coff && c0 == ca.colbase[ch]) ok = L.seed(ca.cs, ca.ce, ca.coff[ch], ca.coff[ch + 1], ca.ubase) && ok;
       for (uint32_t i = c0; i < c1; ++i) {
         const uint32_t g = chain[i];
         const int dist = yd_step(in, L, desc[g], rep[g], ok);
         if (dist > 0) atomicMax(&yd[g], dist);
       }
+      if (CARRY && ca.os && c1 == ca.colbase[ch + 1]) L.export_carry(ch, ca);
     }
     unsigned longs = __ballot_sync(0xffffffffu, len > YD_LONG);
     while (longs) {                    // long sub-chains: the whole warp walks them one after the other
       const int q = __ffs(longs) - 1; longs &= longs - 1;
       const uint32_t a = __shfl_sync(0xffffffffu, c0, q), b = __shfl_sync(0xffffffffu, c1, q);
+      const uint32_t chq = __shfl_sync(0xffffffffu, ch, q);
       L0.reset();
+      if (CARRY && lane == 0 && ca.coff && a == ca.colbase[chq]) ok = L0.seed(ca.cs, ca.ce, ca.coff[chq], ca.coff[chq + 1], ca.ubase) && ok;
       uint32_t gnext = 0; GDesc dnext; dnext.start = 0; dnext.meta = 0; dnext.e0 = dnext.s1 = dnext.e1 = dnext.s2 = dnext.e2 = dnext.zend = 0;
       if (a + lane < b) { gnext = chain[a + lane]; dnext = desc[gnext]; }
       for (uint32_t cb = a; cb < b; cb += 32) {
@@ -668,6 +860,7 @@ __global__ void __launch_bounds__(YD_WARPS * 32) yd_chain_kernel(ColIn in, const
         if (cb + lane < b) { const int dist = s_d[wl][lane]; if (dist > 0) atomicMax(&yd[g], dist); }
         __syncwarp();
       }
+      if (CARRY && lane == 0 && ca.os && b == ca.colbase[chq + 1]) L0.export_carry(chq, ca);
     }
   }
   if (!ok) status[CS_YD_OVERFLOW] = 1;
@@ -681,7 +874,7 @@ __global__ void yd_store_lc_kernel(const uint32_t* tot, long long* status) { sta
 
 }  // namespace
 
-int col_yd(tb_ctx* ctx, const ColIn& in, const ColGeom& g, const ColGroups& grp, int64_t G) {
+int col_yd(tb_ctx* ctx, const ColIn& in, const ColGeom& g, const ColGroups& grp, int64_t G, const YdCarry& cy) {
   cudaStream_t st = ctx->stream;
   DevBuf* B = ctx->buf;
   const uint32_t W = g.W; const int k = g.k; const int nchains = 2 * k;
@@ -717,11 +910,16 @@ int col_yd(tb_ctx* ctx, const ColIn& in, const ColGeom& g, const ColGroups& grp,
   }
   TB_CUDA(cudaMemsetAsync(ydc, 0, sizeof(int32_t) * (size_t)G, st));
   TB_CUDA(cudaMemsetAsync(g.d_status + YS_FALLBACK, 0, 2 * sizeof(long long), st));
+  if (cy.out) TB_CUDA(cudaMemsetAsync(cy.ometa + 2 * nchains, 0, sizeof(long long), st));
   int64_t agg_need = tb_scan_blocks((int64_t)nblk * nchains); if (tb_scan_blocks(nuw) > agg_need) agg_need = tb_scan_blocks(nuw);
   TB_CUDA(B[XB_AGG].ensure((size_t)(agg_need + 8) * sizeof(uint64_t)));
   // ---- Y1, Y2 ----
   yd_desc_kernel<<<tb_grid_for(G, 256), 256, 0, st>>>(in, grp.rep, G, desc, gend, gstart, gstrand, U, ubits, g.d_status);
   ctx->launches++;
+  if (parallel && cy.in && cy.nin > 0) {   // carried nodes take part in the compact coordinates
+    yd_carry_u_kernel<<<tb_grid_for(cy.nin, 256), 256, 0, st>>>(cy.cs, cy.ce, cy.nin, ubase, U, ubits, g.d_status);
+    ctx->launches++;
+  }
   if (parallel) {
     TB_CUDA((tb_device_scan<OpSumU32>(ctx, UPopIn{U}, nuw, B[XB_AGG].as<uint32_t>(), UPopOut{rankpre})));
     yd_store_lc_kernel<<<1, 1, 0, st>>>(B[XB_AGG].as<uint32_t>() + tb_scan_blocks(nuw), g.d_status);
@@ -743,6 +941,15 @@ int col_yd(tb_ctx* ctx, const ColIn& in, const ColGeom& g, const ColGroups& grp,
   if (h_status[YS_FALLBACK]) parallel = false;
   const int64_t Lc = h_status[YS_LC];
   ctx->last_yd_path = parallel ? 0 : 1;
+  if (cy.in) {
+    yd_carry_seed_kernel<<<tb_grid_for(nchains, 128), 128, 0, st>>>(cy.coff, cy.cs, cy.ce, nchains, ubase, parallel ? U : nullptr, rankpre, cy.seed, cy.ext,
+                                                                  parallel && cy.out ? cy.efin : nullptr);
+    ctx->launches++;
+  } else if (parallel && cy.out) {
+    TB_CUDA(cudaMemsetAsync(cy.efin, 0xff, sizeof(int32_t) * (size_t)nchains, st));
+  }
+  const int32_t* seed = cy.in ? cy.seed : nullptr;
+  YdParOut pout; memset(&pout, 0, sizeof(pout));
   if (n_members > 0) {
     TB_CUDA(B[XB_YDCHAIN].ensure(sizeof(uint32_t) * ((size_t)n_members + 32)));
     TB_CUDA(B[XB_BHEAD].ensure(sizeof(uint32_t) * ((size_t)n_members + 32)));
@@ -771,7 +978,7 @@ int col_yd(tb_ctx* ctx, const ColIn& in, const ColGeom& g, const ColGroups& grp,
       unsigned long long* ticket = st_cnt + ntiles;
       TB_CUDA(cudaMemsetAsync(st_max, 0, sizeof(uint64_t) * (2 * (size_t)ntiles + 8), st));
       yd_heads_kernel<<<(unsigned)ntiles, YDH_THREADS, 0, st>>>(chain, mchain, he, hs, (uint32_t)n_members, st_max, st_cnt, ticket, flag, heads, nsub_dev, work,
-                                                               g.d_status);
+                                                               g.d_status, seed);
       ctx->launches++;
     }
     if (parallel) {
@@ -783,20 +990,30 @@ int col_yd(tb_ctx* ctx, const ColIn& in, const ColGeom& g, const ColGroups& grp,
       unsigned long long* bm = B[XB_YDBM].as<unsigned long long>();
       long long* lz = B[XB_YDLZ].as<long long>();
       TB_CUDA(cudaMemsetAsync(bm, 0, sizeof(uint64_t) * (size_t)nwords, st));
+      if (cy.in && cy.nin > 0) {
+        yd_carry_links_kernel<<<tb_grid_for(cy.nin, 256), 256, 0, st>>>(cy.coff, cy.cs, cy.ce, cy.nin, nchains, ubase, U, rankpre, bm, lpad);
+        ctx->launches++;
+      }
       const uint32_t nunits = (uint32_t)((n_members + YD_UNIT - 1) / YD_UNIT);
       TB_CUDA(B[XB_YDUNIT].ensure(sizeof(uint32_t) * ((size_t)nunits + 2)));
       uint32_t* ustart = B[XB_YDUNIT].as<uint32_t>();
       yd_unit_kernel<<<tb_grid_for((int64_t)nunits + 1, 256), 256, 0, st>>>(heads, nsub_dev, (uint32_t)n_members, nunits, ustart);
-      yd_frontier_kernel<<<(unsigned)ctx->sm_count * 16, YD_FWARPS * 32, 0, st>>>(in, cdesc, grp.rep, chain, flag, ustart, nunits, work, U, rankpre, bm, lpad, mstart);
+      (seed || cy.out ? yd_frontier_kernel<true> : yd_frontier_kernel<false>)<<<(unsigned)ctx->sm_count * 16, YD_FWARPS * 32, 0, st>>>(in, cdesc, grp.rep, chain, flag, ustart, nunits, work, U, rankpre, bm, lpad, mstart,
+                                                                                  seed, cy.out ? cy.efin : nullptr, (uint32_t)n_members);
       ctx->launches++;
       ctx->launches += 2;
       TB_CUDA((tb_device_scan<OpMaxI64>(ctx, LastZeroIn{bm}, nblocks512, B[XB_AGG].as<long long>(), LastZeroOut{lz})));
-      yd_lookup_kernel<<<tb_grid_for(n_members, 256), 256, 0, st>>>(mstart, chain, n_members, flag, bm, lz, lpad, ydc);
+      yd_lookup_kernel<<<tb_grid_for(n_members, 256), 256, 0, st>>>(mstart, chain, n_members, flag, bm, lz, lpad, ydc, cy.in ? cy.ext : nullptr);
       ctx->launches++;
+      pout = YdParOut{bm, lz, lpad, U, rankpre, nuw, ubase, (int64_t)cy.bout - ubase, cy.ext, cy.efin};
+      if (cy.out && !cy.in) TB_CUDA(cudaMemsetAsync(cy.ext, 0, sizeof(int32_t) * (size_t)nchains, st));
     } else {
+      YdSeqCarry ca{cy.in ? cy.coff : nullptr, cy.cs, cy.ce, colbase, flag, nchains, ubase, cy.bout, cy.out ? cy.os : nullptr, cy.oe, cy.cap, cy.ometa};
       const size_t smem = (size_t)YD_WARPS * 2 * YD_CAP_SMEM * 32 * sizeof(uint32_t);
-      TB_CUDA(cudaFuncSetAttribute(yd_chain_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      yd_chain_kernel<true><<<(unsigned)ctx->sm_count * 4, YD_WARPS * 32, smem, st>>>(in, desc, grp.rep, chain, heads, work, ydc, nullptr, g.d_status);
+      const bool carry = cy.in || cy.out;
+      auto chain_smem = carry ? yd_chain_kernel<true, true> : yd_chain_kernel<true, false>;
+      TB_CUDA(cudaFuncSetAttribute(chain_smem, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      chain_smem<<<(unsigned)ctx->sm_count * 4, YD_WARPS * 32, smem, st>>>(in, desc, grp.rep, chain, heads, work, ydc, nullptr, g.d_status, ca);
       ctx->launches++;
       TB_CUDA(cudaMemcpyAsync(h_status, g.d_status, sizeof(int64_t) * 16, cudaMemcpyDeviceToHost, st));
       TB_CUDA(cudaStreamSynchronize(st));
@@ -807,13 +1024,19 @@ int col_yd(tb_ctx* ctx, const ColIn& in, const ColGeom& g, const ColGroups& grp,
         TB_CUDA(cudaMemsetAsync(ydc, 0, sizeof(int32_t) * (size_t)G, st));
         TB_CUDA(cudaMemsetAsync(work, 0, sizeof(unsigned long long), st));
         TB_CUDA(cudaMemsetAsync(g.d_status + CS_YD_OVERFLOW, 0, sizeof(long long), st));
-        yd_chain_kernel<false><<<grid2, YD_WARPS * 32, 0, st>>>(in, desc, grp.rep, chain, heads, work, ydc, B[XB_YDSCRATCH].as<uint32_t>(), g.d_status);
+        if (cy.out) TB_CUDA(cudaMemsetAsync(cy.ometa + 2 * nchains, 0, sizeof(long long), st));
+        (carry ? yd_chain_kernel<false, true> : yd_chain_kernel<false, false>)<<<grid2, YD_WARPS * 32, 0, st>>>(in, desc, grp.rep, chain, heads, work, ydc, B[XB_YDSCRATCH].as<uint32_t>(), g.d_status, ca);
         ctx->launches++;
         TB_CUDA(cudaMemcpyAsync(h_status, g.d_status, sizeof(int64_t) * 16, cudaMemcpyDeviceToHost, st));
         TB_CUDA(cudaStreamSynchronize(st));
         if (h_status[CS_YD_OVERFLOW]) { ctx->set_error("tb_collapse_window: YD segment list exceeded %d live nodes", YD_CAP_GLOBAL); return 1; }
       }
     }
+  }
+  if (cy.out) {
+    yd_carry_out_kernel<<<tb_grid_for(nchains, 128), 128, 0, st>>>(nchains, colbase, cy.in ? cy.coff : nullptr, cy.cs, cy.ce, cy.bout, parallel && n_members > 0,
+                                                                   pout, cy.os, cy.oe, cy.cap, cy.ometa);
+    ctx->launches++;
   }
   yd_combine_kernel<<<tb_grid_for(G, 256), 256, 0, st>>>(grp.yd, ydc, G);
   ctx->launches++;

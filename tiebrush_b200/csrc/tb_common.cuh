@@ -51,7 +51,7 @@ struct HostBuf {  // grow-only pinned host buffer
   template <class T> T* as() { return (T*)p; }
 };
 
-enum { TB_NBUF = 48 };
+enum { TB_NBUF = 52 };
 
 struct tb_ctx {
   int device = 0;

@@ -204,6 +204,8 @@ enum {
   XB_ORD_LIST, XB_ORD_GREP, XB_ORD_GYC, XB_ORD_GYX, XB_ORD_GYD, XB_ORD_VALID, XB_ORD_GBITS,                // ordered path: per-position group lists
   XB_META_DICT,   // u64 [256] dictionary of the packed wire format
   XB_ORD_DEEP,    // ordered path: counter + list of the deep start positions
+  XB_YDCARRY,     // YD carry: device copy of carry_in, per-chain seed / ext / final frontier
+  XB_YDCOUT,      // YD carry: carry_out area (per-chain slots, cursor, segments)
   XB_COUNT_
 };
 static_assert(XB_COUNT_ <= TB_NBUF, "raise TB_NBUF");

@@ -397,6 +397,35 @@ def collapse_shard_local(compute, cols, run_off, lo, hi, extra=()):
     return dict(rep_index=rep[keep], yc=np.asarray(res["yc"])[keep], yx=np.asarray(res["yx"])[keep], yd=np.asarray(res["yd"])[keep])
 
 
+def collapse_cut_windows(compute, cols, run_off, cuts, yd_carry, pos_range=None, extra=()):
+    """Collapse one file-major window (one tid) as a sequence of windows cut at the start positions `cuts` (0-based; a
+    window holds the records with cut_i <= pos < cut_i+1), the YD lists carried from each window to the next. No coverage
+    gap is needed at a cut. `compute(sub_cols, sub_run_off, pos_range=(lo, hi), yd_carry=carry)` is the call of one window
+    (api.Context.collapse_window, or the oracle) and returns the lists it leaves behind as "yd_carry". `yd_carry` = the
+    carry the first window starts from (the result of the previous tid, or an empty one). `pos_range` = (lo, hi) of the
+    whole window, default (min pos, max pos + 1). Returns the concatenated groups with rep_index into `cols`, n_kept, the
+    final yd_carry and the carried segments per cut (`carried`)."""
+    pos = np.asarray(cols["pos"])
+    if pos_range is None:
+        pos_range = (int(pos.min()), int(pos.max()) + 1) if len(pos) else (0, 1)
+    lo, hi = int(pos_range[0]), int(pos_range[1])
+    bounds = [lo] + sorted({int(c) for c in cuts if lo < int(c) < hi}) + [hi]
+    reps, ycs, yxs, yds, carried, kept = [], [], [], [], [], 0
+    for a, b in zip(bounds[:-1], bounds[1:]):
+        idx, sub_off = _file_slices(cols, run_off, a, b)
+        sub = sam.take(cols, idx)
+        for k in extra:
+            sub[k] = cols[k]
+        res = compute(sub, sub_off, pos_range=(a, b), yd_carry=yd_carry)
+        yd_carry = res["yd_carry"]
+        carried.append(int(yd_carry["chain_off"][-1]))
+        reps.append(idx[np.asarray(res["rep_index"]).astype(np.int64)])
+        ycs.append(np.asarray(res["yc"])); yxs.append(np.asarray(res["yx"])); yds.append(np.asarray(res["yd"]))
+        kept += int(res["n_kept"])
+    return dict(rep_index=np.concatenate(reps), yc=np.concatenate(ycs).astype(np.float32), yx=np.concatenate(yxs).astype(np.uint32),
+                yd=np.concatenate(yds).astype(np.int32), n_kept=kept, yd_carry=yd_carry, carried=carried)
+
+
 def collapse_sharded(compute, cols, run_off, cuts, group=None):
     """Sharded tiebrush over one window every rank can read (each rank slices its own coordinate range, as a host
     reader with a BAM index would). Ordered gather of the groups on rank 0."""
