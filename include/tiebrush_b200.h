@@ -294,6 +294,10 @@ int tb_last_path(tb_ctx*);
 /* YD stage of the last tb_collapse_window call: 0 = parallel formulation (frontier recurrence + link bitmaps),
  * 1 = sequential segment lists (degenerate exons / more than 255 exons in a representative, or TB_YD_PATH=seq). */
 int tb_last_yd_path(tb_ctx*);
+/* Sizes of the YD stage of the last tb_collapse_window call: 0 chain members (one per group, sample and strand list),
+ * 1 sub-chains (independent runs of a chain's members), 2 compact length Lc (covered positions; 0 on the sequential
+ * path), 3 blocks of 1024 groups the member lists are counted in. -1 for another `which`. */
+int64_t tb_last_yd_stat(tb_ctx*, int which);
 /* Tile slots of the last call that were redone by the full-size-table launch (pile-up positions with more distinct
  * alignments than a quarter-SM table holds). */
 int64_t tb_last_heavy_slots(tb_ctx*);

@@ -181,6 +181,10 @@ class Context:
         """0 parallel YD formulation, 1 sequential segment lists."""
         return int(self.lib.tb_last_yd_path(self.h))
 
+    def last_yd_stats(self):
+        """YD stage of the last collapse call: chain members, sub-chains, compact length Lc (0 on the sequential path), 1024-group blocks."""
+        return dict(zip(("n_members", "n_subchains", "lc", "nblk"), (int(self.lib.tb_last_yd_stat(self.h, i)) for i in range(4))))
+
     def last_path(self):
         """0 tile path, 1 ordered path (by options), 2 ordered path (table-overflow fallback)."""
         return int(self.lib.tb_last_path(self.h))

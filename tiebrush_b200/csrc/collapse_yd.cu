@@ -19,8 +19,9 @@
 //       last_pos cache).
 //   So: Y1 group descriptors + union bitmap U of all exon positions; Y2 rank(U) gives compact coordinates (runs of links
 //   are preserved: a link at p implies p+1 is covered); Y3-Y5 chain member lists by a stable counting scatter over the
-//   sample bitsets, cut into independent sub-chains where a member starts beyond every earlier end of its chain (one
-//   single-pass look-back kernel: segmented prefix max of the ends, head test, head list);
+//   sample bitsets, cut into independent sub-chains where a member starts beyond every earlier end of its chain (the
+//   count pass also keeps each chain's largest end per block of groups, a scan turns those into prefix maxima, and the
+//   scatter runs the head test in registers as it writes the members; one stream compaction of the head bits);
 //   Y6 the frontier recurrence per sub-chain (one scalar, lane-parallel; long sub-chains are walked by a whole warp with
 //   prefetch) -> kept-exon count per member; Y7 kept exons OR their links into the chain's bitmap; Y8 prefix max of
 //   "last clear link" over 512-bit blocks; Y9 one lookup per member, atomicMax into the group.
@@ -97,8 +98,7 @@ __device__ __forceinline__ int32_t yd_rank(const uint32_t* __restrict__ U, const
   return (int32_t)(rankpre[w] + (uint32_t)__popc(U[w] & ((1u << (bit & 31)) - 1u)));
 }
 __global__ void __launch_bounds__(256) yd_compact_kernel(const GDesc* __restrict__ desc, int64_t G, const uint32_t* __restrict__ U,
-                                                         const uint32_t* __restrict__ rankpre, int ubase, GDesc* __restrict__ cdesc, uint32_t* __restrict__ cend,
-                                                         uint32_t* __restrict__ cstart) {
+                                                         const uint32_t* __restrict__ rankpre, int ubase, GDesc* __restrict__ cdesc) {
   const int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (g >= G) return;
   GDesc d = desc[g];
@@ -109,165 +109,130 @@ __global__ void __launch_bounds__(256) yd_compact_kernel(const GDesc* __restrict
   if (ne >= 3) { d.s2 = yd_rank(U, rankpre, (int64_t)d.s2 - ubase); d.e2 = yd_rank(U, rankpre, (int64_t)d.e2 - ubase); }
   d.zend = yd_rank(U, rankpre, (int64_t)d.zend - ubase);
   cdesc[g] = d;
-  cend[g] = (uint32_t)d.zend;
-  cstart[g] = (uint32_t)d.start;
 }
 
-// ---- Y3-Y5: chain member lists ---------------------------------------------------------------------------------------
+// ---- Y3-Y5: chain member lists and their sub-chain heads ---------------------------------------------------------------
+// A member heads a sub-chain when it is its chain's first, or when its start lies beyond every earlier end of the chain
+// (and beyond the carried frontier). The test runs in GENOMIC coordinates on both paths: on the parallel path every group
+// start and end and every carried frontier is a covered position, and rank() is strictly increasing over covered
+// positions, so the answer is the one of the compact coordinates. The member pass therefore needs neither the compact
+// coordinates nor the path choice (known only at the host sync after the count).
 constexpr int YD_BLOCK = 1024;   // groups per counting block
-// members per (chain, block of groups); chain c = side*k + sample, table is chain-major: blkcnt[c*nblk + b]
+// key of a chain's largest end (group end, raised to the carried frontier) in the prefix-maximum table: chain ids ascend
+// in the chain-major table, so the plain prefix maximum is the segmented one; 0 = no member of the chain so far
+__device__ __forceinline__ unsigned long long yd_end_key(int c, uint32_t e) { return ((unsigned long long)(c + 1) << 32) | e; }
+// per (chain, block of groups): members, and the key of their largest end (0 without members); chain c = side*k + sample,
+// tables are chain-major: blkcnt[c*nblk + b]. seed: carried frontier per chain (genomic, -1 = none), nullptr without carry.
 __global__ void __launch_bounds__(128) yd_count_kernel(const uint32_t* __restrict__ bits, uint32_t W, int k, int64_t G, const uint8_t* __restrict__ gstrand,
-                                                      uint32_t* __restrict__ blkcnt, int64_t nblk) {
+                                                      const uint32_t* __restrict__ gend, const int32_t* __restrict__ seed,
+                                                      uint32_t* __restrict__ blkcnt, unsigned long long* __restrict__ blkkey, int64_t nblk) {
   const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   if (warp >= nblk * W) return;
   const int64_t b = warp / W; const uint32_t w = (uint32_t)(warp % W);
   const int lane = tb_lane();
   const int64_t g0 = b * YD_BLOCK, g1 = (g0 + YD_BLOCK < G) ? g0 + YD_BLOCK : G;
-  uint32_t cf = 0, cr = 0;
+  uint32_t cf = 0, cr = 0, mf = 0, mr = 0;
   for (int64_t base = g0; base < g1; base += 32) {
     const int64_t g = base + lane;
-    uint32_t word = 0; uint8_t sc = 0;
-    if (g < g1) { word = bits[(uint64_t)g * W + w]; sc = gstrand[g]; }
+    uint32_t word = 0, ge = 0; uint8_t sc = 0;
+    if (g < g1) { word = bits[(uint64_t)g * W + w]; if (word) { sc = gstrand[g]; ge = gend[g]; } }
     unsigned any = __ballot_sync(0xffffffffu, word != 0);
     while (any) {
       const int q = __ffs(any) - 1; any &= any - 1;
       const uint32_t wq = __shfl_sync(0xffffffffu, word, q);
       const int sq = __shfl_sync(0xffffffffu, (int)sc, q);
-      if ((wq >> lane) & 1u) { cf += (sq != '-'); cr += (sq != '+'); }
+      const uint32_t eq = __shfl_sync(0xffffffffu, ge, q);
+      if ((wq >> lane) & 1u) {
+        if (sq != '-') { ++cf; mf = eq > mf ? eq : mf; }
+        if (sq != '+') { ++cr; mr = eq > mr ? eq : mr; }
+      }
     }
   }
   const int s = (int)(w * 32 + lane);
-  if (s < k) { blkcnt[(int64_t)s * nblk + b] = cf; blkcnt[((int64_t)k + s) * nblk + b] = cr; }
+  if (s < k) {
+    const int cfw = s, crv = k + s;
+    if (seed) {
+      if (seed[cfw] >= 0 && (uint32_t)seed[cfw] > mf) mf = (uint32_t)seed[cfw];
+      if (seed[crv] >= 0 && (uint32_t)seed[crv] > mr) mr = (uint32_t)seed[crv];
+    }
+    blkcnt[(int64_t)cfw * nblk + b] = cf; blkkey[(int64_t)cfw * nblk + b] = cf ? yd_end_key(cfw, mf) : 0ULL;
+    blkcnt[(int64_t)crv * nblk + b] = cr; blkkey[(int64_t)crv * nblk + b] = cr ? yd_end_key(crv, mr) : 0ULL;
+  }
 }
 struct CntIn { const uint32_t* c; __device__ unsigned long long operator()(int64_t i) const { return c[i]; } };
 struct CntOut { unsigned long long* o; __device__ void operator()(int64_t i, unsigned long long exc, unsigned long long) const { o[i] = exc; } };
 struct OpSumU64 { typedef unsigned long long T; __host__ __device__ static T identity() { return 0; } __host__ __device__ static T combine(T a, T b) { return a + b; } };
+// exclusive prefix maximum of the end keys, in place: every element is read by the thread that later overwrites it
+struct EndMaxIn { const unsigned long long* t; __device__ unsigned long long operator()(int64_t i) const { return t[i]; } };
+struct EndMaxOut { unsigned long long* t; __device__ void operator()(int64_t i, unsigned long long exc, unsigned long long) const { t[i] = exc; } };
 __global__ void __launch_bounds__(128) yd_colbase_kernel(const unsigned long long* __restrict__ blkoff, const unsigned long long* __restrict__ total, int64_t nblk,
                                                          int nchains, unsigned long long* __restrict__ colbase) {
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c < nchains) colbase[c] = blkoff[(int64_t)c * nblk];
   if (c == nchains) colbase[c] = *total;
 }
-// stable scatter of the group ids into the chain lists
+// stable scatter of the members into the chain lists: mem[i] = (group id, head | chain << 1), one 8-byte store per member
+// (the lanes of a warp write 32 different chains, so every store instruction costs a sector per lane). Each lane owns two
+// chains (the sample's two strand lists) and carries their running end key in a register, from the prefix maximum of the
+// earlier blocks.
 __global__ void __launch_bounds__(128) yd_scatter_kernel(const uint32_t* __restrict__ bits, uint32_t W, int k, int64_t G, const uint8_t* __restrict__ gstrand,
-                                                        const unsigned long long* __restrict__ blkoff, int64_t nblk, uint32_t* __restrict__ chain) {
+                                                        const uint32_t* __restrict__ gstart, const uint32_t* __restrict__ gend, const int32_t* __restrict__ seed,
+                                                        const unsigned long long* __restrict__ blkoff, const unsigned long long* __restrict__ blkpre, int64_t nblk,
+                                                        uint2* __restrict__ mem) {
   const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   if (warp >= nblk * W) return;
   const int64_t b = warp / W; const uint32_t w = (uint32_t)(warp % W);
   const int lane = tb_lane();
   const int s = (int)(w * 32 + lane);
   const int64_t g0 = b * YD_BLOCK, g1 = (g0 + YD_BLOCK < G) ? g0 + YD_BLOCK : G;
-  unsigned long long pf = 0, pr = 0;
-  if (s < k) { pf = blkoff[(int64_t)s * nblk + b]; pr = blkoff[((int64_t)k + s) * nblk + b]; }
+  const int cf = s, cr = k + s;
+  unsigned long long pf = 0, pr = 0, runf = 0, runr = 0;
+  uint32_t sf = 0, sr = 0;   // carried frontiers (0 = none: every end key is above it)
+  if (s < k) {
+    pf = blkoff[(int64_t)cf * nblk + b]; pr = blkoff[(int64_t)cr * nblk + b];
+    runf = blkpre[(int64_t)cf * nblk + b]; runr = blkpre[(int64_t)cr * nblk + b];
+    if (seed) { sf = seed[cf] > 0 ? (uint32_t)seed[cf] : 0u; sr = seed[cr] > 0 ? (uint32_t)seed[cr] : 0u; }
+  }
+  const unsigned long long hf = (unsigned long long)(cf + 1) << 32, hr = (unsigned long long)(cr + 1) << 32;
   for (int64_t base = g0; base < g1; base += 32) {
     const int64_t g = base + lane;
-    uint32_t word = 0; uint8_t sc = 0;
-    if (g < g1) { word = bits[(uint64_t)g * W + w]; sc = gstrand[g]; }
+    uint32_t word = 0, gs = 0, ge = 0; uint8_t sc = 0;
+    if (g < g1) { word = bits[(uint64_t)g * W + w]; if (word) { sc = gstrand[g]; gs = gstart[g]; ge = gend[g]; } }
     unsigned any = __ballot_sync(0xffffffffu, word != 0);
     while (any) {
       const int q = __ffs(any) - 1; any &= any - 1;
       const uint32_t wq = __shfl_sync(0xffffffffu, word, q);
       const int sq = __shfl_sync(0xffffffffu, (int)sc, q);
+      const uint32_t sx = __shfl_sync(0xffffffffu, gs, q), ex = __shfl_sync(0xffffffffu, ge, q);
       if ((wq >> lane) & 1u) {
-        if (sq != '-') chain[pf++] = (uint32_t)(base + q);
-        if (sq != '+') chain[pr++] = (uint32_t)(base + q);
+        // head: first member of the chain (no key of this chain yet), or a start beyond every earlier end and the seed
+        if (sq != '-') {
+          const bool h = runf < hf || sx > (uint32_t)runf;
+          mem[pf++] = make_uint2((uint32_t)(base + q), (h ? 1u : 0u) | ((uint32_t)cf << 1));
+          const unsigned long long key = hf | (ex > sf ? ex : sf);
+          runf = key > runf ? key : runf;
+        }
+        if (sq != '+') {
+          const bool h = runr < hr || sx > (uint32_t)runr;
+          mem[pr++] = make_uint2((uint32_t)(base + q), (h ? 1u : 0u) | ((uint32_t)cr << 1));
+          const unsigned long long key = hr | (ex > sr ? ex : sr);
+          runr = key > runr ? key : runr;
+        }
       }
     }
   }
 }
 
-// chain id of every member: chain c owns members [colbase[c], colbase[c+1]). One binary search per block of YD_FILL members,
-// then every thread walks forward over the (few) chain boundaries inside the block; coalesced 2-byte stores.
-constexpr int YD_FILL = 16384;
-__global__ void __launch_bounds__(256) yd_fill_mchain_kernel(const unsigned long long* __restrict__ colbase, int nchains, unsigned long long n_members,
-                                                             uint16_t* __restrict__ mchain) {
-  __shared__ int s_c0;
-  const unsigned long long a = (unsigned long long)blockIdx.x * YD_FILL;
-  if (threadIdx.x == 0) {
-    int lo = 0, hi = nchains;   // last c with colbase[c] <= a
-    while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (colbase[mid] <= a) lo = mid; else hi = mid; }
-    s_c0 = lo;
+// Y5: list of the sub-chain heads by one stream compaction of the head bits. heads[nsub] = n_members closes the last
+// sub-chain; work[0] (the work-unit counter of the frontier / sequential kernels) starts at 0 and work[1] = nsub.
+struct HeadIn { const uint2* mem; __device__ uint32_t operator()(int64_t i) const { return mem[i].y & 1u; } };
+struct HeadOut {
+  uint32_t* heads; int64_t n; unsigned long long* work;
+  __device__ void operator()(int64_t i, uint32_t exc, uint32_t inc) const {
+    if (inc != exc) heads[exc] = (uint32_t)i;
+    if (i == n - 1) { heads[inc] = (uint32_t)n; work[0] = 0; work[1] = inc; }
   }
-  __syncthreads();
-  int c = s_c0;
-  for (unsigned long long i = a + threadIdx.x; i < a + YD_FILL && i < n_members; i += 256) {
-    while (c + 1 < nchains && colbase[c + 1] <= i) ++c;
-    mchain[i] = (uint16_t)c;
-  }
-}
-
-// Y5 in ONE pass over the members (decoupled look-back, see tb_common.cuh): the segmented prefix maximum of the group ends
-// (key = chain << 32 | end: chain ids ascend, so the plain prefix maximum is the segmented one), the head test against it,
-// flag[i] = head | chain << 1, and the list of sub-chain heads (a head's list slot is the prefix count of heads before it).
-// Replaces two three-phase scans (the member keys were gathered three times).
-constexpr int YDH_THREADS = 256, YDH_ITEMS = 8, YDH_TILE = YDH_THREADS * YDH_ITEMS;
-enum { YS_LBFAIL = 10 };
-__global__ void __launch_bounds__(YDH_THREADS, 4) yd_heads_kernel(const uint32_t* __restrict__ chain, const uint16_t* __restrict__ mchain,
-                                                                 const uint32_t* __restrict__ gend, const uint32_t* __restrict__ gstart, uint32_t n_members,
-                                                                 unsigned long long* __restrict__ st_max, unsigned long long* __restrict__ st_cnt,
-                                                                 unsigned long long* __restrict__ ticket, uint32_t* __restrict__ flag,
-                                                                 uint32_t* __restrict__ heads, uint32_t* __restrict__ nsub_out, unsigned long long* work,
-                                                                 long long* __restrict__ status, const int32_t* __restrict__ seed) {
-  __shared__ unsigned long long s_scan64[33];
-  __shared__ uint32_t s_scan32[33];
-  __shared__ unsigned long long s_tile, s_pa, s_pb;
-  if (threadIdx.x == 0) s_tile = atomicAdd(ticket, 1ULL);
-  __syncthreads();
-  const long long tile = (long long)s_tile;
-  const uint32_t base = (uint32_t)tile * YDH_TILE + threadIdx.x * YDH_ITEMS;
-  unsigned long long key[YDH_ITEMS]; uint32_t gs[YDH_ITEMS];
-  unsigned long long tm = 0;
-#pragma unroll
-  for (int k = 0; k < YDH_ITEMS; ++k) {
-    const uint32_t i = base + k;
-    key[k] = 0; gs[k] = 0;
-    if (i < n_members) {
-      const uint32_t g = chain[i];
-      uint32_t ge = gend[g];
-      if (seed) { const int32_t sd = seed[mchain[i]]; if (sd >= 0 && (uint32_t)sd > ge) ge = (uint32_t)sd; }   // carried frontier
-      key[k] = ((unsigned long long)mchain[i] << 32) | ge;
-      gs[k] = gstart[g];
-      tm = key[k] > tm ? key[k] : tm;
-    }
-  }
-  unsigned long long tot;
-  const unsigned long long texc = tb_block_exscan<OpMaxU64>(tm, s_scan64, &tot);
-  if (threadIdx.x == 0) lb_store(&st_max[tile], LB_AGG | tot);
-  if (threadIdx.x < 32) {
-    const unsigned long long pa = lb_lookback<true>(st_max, tile, &status[YS_LBFAIL]);
-    if (threadIdx.x == 0) { s_pa = pa; lb_store(&st_max[tile], LB_INC | (pa > tot ? pa : tot)); }
-  }
-  __syncthreads();
-  unsigned long long run = s_pa > texc ? s_pa : texc;   // exclusive prefix maximum at this thread's first member
-  uint32_t headm = 0, hc = 0;
-#pragma unroll
-  for (int k = 0; k < YDH_ITEMS; ++k) {
-    const uint32_t i = base + k;
-    if (i < n_members) {
-      const uint32_t c = (uint32_t)(key[k] >> 32);
-      const bool h = i == 0 || (uint32_t)(run >> 32) != c || gs[k] > (uint32_t)run;
-      if (h) { headm |= 1u << k; ++hc; }
-      flag[i] = (h ? 1u : 0u) | (c << 1);
-      run = key[k] > run ? key[k] : run;
-    }
-  }
-  uint32_t htot;
-  const uint32_t hexc = tb_block_exscan<OpSumU32>(hc, s_scan32, &htot);
-  if (threadIdx.x == 0) lb_store(&st_cnt[tile], LB_AGG | (unsigned long long)htot);
-  if (threadIdx.x < 32) {
-    const unsigned long long pb = lb_lookback<false>(st_cnt, tile, &status[YS_LBFAIL]);
-    if (threadIdx.x == 0) { s_pb = pb; lb_store(&st_cnt[tile], LB_INC | (pb + htot)); }
-  }
-  __syncthreads();
-  uint32_t cnt = (uint32_t)s_pb + hexc;   // heads before this thread's first member
-#pragma unroll
-  for (int k = 0; k < YDH_ITEMS; ++k) {
-    const uint32_t i = base + k;
-    if (i >= n_members) break;
-    if (headm & (1u << k)) heads[cnt++] = i;
-    if (i == n_members - 1) { heads[cnt] = n_members; *nsub_out = cnt; work[0] = 0; work[1] = cnt; }
-  }
-}
+};
 
 constexpr int YD_WARPS = 8;
 constexpr uint32_t YD_LONG = 16;     // sub-chains longer than this are walked by the whole warp
@@ -342,10 +307,10 @@ __device__ __forceinline__ void yd_emit_links(const ColIn& in, const GDesc& d, u
 // classes (later exons of a spliced read dropped; or everything reached after a spanning read) settle in 1-2 scans.
 constexpr int YD_PF = 4;
 constexpr uint32_t YD_UNIT = 2048;
-__global__ void __launch_bounds__(256) yd_unit_kernel(const uint32_t* __restrict__ heads, const uint32_t* __restrict__ nsub_p, uint32_t n_members, uint32_t nunits,
-                                                      uint32_t* __restrict__ ustart) {
+__global__ void __launch_bounds__(256) yd_unit_kernel(const uint32_t* __restrict__ heads, const unsigned long long* __restrict__ nsub_p, uint32_t n_members,
+                                                      uint32_t nunits, uint32_t* __restrict__ ustart) {
   const uint32_t u = blockIdx.x * blockDim.x + threadIdx.x;
-  const uint32_t nsub = *nsub_p;
+  const uint32_t nsub = (uint32_t)*nsub_p;
   if (u > nunits) return;
   if (u == nunits) { ustart[u] = n_members; return; }
   const uint32_t target = u * YD_UNIT;
@@ -357,8 +322,8 @@ __global__ void __launch_bounds__(256) yd_unit_kernel(const uint32_t* __restrict
 // asynchronous global -> shared copies (LDGSTS): the gathers of the software pipeline below land in shared memory
 // without holding registers, so the loop body exists once (no unrolled register queues) and stays inside the
 // instruction cache
-__device__ __forceinline__ void yd_cp_async4(void* smem_dst, const void* gsrc) {
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 4;\n" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)), "l"(gsrc) : "memory");
+__device__ __forceinline__ void yd_cp_async8(void* smem_dst, const void* gsrc) {
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 8;\n" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)), "l"(gsrc) : "memory");
 }
 __device__ __forceinline__ void yd_cp_async16(void* smem_dst, const void* gsrc) {
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)), "l"(gsrc) : "memory");
@@ -367,8 +332,8 @@ __device__ __forceinline__ void yd_cp_commit() { asm volatile("cp.async.commit_g
 template <int N> __device__ __forceinline__ void yd_cp_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N) : "memory"); }
 
 // frontier after member i, kept when i is the last member of chain c (the carry_out of the parallel path needs it)
-__device__ __forceinline__ void yd_note_frontier(const uint32_t* headflag, uint32_t i, uint32_t c, uint32_t n_members, int E, int32_t* efin) {
-  if (i + 1 == n_members || (headflag[i + 1] >> 1) != c) efin[c] = E;
+__device__ __forceinline__ void yd_note_frontier(const uint2* mem, uint32_t i, uint32_t c, uint32_t n_members, int E, int32_t* efin) {
+  if (i + 1 == n_members || (mem[i + 1].y >> 1) != c) efin[c] = E;
 }
 
 constexpr int YD_FWARPS = 4;   // warps per CTA of the frontier kernel (6 KB of shared-memory rings each)
@@ -376,7 +341,7 @@ constexpr int YD_FWARPS = 4;   // warps per CTA of the frontier kernel (6 KB of 
 // them is the kernel of a plain tb_collapse_window call
 template <bool CARRY>
 __global__ void __launch_bounds__(YD_FWARPS * 32) yd_frontier_kernel(ColIn in, const GDesc* __restrict__ cdesc, const uint32_t* __restrict__ rep,
-                                                                    const uint32_t* __restrict__ chain, const uint32_t* __restrict__ headflag,
+                                                                    const uint2* __restrict__ mem,
                                                                     const uint32_t* __restrict__ ustart, uint32_t nunits, unsigned long long* work,
                                                                     const uint32_t* __restrict__ U, const uint32_t* __restrict__ rankpre,
                                                                     unsigned long long* __restrict__ bm, int64_t lpad, int32_t* __restrict__ mstart,
@@ -385,8 +350,7 @@ __global__ void __launch_bounds__(YD_FWARPS * 32) yd_frontier_kernel(ColIn in, c
   // ahead, so each of the two dependent gathers has YD_PF steps to land. A lane only ever reads ring entries it
   // requested itself (except in the replay, which synchronises the warp first).
   __shared__ __align__(16) GDesc s_ring[YD_FWARPS][YD_PF][32];
-  __shared__ uint32_t s_gid[YD_FWARPS][2 * YD_PF][32];
-  __shared__ uint32_t s_flg[YD_FWARPS][2 * YD_PF][32];
+  __shared__ __align__(8) uint2 s_mem[YD_FWARPS][2 * YD_PF][32];   // (group id, head | chain << 1)
   __shared__ uint8_t s_r[YD_FWARPS][32];
   const int wl = tb_warp(), lane = tb_lane();
   for (;;) {
@@ -401,14 +365,14 @@ __global__ void __launch_bounds__(YD_FWARPS * 32) yd_frontier_kernel(ColIn in, c
 #pragma unroll
     for (int p = 0; p < 2 * YD_PF; ++p) {
       const uint32_t idx = a + (uint32_t)p * 32u + lane;
-      if (idx < b) { yd_cp_async4(&s_gid[wl][p][lane], chain + idx); yd_cp_async4(&s_flg[wl][p][lane], headflag + idx); }
+      if (idx < b) yd_cp_async8(&s_mem[wl][p][lane], mem + idx);
     }
     yd_cp_commit();
     yd_cp_wait<0>();
 #pragma unroll
     for (int p = 0; p < YD_PF; ++p) {
       if (a + (uint32_t)p * 32u + lane < b) {
-        const GDesc* src = cdesc + s_gid[wl][p][lane];
+        const GDesc* src = cdesc + s_mem[wl][p][lane].x;
         yd_cp_async16(&s_ring[wl][p][lane], src); yd_cp_async16(reinterpret_cast<char*>(&s_ring[wl][p][lane]) + 16, reinterpret_cast<const char*>(src) + 16);
       }
       yd_cp_commit();
@@ -422,7 +386,7 @@ __global__ void __launch_bounds__(YD_FWARPS * 32) yd_frontier_kernel(ColIn in, c
       const bool live = lane < cnt;
       GDesc dm; dm.start = 0; dm.meta = 0; dm.e0 = dm.s1 = dm.e1 = dm.s2 = dm.e2 = dm.zend = 0;
       uint32_t g = 0; int head = 0;
-      if (live) { dm = s_ring[wl][slot][lane]; g = s_gid[wl][islot][lane]; head = (int)(s_flg[wl][islot][lane] & 1u); }
+      if (live) { dm = s_ring[wl][slot][lane]; g = s_mem[wl][islot][lane].x; head = (int)(s_mem[wl][islot][lane].y & 1u); }
       const int ne = (int)(dm.meta & 0xffffu);
       // For a frontier E >= start the step is  E' = max(E, end of the last exon whose start <= E)  and exactly the
       // exons up to that one are kept (exon starts lie beyond the previous exon's end); for E < start every exon is
@@ -433,7 +397,7 @@ __global__ void __launch_bounds__(YD_FWARPS * 32) yd_frontier_kernel(ColIn in, c
       int jx = 0; bool bulk = head != 0;
       int contrib = live ? (bulk ? dm.zend : dm.e0) : -1;
       if (CARRY && seed && live && head) {   // a chain's first member after a cut: its step starts from the carried frontier
-        const int E0 = seed[s_flg[wl][islot][lane] >> 1];
+        const int E0 = seed[s_mem[wl][islot][lane].y >> 1];
         if (E0 >= dm.start) {
           bulk = false;
           if (ne <= YD_INLINE_EX) {
@@ -476,11 +440,11 @@ __global__ void __launch_bounds__(YD_FWARPS * 32) yd_frontier_kernel(ColIn in, c
         if (lane == 0) {
           for (int t = 0; t < cnt; ++t) {
             const GDesc& d = s_ring[wl][slot][t];
-            const uint32_t fl = s_flg[wl][islot][t];
+            const uint32_t fl = s_mem[wl][islot][t].y;
             if (fl & 1u) { F.reset(); if (CARRY && seed) F.E = seed[fl >> 1]; }
-            const uint32_t rr = ((d.meta & 0xffffu) > (uint32_t)YD_INLINE_EX) ? rep[s_gid[wl][islot][t]] : 0u;
+            const uint32_t rr = ((d.meta & 0xffffu) > (uint32_t)YD_INLINE_EX) ? rep[s_mem[wl][islot][t].x] : 0u;
             s_r[wl][t] = (uint8_t)F.step(in, d, rr, U, rankpre);
-            if (CARRY && efin) yd_note_frontier(headflag, cb + (uint32_t)t, fl >> 1, n_members, F.E, efin);
+            if (CARRY && efin) yd_note_frontier(mem, cb + (uint32_t)t, fl >> 1, n_members, F.E, efin);
           }
         }
         F.E = __shfl_sync(0xffffffffu, F.E, 0);
@@ -489,11 +453,11 @@ __global__ void __launch_bounds__(YD_FWARPS * 32) yd_frontier_kernel(ColIn in, c
         __syncwarp();
       } else {
         F.E = e_after;
-        if (CARRY && efin && live) yd_note_frontier(headflag, cb + lane, s_flg[wl][islot][lane] >> 1, n_members, e_lane, efin);
+        if (CARRY && efin && live) yd_note_frontier(mem, cb + lane, s_mem[wl][islot][lane].y >> 1, n_members, e_lane, efin);
       }
       // Y7 fused: the kept exons OR their links into the chain's bitmap; compact start per member for the lookup
       if (live) {
-        const int64_t base = (int64_t)(s_flg[wl][islot][lane] >> 1) * lpad;
+        const int64_t base = (int64_t)(s_mem[wl][islot][lane].y >> 1) * lpad;
         yd_emit_links(in, dm, r, r > (uint32_t)YD_INLINE_EX ? rep[g] : 0u, U, rankpre, bm, base);
         mstart[cb + lane] = dm.start;
       }
@@ -501,11 +465,11 @@ __global__ void __launch_bounds__(YD_FWARPS * 32) yd_frontier_kernel(ColIn in, c
       {
         const uint32_t idx = cb + 32u * YD_PF + lane;
         if (idx < b) {
-          const GDesc* src = cdesc + s_gid[wl][nslot][lane];
+          const GDesc* src = cdesc + s_mem[wl][nslot][lane].x;
           yd_cp_async16(&s_ring[wl][slot][lane], src); yd_cp_async16(reinterpret_cast<char*>(&s_ring[wl][slot][lane]) + 16, reinterpret_cast<const char*>(src) + 16);
         }
         const uint32_t idx2 = cb + 32u * 2 * YD_PF + lane;
-        if (idx2 < b) { yd_cp_async4(&s_gid[wl][islot][lane], chain + idx2); yd_cp_async4(&s_flg[wl][islot][lane], headflag + idx2); }
+        if (idx2 < b) yd_cp_async8(&s_mem[wl][islot][lane], mem + idx2);
         yd_cp_commit();
       }
     }
@@ -541,25 +505,26 @@ __device__ __forceinline__ long long yd_clear_below(const unsigned long long* __
 }
 // ext (carried lists only): a run of links that reaches the chain's first bit continues the carried node that began before
 // the window, ext[chain] positions further down
-__global__ void __launch_bounds__(256) yd_lookup_kernel(const int32_t* __restrict__ mstart, const uint32_t* __restrict__ chain, int64_t n_members,
-                                                        const uint32_t* __restrict__ flag, const unsigned long long* __restrict__ bm,
+__global__ void __launch_bounds__(256) yd_lookup_kernel(const int32_t* __restrict__ mstart, const uint2* __restrict__ mem, int64_t n_members,
+                                                        const unsigned long long* __restrict__ bm,
                                                         const long long* __restrict__ lz, int64_t lpad, int32_t* __restrict__ yd,
                                                         const int32_t* __restrict__ ext) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n_members) return;
   const int x = mstart[i];
   if (x <= 0) {
-    if (ext && x == 0) { const int32_t d = ext[flag[i] >> 1]; if (d > 0) atomicMax(&yd[chain[i]], d); }
+    if (ext && x == 0) { const int32_t d = ext[mem[i].y >> 1]; if (d > 0) atomicMax(&yd[mem[i].x], d); }
     return;
   }
-  const uint32_t g = chain[i];
-  const int64_t base = (int64_t)(flag[i] >> 1) * lpad;
+  const uint2 m = mem[i];
+  const uint32_t g = m.x;
+  const int64_t base = (int64_t)(m.y >> 1) * lpad;
   const int64_t q = base + x - 1;
   if (!((bm[q >> 6] >> (q & 63)) & 1ULL)) return;
   long long z = yd_clear_below(bm, lz, q);
   if (z < base - 1) z = base - 1;   // cannot happen (every chain's region ends with clear padding); keeps d bounded
   long long d = q - z;
-  if (ext && z == base - 1) d += ext[flag[i] >> 1];
+  if (ext && z == base - 1) d += ext[m.y >> 1];
   if (d > 0) atomicMax(&yd[g], (int32_t)d);
 }
 
@@ -693,7 +658,7 @@ __global__ void __launch_bounds__(128) yd_carry_out_kernel(int nchains, const un
 // everything the sequential kernel needs for the carry
 struct YdSeqCarry {
   const long long* coff; const int32_t* cs; const int32_t* ce;   // carry_in, nullptr = lists start empty
-  const unsigned long long* colbase; const uint32_t* flag; int nchains; int ubase;
+  const unsigned long long* colbase; const uint2* mem; int nchains; int ubase;
   int32_t B; int32_t* os; int32_t* oe; int64_t cap; long long* ometa;   // os == nullptr: no carry_out
 };
 
@@ -800,7 +765,7 @@ constexpr int YD_CAP_GLOBAL = 4096;  // live nodes per list in the global-memory
 
 template <bool SMEM, bool CARRY>   // CARRY: lists seeded from / exported to a carry (ca); false = plain tb_collapse_window
 __global__ void __launch_bounds__(YD_WARPS * 32) yd_chain_kernel(ColIn in, const GDesc* __restrict__ desc, const uint32_t* __restrict__ rep,
-                                                                const uint32_t* __restrict__ chain, const uint32_t* __restrict__ heads,
+                                                                const uint2* __restrict__ mem, const uint32_t* __restrict__ heads,
                                                                 unsigned long long* work, int32_t* __restrict__ yd, uint32_t* gscratch, long long* status,
                                                                 YdSeqCarry ca) {
   extern __shared__ __align__(16) uint32_t s_dyn[];   // SMEM: YD_WARPS * 2 * YD_CAP_SMEM * 32 words of lists
@@ -823,12 +788,12 @@ __global__ void __launch_bounds__(YD_WARPS * 32) yd_chain_kernel(ColIn in, const
     uint32_t c0 = 0, c1 = 0;
     if (j < nsub) { c0 = heads[j]; c1 = heads[j + 1]; }
     const uint32_t len = c1 - c0;
-    const uint32_t ch = (CARRY && len > 0) ? ca.flag[c0] >> 1 : 0u;
+    const uint32_t ch = (CARRY && len > 0) ? ca.mem[c0].y >> 1 : 0u;
     if (len > 0 && len <= YD_LONG) {   // short sub-chains: one per lane
       L.reset();
       if (CARRY && ca.coff && c0 == ca.colbase[ch]) ok = L.seed(ca.cs, ca.ce, ca.coff[ch], ca.coff[ch + 1], ca.ubase) && ok;
       for (uint32_t i = c0; i < c1; ++i) {
-        const uint32_t g = chain[i];
+        const uint32_t g = mem[i].x;
         const int dist = yd_step(in, L, desc[g], rep[g], ok);
         if (dist > 0) atomicMax(&yd[g], dist);
       }
@@ -842,12 +807,12 @@ __global__ void __launch_bounds__(YD_WARPS * 32) yd_chain_kernel(ColIn in, const
       L0.reset();
       if (CARRY && lane == 0 && ca.coff && a == ca.colbase[chq]) ok = L0.seed(ca.cs, ca.ce, ca.coff[chq], ca.coff[chq + 1], ca.ubase) && ok;
       uint32_t gnext = 0; GDesc dnext; dnext.start = 0; dnext.meta = 0; dnext.e0 = dnext.s1 = dnext.e1 = dnext.s2 = dnext.e2 = dnext.zend = 0;
-      if (a + lane < b) { gnext = chain[a + lane]; dnext = desc[gnext]; }
+      if (a + lane < b) { gnext = mem[a + lane].x; dnext = desc[gnext]; }
       for (uint32_t cb = a; cb < b; cb += 32) {
         const uint32_t g = gnext;
         s_desc[wl][lane] = dnext; s_g[wl][lane] = gnext;
         __syncwarp();
-        if (cb + 32 + lane < b) { gnext = chain[cb + 32 + lane]; dnext = desc[gnext]; }   // prefetch the next batch
+        if (cb + 32 + lane < b) { gnext = mem[cb + 32 + lane].x; dnext = desc[gnext]; }   // prefetch the next batch
         if (lane == 0) {
           const int cnt = (int)((b - cb) < 32u ? (b - cb) : 32u);
           for (int t = 0; t < cnt; ++t) {
@@ -885,20 +850,20 @@ int col_yd(tb_ctx* ctx, const ColIn& in, const ColGeom& g, const ColGroups& grp,
   const int64_t nuw = (ubits + 31) / 32 + 1;
   const int ubase = in.pos_lo + 1;
   TB_CUDA(B[XB_GDESC].ensure(sizeof(GDesc) * (size_t)G * 2));
-  TB_CUDA(B[XB_YDPM].ensure(sizeof(uint32_t) * (size_t)G * 4 + (size_t)G + 64));
-  TB_CUDA(B[XB_YDBLK].ensure(sizeof(uint32_t) * (size_t)nblk * nchains + sizeof(uint64_t) * ((size_t)nblk * nchains + nchains + 16)));
+  TB_CUDA(B[XB_YDPM].ensure(sizeof(uint32_t) * (size_t)G * 2 + (size_t)G + 64));
+  TB_CUDA(B[XB_YDBLK].ensure(sizeof(uint32_t) * ((size_t)nblk * nchains + nchains) + sizeof(uint64_t) * (2 * (size_t)nblk * nchains + nchains + 16)));
   TB_CUDA(B[XB_WORK].ensure(256));
   TB_CUDA(B[XB_YDC].ensure(sizeof(int32_t) * (size_t)G));
   GDesc* desc = B[XB_GDESC].as<GDesc>();
   GDesc* cdesc = desc + G;
   uint32_t* gend = B[XB_YDPM].as<uint32_t>();
-  uint32_t* cend = gend + G;
-  uint32_t* gstart = cend + G;
-  uint32_t* cstart = gstart + G;
-  uint8_t* gstrand = (uint8_t*)(cstart + G);
+  uint32_t* gstart = gend + G;
+  uint8_t* gstrand = (uint8_t*)(gstart + G);
   unsigned long long* blkoff = B[XB_YDBLK].as<unsigned long long>();            // [nchains*nblk] exclusive member offsets, chain-major
-  unsigned long long* colbase = blkoff + (size_t)nblk * nchains;                // [nchains+1]
+  unsigned long long* blkkey = blkoff + (size_t)nblk * nchains;                 // [nchains*nblk] end keys, then their exclusive prefix maxima
+  unsigned long long* colbase = blkkey + (size_t)nblk * nchains;                // [nchains+1]
   uint32_t* blkcnt = (uint32_t*)(colbase + nchains + 16);                       // [nchains*nblk]
+  int32_t* gseed = (int32_t*)(blkcnt + (size_t)nblk * nchains);                 // [nchains] carried frontier, genomic
   unsigned long long* work = B[XB_WORK].as<unsigned long long>() + 8;           // the tile kernel's slot counter sits at +0
   int32_t* ydc = B[XB_YDC].as<int32_t>();
   long long* h_status = ctx->pinned[0].as<long long>();
@@ -925,13 +890,18 @@ int col_yd(tb_ctx* ctx, const ColIn& in, const ColGeom& g, const ColGroups& grp,
     yd_store_lc_kernel<<<1, 1, 0, st>>>(B[XB_AGG].as<uint32_t>() + tb_scan_blocks(nuw), g.d_status);
     ctx->launches++;
   }
-  // ---- Y3: member counts -> offsets ----
+  // ---- Y3: member counts -> offsets; largest ends -> per-chain prefix maxima (head test in genomic coordinates, see Y3-Y5) ----
+  if (cy.in) {
+    yd_carry_seed_kernel<<<tb_grid_for(nchains, 128), 128, 0, st>>>(cy.coff, cy.cs, cy.ce, nchains, ubase, nullptr, nullptr, gseed, cy.ext, nullptr);
+    ctx->launches++;
+  }
   const int64_t nwarps = nblk * W;
-  yd_count_kernel<<<tb_grid_for(nwarps * 32, 128), 128, 0, st>>>(grp.bits, W, k, G, gstrand, blkcnt, nblk);
+  yd_count_kernel<<<tb_grid_for(nwarps * 32, 128), 128, 0, st>>>(grp.bits, W, k, G, gstrand, gend, cy.in ? gseed : nullptr, blkcnt, blkkey, nblk);
   ctx->launches++;
   TB_CUDA((tb_device_scan<OpSumU64>(ctx, CntIn{blkcnt}, (int64_t)nblk * nchains, B[XB_AGG].as<unsigned long long>(), CntOut{blkoff})));
   yd_colbase_kernel<<<tb_grid_for(nchains + 1, 128), 128, 0, st>>>(blkoff, B[XB_AGG].as<unsigned long long>() + tb_scan_blocks((int64_t)nblk * nchains), nblk, nchains, colbase);
   ctx->launches++;
+  TB_CUDA((tb_device_scan<OpMaxU64>(ctx, EndMaxIn{blkkey}, (int64_t)nblk * nchains, B[XB_AGG].as<unsigned long long>(), EndMaxOut{blkkey})));
   // member count, compact length and the fallback flag are only known on the device
   TB_CUDA(cudaMemcpyAsync(h_status, g.d_status, sizeof(int64_t) * 16, cudaMemcpyDeviceToHost, st));
   TB_CUDA(cudaMemcpyAsync(h_status + 16, colbase + nchains, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
@@ -941,6 +911,7 @@ int col_yd(tb_ctx* ctx, const ColIn& in, const ColGeom& g, const ColGroups& grp,
   if (h_status[YS_FALLBACK]) parallel = false;
   const int64_t Lc = h_status[YS_LC];
   ctx->last_yd_path = parallel ? 0 : 1;
+  ctx->last_yd_stat[0] = n_members; ctx->last_yd_stat[1] = 0; ctx->last_yd_stat[2] = parallel ? Lc : 0; ctx->last_yd_stat[3] = nblk;
   if (cy.in) {
     yd_carry_seed_kernel<<<tb_grid_for(nchains, 128), 128, 0, st>>>(cy.coff, cy.cs, cy.ce, nchains, ubase, parallel ? U : nullptr, rankpre, cy.seed, cy.ext,
                                                                   parallel && cy.out ? cy.efin : nullptr);
@@ -951,34 +922,19 @@ int col_yd(tb_ctx* ctx, const ColIn& in, const ColGeom& g, const ColGroups& grp,
   const int32_t* seed = cy.in ? cy.seed : nullptr;
   YdParOut pout; memset(&pout, 0, sizeof(pout));
   if (n_members > 0) {
-    TB_CUDA(B[XB_YDCHAIN].ensure(sizeof(uint32_t) * ((size_t)n_members + 32)));
+    TB_CUDA(B[XB_YDCHAIN].ensure(sizeof(uint2) * ((size_t)n_members + 32)));
     TB_CUDA(B[XB_BHEAD].ensure(sizeof(uint32_t) * ((size_t)n_members + 32)));
-    TB_CUDA(B[XB_YDFLAG].ensure((sizeof(uint32_t) + sizeof(uint16_t)) * ((size_t)n_members + 32)));
     const int64_t lpad = ((Lc + 1 + 511) / 512) * 512;            // bits per chain, at least one clear padding bit
     const int64_t nwords = lpad / 64 * nchains, nblocks512 = nwords / 8;
     TB_CUDA(B[XB_AGG].ensure((size_t)(tb_scan_blocks(nblocks512 > n_members ? nblocks512 : n_members) + 8) * sizeof(uint64_t)));
-    uint32_t* chain = B[XB_YDCHAIN].as<uint32_t>(); uint32_t* heads = B[XB_BHEAD].as<uint32_t>(); uint32_t* flag = B[XB_YDFLAG].as<uint32_t>();
-    uint16_t* mchain = (uint16_t*)(flag + n_members + 32);
-    yd_scatter_kernel<<<tb_grid_for(nwarps * 32, 128), 128, 0, st>>>(grp.bits, W, k, G, gstrand, blkoff, nblk, chain);
-    yd_fill_mchain_kernel<<<(unsigned)((n_members + YD_FILL - 1) / YD_FILL), 256, 0, st>>>(colbase, nchains, (unsigned long long)n_members, mchain);
-    ctx->launches += 2;
-    const uint32_t* hs = gstart; const uint32_t* he = gend;
-    if (parallel) {
-      yd_compact_kernel<<<tb_grid_for(G, 256), 256, 0, st>>>(desc, G, U, rankpre, ubase, cdesc, cend, cstart);
-      ctx->launches++;
-      hs = cstart; he = cend;
-    }
+    uint2* mem = B[XB_YDCHAIN].as<uint2>(); uint32_t* heads = B[XB_BHEAD].as<uint32_t>();
+    yd_scatter_kernel<<<tb_grid_for(nwarps * 32, 128), 128, 0, st>>>(grp.bits, W, k, G, gstrand, gstart, gend, cy.in ? gseed : nullptr, blkoff, blkkey, nblk,
+                                                                     mem);
+    ctx->launches++;
     // ---- Y5: sub-chain heads ----
-    uint32_t* nsub_dev = B[XB_AGG].as<uint32_t>();   // number of sub-chains, written by the heads kernel
-    {
-      const int64_t ntiles = (n_members + YDH_TILE - 1) / YDH_TILE;
-      TB_CUDA(B[XB_YDLB].ensure(sizeof(uint64_t) * (2 * (size_t)ntiles + 8)));
-      unsigned long long* st_max = B[XB_YDLB].as<unsigned long long>();
-      unsigned long long* st_cnt = st_max + ntiles;
-      unsigned long long* ticket = st_cnt + ntiles;
-      TB_CUDA(cudaMemsetAsync(st_max, 0, sizeof(uint64_t) * (2 * (size_t)ntiles + 8), st));
-      yd_heads_kernel<<<(unsigned)ntiles, YDH_THREADS, 0, st>>>(chain, mchain, he, hs, (uint32_t)n_members, st_max, st_cnt, ticket, flag, heads, nsub_dev, work,
-                                                               g.d_status, seed);
+    TB_CUDA((tb_device_scan<OpSumU32>(ctx, HeadIn{mem}, n_members, B[XB_AGG].as<uint32_t>(), HeadOut{heads, n_members, work})));
+    if (parallel) {
+      yd_compact_kernel<<<tb_grid_for(G, 256), 256, 0, st>>>(desc, G, U, rankpre, ubase, cdesc);
       ctx->launches++;
     }
     if (parallel) {
@@ -997,23 +953,23 @@ int col_yd(tb_ctx* ctx, const ColIn& in, const ColGeom& g, const ColGroups& grp,
       const uint32_t nunits = (uint32_t)((n_members + YD_UNIT - 1) / YD_UNIT);
       TB_CUDA(B[XB_YDUNIT].ensure(sizeof(uint32_t) * ((size_t)nunits + 2)));
       uint32_t* ustart = B[XB_YDUNIT].as<uint32_t>();
-      yd_unit_kernel<<<tb_grid_for((int64_t)nunits + 1, 256), 256, 0, st>>>(heads, nsub_dev, (uint32_t)n_members, nunits, ustart);
-      (seed || cy.out ? yd_frontier_kernel<true> : yd_frontier_kernel<false>)<<<(unsigned)ctx->sm_count * 16, YD_FWARPS * 32, 0, st>>>(in, cdesc, grp.rep, chain, flag, ustart, nunits, work, U, rankpre, bm, lpad, mstart,
+      yd_unit_kernel<<<tb_grid_for((int64_t)nunits + 1, 256), 256, 0, st>>>(heads, work + 1, (uint32_t)n_members, nunits, ustart);
+      (seed || cy.out ? yd_frontier_kernel<true> : yd_frontier_kernel<false>)<<<(unsigned)ctx->sm_count * 16, YD_FWARPS * 32, 0, st>>>(in, cdesc, grp.rep, mem, ustart, nunits, work, U, rankpre, bm, lpad, mstart,
                                                                                   seed, cy.out ? cy.efin : nullptr, (uint32_t)n_members);
       ctx->launches++;
       ctx->launches += 2;
       TB_CUDA((tb_device_scan<OpMaxI64>(ctx, LastZeroIn{bm}, nblocks512, B[XB_AGG].as<long long>(), LastZeroOut{lz})));
-      yd_lookup_kernel<<<tb_grid_for(n_members, 256), 256, 0, st>>>(mstart, chain, n_members, flag, bm, lz, lpad, ydc, cy.in ? cy.ext : nullptr);
+      yd_lookup_kernel<<<tb_grid_for(n_members, 256), 256, 0, st>>>(mstart, mem, n_members, bm, lz, lpad, ydc, cy.in ? cy.ext : nullptr);
       ctx->launches++;
       pout = YdParOut{bm, lz, lpad, U, rankpre, nuw, ubase, (int64_t)cy.bout - ubase, cy.ext, cy.efin};
       if (cy.out && !cy.in) TB_CUDA(cudaMemsetAsync(cy.ext, 0, sizeof(int32_t) * (size_t)nchains, st));
     } else {
-      YdSeqCarry ca{cy.in ? cy.coff : nullptr, cy.cs, cy.ce, colbase, flag, nchains, ubase, cy.bout, cy.out ? cy.os : nullptr, cy.oe, cy.cap, cy.ometa};
+      YdSeqCarry ca{cy.in ? cy.coff : nullptr, cy.cs, cy.ce, colbase, mem, nchains, ubase, cy.bout, cy.out ? cy.os : nullptr, cy.oe, cy.cap, cy.ometa};
       const size_t smem = (size_t)YD_WARPS * 2 * YD_CAP_SMEM * 32 * sizeof(uint32_t);
       const bool carry = cy.in || cy.out;
       auto chain_smem = carry ? yd_chain_kernel<true, true> : yd_chain_kernel<true, false>;
       TB_CUDA(cudaFuncSetAttribute(chain_smem, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      chain_smem<<<(unsigned)ctx->sm_count * 4, YD_WARPS * 32, smem, st>>>(in, desc, grp.rep, chain, heads, work, ydc, nullptr, g.d_status, ca);
+      chain_smem<<<(unsigned)ctx->sm_count * 4, YD_WARPS * 32, smem, st>>>(in, desc, grp.rep, mem, heads, work, ydc, nullptr, g.d_status, ca);
       ctx->launches++;
       TB_CUDA(cudaMemcpyAsync(h_status, g.d_status, sizeof(int64_t) * 16, cudaMemcpyDeviceToHost, st));
       TB_CUDA(cudaStreamSynchronize(st));
@@ -1025,7 +981,7 @@ int col_yd(tb_ctx* ctx, const ColIn& in, const ColGeom& g, const ColGroups& grp,
         TB_CUDA(cudaMemsetAsync(work, 0, sizeof(unsigned long long), st));
         TB_CUDA(cudaMemsetAsync(g.d_status + CS_YD_OVERFLOW, 0, sizeof(long long), st));
         if (cy.out) TB_CUDA(cudaMemsetAsync(cy.ometa + 2 * nchains, 0, sizeof(long long), st));
-        (carry ? yd_chain_kernel<false, true> : yd_chain_kernel<false, false>)<<<grid2, YD_WARPS * 32, 0, st>>>(in, desc, grp.rep, chain, heads, work, ydc, B[XB_YDSCRATCH].as<uint32_t>(), g.d_status, ca);
+        (carry ? yd_chain_kernel<false, true> : yd_chain_kernel<false, false>)<<<grid2, YD_WARPS * 32, 0, st>>>(in, desc, grp.rep, mem, heads, work, ydc, B[XB_YDSCRATCH].as<uint32_t>(), g.d_status, ca);
         ctx->launches++;
         TB_CUDA(cudaMemcpyAsync(h_status, g.d_status, sizeof(int64_t) * 16, cudaMemcpyDeviceToHost, st));
         TB_CUDA(cudaStreamSynchronize(st));
@@ -1040,8 +996,10 @@ int col_yd(tb_ctx* ctx, const ColIn& in, const ColGeom& g, const ColGroups& grp,
   }
   yd_combine_kernel<<<tb_grid_for(G, 256), 256, 0, st>>>(grp.yd, ydc, G);
   ctx->launches++;
-  TB_CUDA(cudaMemcpyAsync(h_status + YS_LBFAIL, g.d_status + YS_LBFAIL, sizeof(long long), cudaMemcpyDeviceToHost, st));
-  TB_CUDA(cudaStreamSynchronize(st));
-  if (h_status[YS_LBFAIL]) { ctx->set_error("tb_collapse_window: sub-chain head scan did not make progress (internal error)"); return 1; }
+  if (n_members > 0) {   // sub-chain count for tb_last_yd_stat
+    TB_CUDA(cudaMemcpyAsync(h_status + 17, work + 1, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    TB_CUDA(cudaStreamSynchronize(st));
+    ctx->last_yd_stat[1] = h_status[17];
+  }
   return 0;
 }

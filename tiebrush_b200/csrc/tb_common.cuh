@@ -72,6 +72,7 @@ struct tb_ctx {
   int64_t launches = 0;
   int64_t last_heavy = 0;   // slots redone by the full-size tile launch in the last collapse call
   int last_yd_path = 0;     // YD stage of the last collapse call: 0 parallel (frontier + link bitmaps), 1 sequential lists
+  int64_t last_yd_stat[4] = {};   // YD stage of the last collapse call: members | sub-chains | compact length | 1024-group blocks
   int last_path = 0;        // front end of the last collapse call: 0 tile, 1 ordered (by options), 2 ordered (table overflow fallback)
   int64_t last_ord_deep = 0;   // ordered front end, last call: start positions handled by the warp kernel
   int last_cov_exact = 0;   // last coverage call took the exact ordered-double path (weights that are not multiples of 2^-20)

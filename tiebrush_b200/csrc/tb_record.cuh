@@ -195,11 +195,11 @@ enum {
   XB_BITS,       // u32 [G*W] compacted
   XB_GDESC,      // YD: group descriptors
   XB_BHEAD,      // YD: bundle heads
-  XB_YDPM,       // YD: prefix max of group ends
+  XB_YDPM,       // YD: group ends, starts and strands (genomic)
   XB_WORK,       // small device counters
   XB_YDC,        // YD: chain distances per group
   XB_YDSCRATCH,  // YD: global-memory lists of the repeat launch
-  XB_YDBLK, XB_YDCHAIN, XB_YDFLAG, XB_YDU, XB_YDKEPT, XB_YDBM, XB_YDLZ, XB_YDUNIT, XB_YDLB, XB_HEAVY,   // YD: per-block member counts, chain member lists, sub-chain head flags
+  XB_YDBLK, XB_YDCHAIN, XB_YDU, XB_YDKEPT, XB_YDBM, XB_YDLZ, XB_YDUNIT, XB_HEAVY,   // YD: per-block member counts, chain members (group id, head flag | chain)
   XB_ORD_KEY, XB_ORD_KEY2, XB_ORD_VAL, XB_ORD_VAL2, XB_ORD_REFLEN, XB_ORD_TABLE, XB_ORD_AGG,   // ordered path: merge-order sort
   XB_ORD_LIST, XB_ORD_GREP, XB_ORD_GYC, XB_ORD_GYX, XB_ORD_GYD, XB_ORD_VALID, XB_ORD_GBITS,                // ordered path: per-position group lists
   XB_META_DICT,   // u64 [256] dictionary of the packed wire format
