@@ -301,6 +301,10 @@ int64_t tb_last_yd_stat(tb_ctx*, int which);
 /* Tile slots of the last call that were redone by the full-size-table launch (pile-up positions with more distinct
  * alignments than a quarter-SM table holds). */
 int64_t tb_last_heavy_slots(tb_ctx*);
+/* Start positions of the last ordered-path call (tb_last_path() 1 or 2) handed to the one-warp-per-position kernel: those
+ * with at least TB_ORD_DEEP records (default 96, counting records the filters drop; 0 sends every position to the
+ * one-thread kernel). */
+int64_t tb_last_ord_deep(tb_ctx*);
 /* Tile kernel generation the last tile-path call launched first: 2 = col_tile2_kernel (slices staged into shared memory by
  * cp.async.bulk / mbarrier, one optimistic table per slot; needs <= 128 files and 16-byte aligned pos / cig_off / cigar
  * columns; opt-in with TB_TILE_GEN=2: exact, but measured slower than generation 1 on the C2 cohort), 1 = col_tile_kernel

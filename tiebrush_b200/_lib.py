@@ -12,7 +12,7 @@ LIB_PATH = os.path.join(HERE, "libtiebrush_b200.so")
 
 SYMBOLS = ["tb_create", "tb_destroy", "tb_last_error", "tb_set_stream", "tb_get_stream", "tb_sync",
            "tb_collapse_window", "tb_collapse_window_carry", "tc_coverage_window", "tc_sample_window", "tb_launch_count", "tb_set_profiling",
-           "tb_last_kernel_ms", "tb_version", "tb_last_path", "tb_last_yd_path", "tb_last_yd_stat", "tb_last_heavy_slots", "tb_last_tile_gen", "tb_last_tile_stat",
+           "tb_last_kernel_ms", "tb_version", "tb_last_path", "tb_last_yd_path", "tb_last_yd_stat", "tb_last_heavy_slots", "tb_last_ord_deep", "tb_last_tile_gen", "tb_last_tile_stat",
            "tc_coverage_stream", "tb_comm_unique_id", "tb_comm_init", "tb_comm_destroy", "tb_comm_rank", "tb_comm_world",
            "tc_shard_coverage", "tc_shard_coverage_gather", "tc_shard_gather", "tc_shard_stat", "tc_stream_windows", "tc_last_exact"]
 
@@ -94,6 +94,8 @@ def load():
     lib.tb_last_yd_stat.restype = C.c_int64
     lib.tb_last_heavy_slots.argtypes = [C.c_void_p]
     lib.tb_last_heavy_slots.restype = C.c_int64
+    lib.tb_last_ord_deep.argtypes = [C.c_void_p]
+    lib.tb_last_ord_deep.restype = C.c_int64
     lib.tb_last_tile_gen.argtypes = [C.c_void_p]
     lib.tb_last_tile_gen.restype = C.c_int
     lib.tb_last_tile_stat.argtypes = [C.c_void_p, C.c_int]

@@ -169,6 +169,10 @@ class Context:
     def last_heavy_slots(self):
         return int(self.lib.tb_last_heavy_slots(self.h))
 
+    def last_ord_deep(self):
+        """Ordered front end, last call: start positions handled by the one-warp-per-position kernel."""
+        return int(self.lib.tb_last_ord_deep(self.h))
+
     def last_tile_gen(self):
         """2 = TMA-staged tile kernel (col_tile2_kernel), 1 = col_tile_kernel."""
         return int(self.lib.tb_last_tile_gen(self.h))

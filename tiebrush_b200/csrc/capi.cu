@@ -96,6 +96,7 @@ int tb_last_path(tb_ctx* ctx) { return ctx ? ctx->last_path : -1; }
 int tb_last_yd_path(tb_ctx* ctx) { return ctx ? ctx->last_yd_path : -1; }
 int64_t tb_last_yd_stat(tb_ctx* ctx, int which) { return (ctx && which >= 0 && which < 4) ? ctx->last_yd_stat[which] : -1; }
 int64_t tb_last_heavy_slots(tb_ctx* ctx) { return ctx ? ctx->last_heavy : -1; }
+int64_t tb_last_ord_deep(tb_ctx* ctx) { return ctx ? ctx->last_ord_deep : -1; }
 int64_t tc_stream_windows(tb_ctx* ctx) { return ctx ? ctx->stream_windows : -1; }
 int tc_last_exact(tb_ctx* ctx) { return ctx ? ctx->last_cov_exact : -1; }
 int tb_last_tile_gen(tb_ctx* ctx) { return ctx ? ctx->last_tile_gen : -1; }
