@@ -305,15 +305,11 @@ int64_t tb_last_heavy_slots(tb_ctx*);
  * with at least TB_ORD_DEEP records (default 96, counting records the filters drop; 0 sends every position to the
  * one-thread kernel). */
 int64_t tb_last_ord_deep(tb_ctx*);
-/* Tile kernel generation the last tile-path call launched first: 2 = col_tile2_kernel (slices staged into shared memory by
- * cp.async.bulk / mbarrier, one optimistic table per slot; needs <= 128 files and 16-byte aligned pos / cig_off / cigar
- * columns; opt-in with TB_TILE_GEN=2: exact, but measured slower than generation 1 on the C2 cohort), 1 = col_tile_kernel
- * (position-partitioned tables, plain loads; the default). Results are identical; slots generation 2 defers show up in
- * tb_last_heavy_slots(). */
+/* Tile kernel generation: 1 once a tb_collapse_window call has run the tile front end (col_tile_kernel, the only
+ * generation), 0 before. */
 int tb_last_tile_gen(tb_ctx*);
-/* Generation-2 statistics of the last call: 0 slots done in several passes (more groups than one table), 1 records of the
- * deferred slots, 2 slots deferred (a pile-up of more distinct alignments at one position than the table holds, or CIGARs
- * beyond the staging area), 3 slots in all. */
+/* Tile statistics: 0, 1 and 2 are always 0; 3 is the number of slots of the last tile-path call that ran the 256-thread
+ * geometry (0 before any such call). -1 for another `which`. */
 int64_t tb_last_tile_stat(tb_ctx*, int which);
 /* Device time in ms of one stage of the last call, measured with CUDA events on the launching stream
  * (enabled by tb_set_profiling(ctx,1)):

@@ -29,10 +29,8 @@ def gpu_carry_fn(k, opts):
     return fn
 
 
-@pytest.mark.parametrize("tile", [1, 2])
 @pytest.mark.parametrize("npz,pattern", [("collapse_random.npz", 7), ("collapse_fixture.npz", "random"), ("collapse_merged.npz", "every")])
-def test_carry_goldens(npz, pattern, tile, yd_path, monkeypatch):
-    monkeypatch.setenv("TB_TILE_GEN", str(tile))
+def test_carry_goldens(npz, pattern, yd_path):
     carried = []
     for case in H.case_names(npz):
         files, opts, fm, exp = H.load_collapse_case(npz, case)

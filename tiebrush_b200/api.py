@@ -174,11 +174,12 @@ class Context:
         return int(self.lib.tb_last_ord_deep(self.h))
 
     def last_tile_gen(self):
-        """2 = TMA-staged tile kernel (col_tile2_kernel), 1 = col_tile_kernel."""
+        """1 once a collapse call has run the tile kernel (col_tile_kernel, the only generation), 0 before."""
         return int(self.lib.tb_last_tile_gen(self.h))
 
     def last_tile_stats(self):
-        """Generation-2 tile kernel, last call: slots done in several passes, records of deferred slots, deferred slots, slots."""
+        """Tile statistics: multi_pass, deferred_records and deferred_slots are always 0; slots is the slot count of the
+        last tile-path call that ran the 256-thread geometry (0 before any)."""
         return dict(zip(("multi_pass", "deferred_records", "deferred_slots", "slots"), (int(self.lib.tb_last_tile_stat(self.h, i)) for i in range(4))))
 
     def last_yd_path(self):

@@ -286,7 +286,7 @@ int tb_collapse_impl(tb_ctx* ctx, const tb_soa_in* hin, tb_groups_out* out, cons
   if (h_status[CS_ERR] == 7) { ctx->set_error("tb_collapse_window: packed wire format: meta8 holds %lld escaped entries but n_meta_ext = %lld", h_status[CS_ERRIDX], (long long)hin->n_meta_ext); return 1; }
   if (h_status[CS_ERR] == 3) { ctx->set_error("tb_collapse_window: unmapped record %lld kept by -M: the reference aborts here (GVec invalid index)", h_status[CS_ERRIDX]); return 1; }
 
-  ColGeom g; g.n = n; g.k = k; g.W = W; g.S = S; g.P = d_hist; g.d_runoff = B[XB_RUNOFF].as<long long>(); g.d_merged = d_merged; g.d_status = d_status; g.n_cig = hin->n_cig;
+  ColGeom g; g.n = n; g.k = k; g.W = W; g.S = S; g.P = d_hist; g.d_runoff = B[XB_RUNOFF].as<long long>(); g.d_merged = d_merged; g.d_status = d_status;
   ColGroups grp; memset(&grp, 0, sizeof(grp));
   grp.capacity = out->capacity;
   grp.rep = out->rep_index; grp.yc = out->yc; grp.yx = out->yx; grp.yd = out->yd;

@@ -9,7 +9,6 @@ struct ColGeom {
   const long long* d_runoff;          // [k+1] device copy of run_off
   const uint8_t* d_merged;            // [k] device copy of file_merged (or nullptr)
   long long* d_status;                // CS_* block
-  int64_t n_cig;                      // words in the CIGAR arena as the caller stated them (0 = unknown)
 };
 
 // dense group outputs of a front end, in final order

@@ -20,7 +20,6 @@
 //   epilogue   occupied entries are compacted in region (= position) order, ranked inside their position by
 //              (strand, end, mode key) with the reference's comparator, and written to the staging arrays.
 #include <limits.h>
-#include <stdlib.h>
 #include "collapse_internal.cuh"
 
 namespace {
@@ -595,28 +594,22 @@ __global__ void __launch_bounds__(128) col_compact_kernel(TileParams tp, const u
 
 __global__ void col_store_total_kernel(const uint32_t* tot, long long* status) { status[CS_NGROUPS] = *tot; }
 
-constexpr int TILE_THREADS_DEFAULT = 256;
-
-#include "collapse_tile2.cuh"
-constexpr int TILE2_THREADS = 512;
-
 }  // namespace
 
 int col_front_tile(tb_ctx* ctx, const ColIn& in, const ColGeom& g, ColGroups& out, int64_t* n_groups, int64_t* n_kept) {
   cudaStream_t st = ctx->stream;
   DevBuf* B = ctx->buf;
   const int64_t n = g.n; const int k = g.k; const uint32_t W = g.W, S = g.S;
-  // ---- geometry: CTAs of `threads` threads, 1024/threads of them per SM, each with an equal share of the opt-in
-  // shared memory for its table (TB_TILE_THREADS=256|512|1024 overrides the default for experiments) ----
-  int threads = TILE_THREADS_DEFAULT;
-  if (const char* e = getenv("TB_TILE_THREADS")) { const int t = atoi(e); if (t == 128 || t == 256 || t == 512 || t == 1024) threads = t; }
+  // ---- geometry: CTAs of 256 threads, 4 of them per SM, each with a quarter of the opt-in shared memory for its table;
+  // one 1024-thread CTA per SM when the 256-thread table does not fit k ----
+  int threads = 256;
   const int ctas_per_sm = 1024 / threads;
   const size_t smem_sm = ctx->smem_optin ? ctx->smem_optin + 1024 : 233472;   // shared memory per SM (opt-in per block + 1 KB reserved)
   const size_t smem_limit = smem_sm / ctas_per_sm - 1024 - 512;               // per CTA: minus the reserved KB and the static part
   uint32_t E = 8192;   // region bases are u16 and the match key keeps 13 bits for the entry
   while (E > 64 && tile_smem_bytes((uint32_t)k, E, W) > smem_limit) E -= 64;
   if (tile_smem_bytes((uint32_t)k, E, W) > smem_limit) {
-    if (threads != 1024) { threads = 1024; }   // fall through to the single-CTA geometry below
+    threads = 1024;   // fall through to the single-CTA geometry below
     const size_t lim1 = smem_sm - 1024 - 512;
     E = 8192;
     while (E > 64 && tile_smem_bytes((uint32_t)k, E, W) > lim1) E -= 64;
@@ -628,41 +621,13 @@ int col_front_tile(tb_ctx* ctx, const ColIn& in, const ColGeom& g, ColGroups& ou
   uint32_t E_full = 8192;
   while (E_full > 64 && tile_smem_bytes((uint32_t)k, E_full, W) > lim_full) E_full -= 64;
   const uint32_t cap_full = (uint32_t)(((uint64_t)(E_full - 1) * 4) / 5);
-  // ---- generation 2 (col_tile2_kernel): slices staged by the TMA unit, one optimistic table per slot. Needs k <= 128
-  // (one producer thread per file in the first four warps, 7 bits of the match key), 16-byte aligned pos / cig_off / cigar
-  // columns (cp.async.bulk) and a slot of a few hundred records at least. TB_TILE_GEN=1 forces generation 1. ----
-  bool gen2 = k <= 128 && !ctx->tile2_off && threads != 1024 && tile_smem_bytes((uint32_t)k, E_full, W) <= lim_full &&
-              (((uintptr_t)in.pos | (uintptr_t)in.cig_off | (uintptr_t)in.cigar) & 15u) == 0 && g.n_cig > 0 && g.n_cig < (1LL << 32);
-  // Measured (profiles/r02a_*): generation 2 is exact but NOT faster on the C2 cohort (69-80 ms against 55.6 ms for the tile
-  // stage at 1e9 alignments): its table (1024 entries beside the staging area) is too small for the pile-up positions that
-  // hold a quarter of the records, and the instruction count per record did not drop. It stays opt-in: TB_TILE_GEN=2.
-  { const char* e = getenv("TB_TILE_GEN"); if (!e || atoi(e) != 2) gen2 = false; }
-  uint32_t T2 = 0, rs_cap = 0, cw_cap = 0;
-  const uint32_t E2g = 1024, logE2g = 10, arena2 = tile2_arena_words(E2g, in.mode);
-  if (gen2) {
-    const size_t lim2 = smem_sm / 2 - 1024 - 1024;
-    uint32_t t = 8128;
-    if (t > cap_full) t = cap_full & ~63u;
-    for (; t >= 256; t -= 64) {
-      rs_cap = (t + 7u * (uint32_t)k + 8u + 3u) & ~3u;
-      cw_cap = (t * 13u / 4u + 6u * (uint32_t)k + 8u + 3u) & ~3u;
-      if (tile2_smem_bytes((uint32_t)k, E2g, W, t, rs_cap, cw_cap, arena2) <= lim2) break;
-    }
-    if (t >= 256) T2 = t; else gen2 = false;
-  }
   // slot size: a slot holds < T records of ordinary positions plus its last position; a slot that outgrows the table
   // splits that last position off as a pile-up sub-tile (tile kernel), so any T <= cap_records is correct. Larger T =
-  // fewer, fuller slots (less per-slot work), but more slots that need the split. TB_TILE_T8 = T in eighths of the table.
-  uint32_t t8 = 7;
-  if (const char* e = getenv("TB_TILE_T8")) { const int t = atoi(e); if (t >= 1 && t <= 8) t8 = (uint32_t)t; }
-  uint32_t T = (uint32_t)(((uint64_t)cap_records * t8) / 8);
-  if (gen2) {
-    T = T2;
-    if (const char* e = getenv("TB_TILE2_T")) { const int t = atoi(e); if (t >= 64 && (uint32_t)t <= T2) T = (uint32_t)t; }
-  }
+  // fewer, fuller slots (less per-slot work), but more slots that need the split; 7/8 of the table.
+  const uint32_t T = (uint32_t)(((uint64_t)cap_records * 7) / 8);
   if (T < 8) { ctx->set_error("tb_collapse_window: %d samples leave no room for a shared-memory tile", k); return 1; }
   const uint32_t M = (uint32_t)((n + T - 1) / T);
-  ctx->last_tile_gen = gen2 ? 2 : 1;
+  ctx->last_tile_gen = 1;
 
   TB_CUDA(B[XB_SLOTPOS].ensure(sizeof(uint32_t) * ((size_t)M + 2)));
   TB_CUDA(B[XB_OFF].ensure(sizeof(uint32_t) * ((size_t)M + 1) * k));
@@ -689,8 +654,7 @@ int col_front_tile(tb_ctx* ctx, const ColIn& in, const ColGeom& g, ColGroups& ou
   tp.gcount = B[XB_GCOUNT].as<uint32_t>(); tp.st_rep = B[XB_ST_REP].as<uint32_t>(); tp.st_yc = B[XB_ST_YC].as<float>();
   tp.st_yx = B[XB_ST_YX].as<uint32_t>(); tp.st_bits = B[XB_ST_BITS].as<uint32_t>(); tp.status = g.d_status; tp.seed = 0x243F6A8885A308D3ULL;
   tp.slot_counter = B[XB_WORK].as<unsigned int>();
-  tp.heavy_records = 24u * E;   // TB_TILE_HEAVY_RECORDS overrides (0 = never shortcut)
-  if (const char* e = getenv("TB_TILE_HEAVY_RECORDS")) tp.heavy_records = (uint32_t)atol(e);
+  tp.heavy_records = 24u * E;
   auto launch = [&](int thr, const TileParams& t, unsigned nslots) -> cudaError_t {
     const size_t smem = tile_smem_bytes((uint32_t)k, t.ecap, W);
     const unsigned want = (unsigned)ctx->sm_count * (1024u / (unsigned)thr);
@@ -704,8 +668,6 @@ int col_front_tile(tb_ctx* ctx, const ColIn& in, const ColGeom& g, ColGroups& ou
   } while (0)
     const bool dflt = in.mode == TB_MODE_CIGAR;
     if (thr == 1024) { if (dflt) TB_TILE_LAUNCH(1024, TB_MODE_CIGAR); else TB_TILE_LAUNCH(1024, -1); }
-    else if (thr == 512) { if (dflt) TB_TILE_LAUNCH(512, TB_MODE_CIGAR); else TB_TILE_LAUNCH(512, -1); }
-    else if (thr == 128) { if (dflt) TB_TILE_LAUNCH(128, TB_MODE_CIGAR); else TB_TILE_LAUNCH(128, -1); }
     else {   // the default geometry has one instantiation per merge strategy
       switch (in.mode) {
         case TB_MODE_CIGAR: TB_TILE_LAUNCH(256, TB_MODE_CIGAR); break;
@@ -719,51 +681,22 @@ int col_front_tile(tb_ctx* ctx, const ColIn& in, const ColGeom& g, ColGroups& ou
     ctx->launches++;
     return cudaGetLastError();
   };
-  // launch 1: every slot — generation 2 (TMA-staged slices, one optimistic table per slot) or generation 1 (small
-  // position-partitioned tables, several CTAs per SM). Slots it cannot finish (a pile-up position with more distinct
-  // alignments than the table holds; generation 2: anything irregular) go to the heavy list; launch 2 redoes those slots
-  // with generation 1's full-size table, one CTA per SM.
-  if (threads != 1024 || gen2) {
+  // launch 1: every slot, small position-partitioned tables, several CTAs per SM. Slots it cannot finish (a pile-up position
+  // with more distinct alignments than the table holds) go to the heavy list; launch 2 redoes those slots with the
+  // full-size table, one CTA per SM. With the single-CTA geometry launch 1 already has the full-size table.
+  if (threads != 1024) {
     TB_CUDA(B[XB_HEAVY].ensure(sizeof(uint32_t) * ((size_t)M + 1)));
     tp.heavy_list = B[XB_HEAVY].as<uint32_t>();
   }
   long long* h_status = ctx->pinned[0].as<long long>();
   if (ctx->profiling) TB_CUDA(cudaEventRecord(ctx->ev[0], st));
-  if (gen2) {
-    Tile2Params t2p; memset(&t2p, 0, sizeof(t2p));
-    t2p.M = M; t2p.E = E2g; t2p.logE = logE2g; t2p.W = W; t2p.T = T; t2p.rs_cap = rs_cap; t2p.cw_cap = cw_cap; t2p.arena = arena2; t2p.k = (uint32_t)k;
-    t2p.P = g.P; t2p.slotpos = tp.slotpos; t2p.off = tp.off; t2p.gcount = tp.gcount; t2p.st_rep = tp.st_rep; t2p.st_yc = tp.st_yc;
-    t2p.st_yx = tp.st_yx; t2p.st_bits = tp.st_bits; t2p.status = tp.status; t2p.slot_counter = tp.slot_counter; t2p.seed = 0x85A308D3u;
-    t2p.heavy_list = tp.heavy_list; t2p.n = (uint32_t)n; t2p.n_cig = (uint32_t)g.n_cig;
-    const size_t smem2 = tile2_smem_bytes((uint32_t)k, E2g, W, T2, rs_cap, cw_cap, arena2);
-    const unsigned want = (unsigned)ctx->sm_count * (1024u / TILE2_THREADS);
-    const unsigned grid = M < want ? M : want;
-    TB_CUDA(cudaMemsetAsync(tp.slot_counter, 0, 64, st));
-#define TB_TILE2_LAUNCH(MODE)                                                                                                          \
-  do {                                                                                                                                 \
-    TB_CUDA(cudaFuncSetAttribute(col_tile2_kernel<TILE2_THREADS, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));     \
-    col_tile2_kernel<TILE2_THREADS, MODE><<<grid, TILE2_THREADS, smem2, st>>>(in, t2p);                                               \
-  } while (0)
-    switch (in.mode) {
-      case TB_MODE_CIGAR: TB_TILE2_LAUNCH(TB_MODE_CIGAR); break;
-      case TB_MODE_FULL: TB_TILE2_LAUNCH(TB_MODE_FULL); break;
-      case TB_MODE_CLIP: TB_TILE2_LAUNCH(TB_MODE_CLIP); break;
-      default: TB_TILE2_LAUNCH(TB_MODE_EXON); break;
-    }
-#undef TB_TILE2_LAUNCH
-    ctx->launches++;
-    TB_CUDA(cudaGetLastError());
-  } else {
-    TB_CUDA(launch(threads, tp, M));
-  }
+  TB_CUDA(launch(threads, tp, M));
   if (tp.heavy_list) {
     TB_CUDA(cudaMemcpyAsync(h_status, g.d_status, sizeof(int64_t) * 16, cudaMemcpyDeviceToHost, st));
     TB_CUDA(cudaStreamSynchronize(st));
     const int64_t nheavy = h_status[CS_NHEAVY];
     ctx->last_heavy = nheavy;
-    ctx->last_tile_stat[0] = h_status[CS_T2_MULTI]; ctx->last_tile_stat[1] = h_status[CS_T2_STAGE]; ctx->last_tile_stat[2] = h_status[CS_T2_TABLE];
-    ctx->last_tile_stat[3] = (int64_t)M;
-    if (gen2 && M >= 64 && nheavy > (int64_t)(M / 4)) ctx->tile2_off = 1;   // few duplicates: the optimistic table does not pay
+    ctx->last_tile_slots = (int64_t)M;
     if (nheavy > 0 && !h_status[CS_TABLE_OVERFLOW]) {
       TileParams t2 = tp;
       t2.ecap = E_full; t2.cap_records = cap_full;

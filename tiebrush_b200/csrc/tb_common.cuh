@@ -76,9 +76,8 @@ struct tb_ctx {
   int last_path = 0;        // front end of the last collapse call: 0 tile, 1 ordered (by options), 2 ordered (table overflow fallback)
   int64_t last_ord_deep = 0;   // ordered front end, last call: start positions handled by the warp kernel
   int last_cov_exact = 0;   // last coverage call took the exact ordered-double path (weights that are not multiples of 2^-20)
-  int last_tile_gen = 0;    // tile kernel generation of the last collapse call: 2 = TMA-staged slices (col_tile2_kernel), 1 = col_tile_kernel
-  int64_t last_tile_stat[4] = {};   // generation 2, last call: slots done in several passes | deferred (staging area) | deferred (table / pile-up) | slots
-  int tile2_off = 0;        // sticky: a call deferred more than a quarter of its slots (few duplicates) -> later calls use generation 1
+  int last_tile_gen = 0;    // 1 once a collapse call has run the tile kernel (col_tile_kernel)
+  int64_t last_tile_slots = 0;   // slots of the last tile-path call that used the heavy list (256-thread geometry)
   std::string err;
   DevBuf buf[TB_NBUF];   // workspace slots (see the enum in each pipeline)
   DevBuf in_stage[20];   // device copies of host input arrays

@@ -210,8 +210,7 @@ enum {
 };
 static_assert(XB_COUNT_ <= TB_NBUF, "raise TB_NBUF");
 
-enum { CS_ERR = 0, CS_ERRIDX, CS_NKEPT, CS_NGROUPS, CS_TABLE_OVERFLOW, CS_NBUNDLES, CS_YD_OVERFLOW, CS_NHEAVY, CS_N_,
-       CS_T2_STAGE = 13, CS_T2_TABLE = 14, CS_T2_MULTI = 15 };   // 8-10: YD (YS_*); 13-15: generation-2 tile kernel statistics (slots deferred because they do not fit the staging area / the table; slots done in several passes)
+enum { CS_ERR = 0, CS_ERRIDX, CS_NKEPT, CS_NGROUPS, CS_TABLE_OVERFLOW, CS_NBUNDLES, CS_YD_OVERFLOW, CS_NHEAVY, CS_N_ };   // 8-10: YD (YS_*)
 enum { ERR_POS_RANGE = 1, ERR_UNSORTED = 2 };
 
 static inline unsigned tb_grid_for(int64_t n, int threads) { return (unsigned)((n + threads - 1) / threads); }
