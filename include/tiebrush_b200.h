@@ -283,6 +283,47 @@ int64_t tc_stream_windows(tb_ctx*);
  * (tiecov.cpp:194-223, :100-112) instead of in 2^-20 fixed point. */
 int tc_last_exact(tb_ctx*);
 
+/* ---- tiecov straight from BAM bytes: BGZF inflate and record parse on the device ------------ */
+/* One chunk of a BAM file (SAM spec §4.1-4.2): BGZF blocks, each a gzip member with the BC extra subfield. The chunk may
+ * end inside a block or inside a record: what is incomplete at its end is left for the next call, which starts at
+ * tb_bgzf_stat.resume_byte of this chunk with skip = resume_skip (the caller re-sends those bytes). */
+typedef struct {
+  const uint8_t* data;  /* BGZF bytes, HOST memory; copied to the device on the context's stream                          */
+  int64_t n_bytes;
+  int64_t skip;         /* inflated bytes of the first block that are not records (the header, or records already decoded) */
+  int32_t first;        /* tc_coverage_bam: 1 = a new stream (drops any records held from an earlier call)                  */
+  int32_t last;         /* 1 = nothing follows: an incomplete block or record at the end is an error                        */
+} tb_bgzf_in;
+
+typedef struct {        /* out */
+  int64_t blocks, bytes_in, bytes_out;   /* complete BGZF blocks of the chunk, their compressed and inflated bytes             */
+  int64_t records, unmapped;             /* records decoded from the chunk: mapped ones (the columns) and dropped flag-0x4 ones */
+  int64_t resume_byte;  /* offset in data of the block the next call starts with (n_bytes: everything consumed)             */
+  int64_t resume_skip;  /* the `skip` of that call                                                                          */
+  int64_t need_rows;    /* tc_coverage_bam: capacity its runs / sample_rows need (junctions: half of it); see return 5      */
+} tb_bgzf_stat;
+
+/* Decodes the complete records of one chunk into device columns owned by the context, valid until the next
+ * tc_bam_columns / tc_coverage_bam call: cols->on_device = 1, n, tid, pos, end (pos + reference length of the CIGAR),
+ * yc ((float)bam_aux2f of YC, 1 when absent), strand (spliceStrand: XS, else ts flipped on flag 0x10), cig_off, cigar,
+ * n_cig; *yx = device YX column (bam_aux2i, 1 when absent). Unmapped records (flag 0x4) are dropped and counted; a mapped
+ * record with refID < 0, an aux field past its record, a CG tag (CIGAR stored in the tag) and every BGZF / DEFLATE defect
+ * (bad header, invalid code, distance before the block start, length or CRC32 mismatch) return non-zero with a message that
+ * names the block's byte offset in `data` (and the record's inflated offset). The context stays usable. Stage times:
+ * tb_last_kernel_ms 10 (inflate) and 11 (record boundaries and parse). */
+int tc_bam_columns(tb_ctx*, const tb_bgzf_in* in, tc_soa_in* cols, const int32_t** yx, tb_bgzf_stat* st);
+
+/* tiecov over a BAM stream fed chunk by chunk (the records after the header: in->skip of the first call is where they
+ * start). Writes, from index 0, the rows of the bundles this chunk closes: runs (-c), juncs (-j), sample_rows (-s, rows of
+ * tc_sample_window); any may be NULL, not all. The open bundle at the end of the chunk is held on the device for the next
+ * call and flushed when in->last. Concatenated over the calls the rows equal, row for row, those of tc_coverage_stream /
+ * tc_sample_window over the columns of the whole file, whatever the chunk sizes: this runs tc_coverage_stream's windows
+ * (cut at bundle heads, at most `window` records) over the decoded columns. Returns 2 for the CIGARs tiecov refuses (as
+ * tc_coverage_window), 5 when a capacity is below st->need_rows (junctions: need_rows / 2): nothing was consumed, and the
+ * same call may be repeated with larger arrays. */
+int tc_coverage_bam(tb_ctx*, const tb_bgzf_in* in, int64_t window, tc_runs_out* runs, tc_juncs_out* juncs,
+                    tc_runs_out* sample_rows, tb_bgzf_stat* st);
+
 /* ---- measurement helpers ------------------------------------------------------------------ */
 /* Kernels launched by this library since the context was created (for bench.py's gpu_launches). */
 int64_t tb_launch_count(tb_ctx*);
@@ -318,6 +359,7 @@ int64_t tb_last_tile_stat(tb_ctx*, int which);
  *   4 collapse C6 compaction               5 collapse C7 YD (descriptors, bundles, chains)
  *   6 coverage K6 bundles                  7 coverage K8 runs      8 coverage K9 junction extraction
  *   9 tc_shard_coverage: halo exchange (allgathers + send / receive of the lead records)
+ *  10 tc_bam_columns / tc_coverage_bam: BGZF inflate + CRC32     11 ... record boundaries, parse and column placement
  * After tc_coverage_stream / tc_shard_coverage, 1, 6 and 7 are sums over the windows of the call. */
 int   tb_set_profiling(tb_ctx*, int on);
 float tb_last_kernel_ms(tb_ctx*, int which);

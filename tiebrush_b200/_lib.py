@@ -14,7 +14,8 @@ SYMBOLS = ["tb_create", "tb_destroy", "tb_last_error", "tb_set_stream", "tb_get_
            "tb_collapse_window", "tb_collapse_window_carry", "tc_coverage_window", "tc_sample_window", "tb_launch_count", "tb_set_profiling",
            "tb_last_kernel_ms", "tb_version", "tb_last_path", "tb_last_yd_path", "tb_last_yd_stat", "tb_last_heavy_slots", "tb_last_ord_deep", "tb_last_tile_gen", "tb_last_tile_stat",
            "tc_coverage_stream", "tb_comm_unique_id", "tb_comm_init", "tb_comm_destroy", "tb_comm_rank", "tb_comm_world",
-           "tc_shard_coverage", "tc_shard_coverage_gather", "tc_shard_gather", "tc_shard_stat", "tc_stream_windows", "tc_last_exact"]
+           "tc_shard_coverage", "tc_shard_coverage_gather", "tc_shard_gather", "tc_shard_stat", "tc_stream_windows", "tc_last_exact",
+           "tc_bam_columns", "tc_coverage_bam"]
 
 
 class SoaIn(C.Structure):
@@ -52,6 +53,15 @@ class RunsOut(C.Structure):
 class JuncsOut(C.Structure):
     _fields_ = [("capacity", C.c_int64), ("n_juncs", C.c_int64), ("tid", C.c_void_p), ("start", C.c_void_p),
                 ("end", C.c_void_p), ("strand", C.c_void_p), ("value", C.c_void_p), ("on_device", C.c_int32)]
+
+
+class BgzfIn(C.Structure):
+    _fields_ = [("data", C.c_void_p), ("n_bytes", C.c_int64), ("skip", C.c_int64), ("first", C.c_int32), ("last", C.c_int32)]
+
+
+class BgzfStat(C.Structure):
+    _fields_ = [("blocks", C.c_int64), ("bytes_in", C.c_int64), ("bytes_out", C.c_int64), ("records", C.c_int64), ("unmapped", C.c_int64),
+                ("resume_byte", C.c_int64), ("resume_skip", C.c_int64), ("need_rows", C.c_int64)]
 
 
 _lib = None
@@ -114,5 +124,7 @@ def load():
     lib.tc_stream_windows.argtypes = [C.c_void_p]
     lib.tc_stream_windows.restype = C.c_int64
     lib.tc_last_exact.argtypes = [C.c_void_p]
+    lib.tc_bam_columns.argtypes = [C.c_void_p, C.POINTER(BgzfIn), C.POINTER(CovIn), C.POINTER(C.c_void_p), C.POINTER(BgzfStat)]
+    lib.tc_coverage_bam.argtypes = [C.c_void_p, C.POINTER(BgzfIn), C.c_int64, C.POINTER(RunsOut), C.POINTER(JuncsOut), C.POINTER(RunsOut), C.POINTER(BgzfStat)]
     _lib = lib
     return lib

@@ -511,6 +511,174 @@ def _shard_coverage_gather(self, segs, window, out, all_out, cap_runs_all, cap_j
     return res
 
 
+# ---------------------------------------------------------------------------------------------------------------------
+# tiecov straight from BAM bytes (csrc/bgzf.cu): BGZF inflate and record parse on the device
+# ---------------------------------------------------------------------------------------------------------------------
+def _bgzf_blocks(f):
+    """(byte offset, inflated bytes) of every BGZF block of an open binary file, from its current position (host zlib)."""
+    import struct
+    import zlib
+    off = f.tell()
+    while True:
+        hdr = f.read(12)
+        if not hdr:
+            return
+        if len(hdr) < 12 or hdr[:4] != b"\x1f\x8b\x08\x04":
+            raise TieBrushError(f"BGZF block at byte offset {off}: bad gzip header")
+        xlen = struct.unpack_from("<H", hdr, 10)[0]
+        extra = f.read(xlen)
+        bsize, x = None, 0
+        while x + 4 <= len(extra):
+            slen = struct.unpack_from("<H", extra, x + 2)[0]
+            if extra[x:x + 2] == b"BC" and slen == 2:
+                bsize = struct.unpack_from("<H", extra, x + 4)[0]
+            x += 4 + slen
+        if bsize is None:
+            raise TieBrushError(f"BGZF block at byte offset {off}: no BC subfield")
+        body = f.read(bsize + 1 - 12 - xlen)
+        yield off, zlib.decompress(body[:-8], -15)
+        off += bsize + 1
+
+
+def read_bam_header(path):
+    """The header of a BAM file, read with zlib on the host: dict(text, names, lengths, n_samples, block_offset, skip).
+    n_samples counts the `@CO\tSAMPLE:` lines of a TieBrush-made header (what tiecov -s normalises by); the records start
+    `skip` inflated bytes into the BGZF block at byte `block_offset`: the tb_bgzf_in of the first chunk."""
+    import struct
+    buf = bytearray()
+    with open(path, "rb") as f:
+        for off, data in _bgzf_blocks(f):
+            start = len(buf)
+            buf += data
+            if len(buf) < 12:
+                continue
+            if bytes(buf[:4]) != b"BAM\1":
+                raise TieBrushError(f"{path}: not a BAM file")
+            l_text = struct.unpack_from("<i", buf, 4)[0]
+            o = 8 + l_text
+            if len(buf) < o + 4:
+                continue
+            n_ref = struct.unpack_from("<i", buf, o)[0]
+            o += 4
+            names, lengths = [], []
+            for _ in range(n_ref):
+                if len(buf) < o + 4:
+                    break
+                ln = struct.unpack_from("<i", buf, o)[0]
+                if len(buf) < o + 8 + ln:
+                    break
+                names.append(bytes(buf[o + 4:o + 3 + ln]).decode())
+                lengths.append(struct.unpack_from("<i", buf, o + 4 + ln)[0])
+                o += 8 + ln
+            if len(names) < n_ref:
+                continue
+            text = bytes(buf[8:8 + l_text]).rstrip(b"\0").decode()
+            if o < len(buf):
+                block_offset, skip = off, o - start
+            else:                      # the header fills its last block: the records start with the next one
+                block_offset, skip = f.tell(), 0
+            n_samples = sum(1 for ln in text.split("\n") if ln.startswith("@CO\tSAMPLE:"))
+            return dict(text=text, names=names, lengths=lengths, n_samples=n_samples, block_offset=block_offset, skip=skip)
+    raise TieBrushError(f"{path}: the file ends inside the BAM header")
+
+
+def _bgzf_in(data, skip, first, last):
+    buf = np.frombuffer(data, np.uint8) if len(data) else np.zeros(1, np.uint8)
+    return _lib.BgzfIn(buf.ctypes.data, len(data), int(skip), int(first), int(last)), buf
+
+
+def _stat(st):
+    return {k: int(getattr(st, k)) for k, _ in _lib.BgzfStat._fields_}
+
+
+class _DevArray:   # a device pointer as a torch-importable array (zero copy; cloned at once)
+    def __init__(self, ptr, n, typestr):
+        self.__cuda_array_interface__ = dict(shape=(n,), typestr=typestr, data=(ptr or 0, False), version=2)
+
+
+def _bam_columns(self, data, skip=0, last=True):
+    """tc_bam_columns: the tiecov columns of the complete records in `data` (bytes of whole or partial BGZF blocks; the
+    records start `skip` inflated bytes into the first block) as torch tensors on this context's device (copies: the
+    library's buffers are reused by the next call). Returns (cols, stat); stat["resume_byte"] / ["resume_skip"] tell where
+    the next chunk starts."""
+    import torch
+    bi, keep = _bgzf_in(data, skip, 1, last)
+    cin, yx, st = _lib.CovIn(), C.c_void_p(), _lib.BgzfStat()
+    if self.lib.tc_bam_columns(self.h, C.byref(bi), C.byref(cin), C.byref(yx), C.byref(st)) != 0:
+        raise TieBrushError(self._err())
+    n = int(cin.n)
+    dev = torch.device("cuda", self.device)
+    with torch.cuda.device(dev):
+        t = lambda p, m, ts: torch.as_tensor(_DevArray(p, m, ts), device=dev).clone() if m else torch.empty(0, dtype={"<i4": torch.int32, "<f4": torch.float32, "|u1": torch.uint8}[ts], device=dev)
+        cols = dict(tid=t(cin.tid, n, "<i4"), pos=t(cin.pos, n, "<i4"), end=t(cin.end, n, "<i4"), yc=t(cin.yc, n, "<f4"), yx=t(yx.value, n, "<i4"),
+                    strand=t(cin.strand, n, "|u1"), cig_off=t(cin.cig_off, n + 1, "<i4"), cigar=t(cin.cigar, int(cin.n_cig), "<i4"))
+    cols["n_cig"] = int(cin.n_cig)
+    return cols, _stat(st)
+
+
+def _coverage_bam(self, path, want_runs=True, want_juncs=True, want_sample=False, chunk_bytes=16 << 20, window=1 << 22):
+    """tiecov -c / -j / -s of a BAM file, read in chunks of `chunk_bytes` and decoded on the device (tc_coverage_bam).
+    Returns dict(runs, juncs, n_runs, n_juncs) like coverage_window, plus sample=(tid, start0, end0, ival) when want_sample
+    (the rows of sample_window), header (read_bam_header) and stat (totals over the chunks)."""
+    hdr = read_bam_header(path)
+    parts = dict(r=[], j=[], s=[])
+    totals = dict(blocks=0, bytes_in=0, bytes_out=0, records=0, unmapped=0, chunks=0)
+    cap = 1 << 16
+    out = srow = None
+    with open(path, "rb") as f:
+        f.seek(hdr["block_offset"])
+        pending, skip, first, eof = b"", hdr["skip"], 1, False
+        while True:
+            new = b"" if eof else f.read(chunk_bytes)
+            eof = eof or len(new) < chunk_bytes
+            data = pending + new
+            last = eof
+            while True:
+                if out is None:
+                    out = cov_out_buffers(cap, cap)
+                    srow = cov_out_buffers(cap, 1)
+                runs, juncs = _out_structs(out)
+                sr, _ = _out_structs(srow)
+                bi, keep = _bgzf_in(data, skip, first, last)
+                st = _lib.BgzfStat()
+                rc = self.lib.tc_coverage_bam(self.h, C.byref(bi), int(window), C.byref(runs) if want_runs else None,
+                                              C.byref(juncs) if want_juncs else None, C.byref(sr) if want_sample else None, C.byref(st))
+                if rc == 5:
+                    cap = max(2 * cap, int(st.need_rows))
+                    out = None
+                    continue
+                if rc == 2:
+                    raise ValueError(self._err())
+                if rc != 0:
+                    raise TieBrushError(self._err())
+                break
+            r, j, ns = int(runs.n_runs), int(juncs.n_juncs), int(sr.n_runs)
+            if r:
+                parts["r"].append(tuple(out[k][:r].copy() for k in ("r_tid", "r_start", "r_end", "r_val")))
+            if j:
+                parts["j"].append(tuple(out[k][:j].copy() for k in ("j_tid", "j_start", "j_end", "j_strand", "j_val")))
+            if ns:
+                parts["s"].append(tuple(srow[k][:ns].copy() for k in ("r_tid", "r_start", "r_end", "r_val")))
+            s = _stat(st)
+            for k in ("blocks", "bytes_in", "bytes_out", "records", "unmapped"):
+                totals[k] += s[k]
+            totals["chunks"] += 1
+            first = 0
+            if last:
+                break
+            pending, skip = data[s["resume_byte"]:], s["resume_skip"]
+    cat = lambda xs, dts: tuple(np.concatenate([x[i] for x in xs]) if xs else np.zeros(0, dt) for i, dt in enumerate(dts))
+    runs = cat(parts["r"], (np.int32, np.int32, np.int32, np.float64))
+    juncs = cat(parts["j"], (np.int32, np.int32, np.int32, np.uint8, np.float64))
+    res = dict(runs=runs, juncs=juncs, n_runs=len(runs[0]), n_juncs=len(juncs[0]), header=hdr, stat=totals)
+    if want_sample:
+        t, s0, e0, v = cat(parts["s"], (np.int32, np.int32, np.int32, np.float64))
+        res["sample"] = (t, s0, e0, v.astype(np.uint64))
+    return res
+
+
+Context.bam_columns = _bam_columns
+Context.coverage_bam = _coverage_bam
 Context.coverage_stream = _coverage_stream
 Context.shard_coverage_gather = _shard_coverage_gather
 Context.comm_init = _comm_init

@@ -74,6 +74,8 @@ void tb_destroy(tb_ctx* ctx) {
   for (auto& b : ctx->out_stage) b.release();
   for (auto& b : ctx->pinned) b.release();
   for (auto& b : ctx->shard_buf) b.release();
+  for (auto& b : ctx->bam_buf) b.release();
+  ctx->bam_pinned.release();
   tb_comm_destroy(ctx);
   if (ctx->gather_stream) cudaStreamDestroy(ctx->gather_stream);
   for (int i = 0; i < 16; ++i) if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);

@@ -258,8 +258,9 @@ static int gather_round(tb_ctx* ctx, GatherState& gs, const tc_runs_out* runs, c
 // One stream slice in windows cut at bundle heads. `skip` leading records are not processed (they belong to a bundle that
 // another rank owns). next = {tid, pos} of the record that follows the slice in the stream (host values), or NULL.
 // Outputs are appended to runs / juncs (n_runs / n_juncs on entry = rows already there). *consumed = records processed.
+// yx (tc_coverage_bam): the YX column of `in`; runs then receives the sample heat-map rows (tc_sample_window) and juncs is NULL.
 int tc_stream_impl(tb_ctx* ctx, const tc_soa_in* in, int64_t skip, int64_t window, const int32_t* next, tc_runs_out* runs, tc_juncs_out* juncs, int64_t* consumed,
-                   const std::function<int()>* after_window = nullptr) {
+                   const std::function<int()>* after_window = nullptr, const int32_t* yx = nullptr) {
   TB_CUDA(cudaSetDevice(ctx->device));
   const int64_t n = in->n;
   if (window < 1024) window = 1024;
@@ -298,7 +299,7 @@ int tc_stream_impl(tb_ctx* ctx, const tc_soa_in* in, int64_t skip, int64_t windo
         j.tid = juncs->tid + juncs->n_juncs; j.start = juncs->start + juncs->n_juncs; j.end = juncs->end + juncs->n_juncs;
         j.strand = juncs->strand + juncs->n_juncs; j.value = juncs->value + juncs->n_juncs;
       }
-      const int rc = tc_coverage_impl(ctx, &sub, runs ? &r : nullptr, juncs ? &j : nullptr, nullptr, &ext);
+      const int rc = tc_coverage_impl(ctx, &sub, runs ? &r : nullptr, juncs ? &j : nullptr, yx ? yx + w0 : nullptr, &ext);
       if (rc == 3) {   // one bundle spans the window
         if (w1 >= n) { *consumed = w0; goto done; }   // ... and the slice: the caller joins it with what follows
         wlen = std::min(wlen * 2, n - w0);

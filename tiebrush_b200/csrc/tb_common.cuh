@@ -51,7 +51,7 @@ struct HostBuf {  // grow-only pinned host buffer
   template <class T> T* as() { return (T*)p; }
 };
 
-enum { TB_NBUF = 52 };
+enum { TB_NBUF = 52, TB_NBAMBUF = 28 };
 
 struct tb_ctx {
   int device = 0;
@@ -89,6 +89,13 @@ struct tb_ctx {
   DevBuf shard_buf[16];
   int64_t shard_stat[8] = {};   // lead records received | sent | ranks received from | bytes sent (halo) | seam records | bytes moved by the gather
   int64_t stream_windows = 0;   // windows of the last tc_coverage_stream / tc_shard_coverage call
+  // BAM decode (bgzf.cu): workspace, and the bundle tc_coverage_bam holds for its next call: records [bam_from, bam_from +
+  // bam_held) of column set bam_set, whose CIGAR words start at bam_cbase (bam_hcig words)
+  DevBuf bam_buf[TB_NBAMBUF];
+  HostBuf bam_pinned;
+  int bam_set = 0;
+  int64_t bam_from = 0, bam_held = 0;
+  uint32_t bam_cbase = 0, bam_hcig = 0;
   void set_error(const char* fmt, ...);
 };
 
