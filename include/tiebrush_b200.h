@@ -349,8 +349,10 @@ int64_t tb_last_ord_deep(tb_ctx*);
 /* Tile kernel generation: 1 once a tb_collapse_window call has run the tile front end (col_tile_kernel, the only
  * generation), 0 before. */
 int tb_last_tile_gen(tb_ctx*);
-/* Tile statistics: 0, 1 and 2 are always 0; 3 is the number of slots of the last tile-path call that ran the 256-thread
- * geometry (0 before any such call). -1 for another `which`. */
+/* Tile statistics of the last tile-path call (0 before any): 0 records streamed through the tile kernel (a record of a slot
+ * that is redone, by the full-size launch or after a table overflow, counts once per pass), 1 run heads probed (a run of
+ * identical neighbours in one warp step probes once), 2 probe batches of 32 heads (full warps); 3 is the number of slots
+ * of the last tile-path call that ran the 256-thread geometry. -1 for another `which`. */
 int64_t tb_last_tile_stat(tb_ctx*, int which);
 /* Device time in ms of one stage of the last call, measured with CUDA events on the launching stream
  * (enabled by tb_set_profiling(ctx,1)):

@@ -178,9 +178,11 @@ class Context:
         return int(self.lib.tb_last_tile_gen(self.h))
 
     def last_tile_stats(self):
-        """Tile statistics: multi_pass, deferred_records and deferred_slots are always 0; slots is the slot count of the
-        last tile-path call that ran the 256-thread geometry (0 before any)."""
-        return dict(zip(("multi_pass", "deferred_records", "deferred_slots", "slots"), (int(self.lib.tb_last_tile_stat(self.h, i)) for i in range(4))))
+        """Tile statistics of the last tile-path call (0 before any): records streamed through the tile kernel (a record of
+        a slot that is redone counts once per pass), heads probed (a run of identical neighbours inside one 32-record warp
+        step probes the table once, for all of its records), batches of 32 heads probed as one full warp, and slots, the
+        slot count of the last tile-path call that ran the 256-thread geometry."""
+        return dict(zip(("records", "heads", "batches", "slots"), (int(self.lib.tb_last_tile_stat(self.h, i)) for i in range(4))))
 
     def last_yd_path(self):
         """0 parallel YD formulation, 1 sequential segment lists."""

@@ -102,7 +102,7 @@ int64_t tb_last_ord_deep(tb_ctx* ctx) { return ctx ? ctx->last_ord_deep : -1; }
 int64_t tc_stream_windows(tb_ctx* ctx) { return ctx ? ctx->stream_windows : -1; }
 int tc_last_exact(tb_ctx* ctx) { return ctx ? ctx->last_cov_exact : -1; }
 int tb_last_tile_gen(tb_ctx* ctx) { return ctx ? ctx->last_tile_gen : -1; }
-int64_t tb_last_tile_stat(tb_ctx* ctx, int which) { return (ctx && which >= 0 && which < 4) ? (which == 3 ? ctx->last_tile_slots : 0) : -1; }
+int64_t tb_last_tile_stat(tb_ctx* ctx, int which) { return (ctx && which >= 0 && which < 4) ? (which == 3 ? ctx->last_tile_slots : ctx->last_tile_runs[which]) : -1; }
 int tb_set_profiling(tb_ctx* ctx, int on) { if (!ctx) return 1; ctx->profiling = on; return 0; }
 float tb_last_kernel_ms(tb_ctx* ctx, int which) { return (ctx && which >= 0 && which < 16) ? ctx->last_ms[which] : 0.f; }
 

@@ -15,8 +15,10 @@
 //              (k slices, located by the per-(slot,file) offsets), so loads are coalesced and the per-file running
 //              maximum of `end` that defines the merge order is a warp-local segmented scan with a register carry.
 //              A record probes its region: tag compare in shared memory, then its real key bytes against the owner's
-//              (grouping never rests on the hash). Lanes of one file hitting one group are merged with match_any:
-//              one count atomic, (rarely) one representative atomicMin, (rarely) one sample-bit atomicOr.
+//              (grouping never rests on the hash). Only the first record of a run of identical neighbours inside a
+//              32-record warp step probes, for the whole run; these run heads are queued in registers and probe 32 at a
+//              time. Heads of one file hitting one group are merged with match_any: one representative atomicMin and
+//              one sample-bit atomicOr (both rarely), plus each head's count atomic.
 //   epilogue   occupied entries are compacted in region (= position) order, ranked inside their position by
 //              (strand, end, mode key) with the reference's comparator, and written to the staging arrays.
 #include <limits.h>
@@ -196,22 +198,24 @@ __device__ __noinline__ unsigned long long tile_tail_chunk(const ColIn& in, uint
 // strand by the tag. Identical raw CIGARs decide every mode but -L at once (identical CIGAR at one position => identical
 // clipped CIGAR and identical exon chain); -L then compares the MD bytes inline. Only records whose raw CIGARs differ
 // (or whose MD lengths differ) go through the general comparator, which is exact for every mode.
-__device__ __forceinline__ bool tile_same_key(const ColIn& in, uint32_t i, uint32_t c0, uint32_t c1, uint32_t o) {
-  const uint32_t o0 = in.cig_off[o], o1 = in.cig_off[o + 1];
+// The inline part: identical raw CIGAR words [c0,c1) vs [o0,o1) and, in -L, identical MD bytes. True is exact for every
+// mode; false only means "not decided here".
+__device__ __forceinline__ bool tile_same_raw(const ColIn& in, uint32_t i, uint32_t c0, uint32_t c1, uint32_t o, uint32_t o0, uint32_t o1) {
   const uint32_t nc = c1 - c0;
   bool same_cigar = (o1 - o0 == nc);
   if (same_cigar)
     for (uint32_t q = 0; q < nc; ++q) if (in.cigar[c0 + q] != in.cigar[o0 + q]) { same_cigar = false; break; }
-  if (in.mode == TB_MODE_CIGAR) return same_cigar;
-  if (same_cigar) {
-    if (in.mode != TB_MODE_FULL) return true;
-    const uint32_t ma = in.md_off[i], na = in.md_off[i + 1] - ma, mb = in.md_off[o], nb = in.md_off[o + 1] - mb;
-    if (na == nb) {
-      bool eq = true;
-      for (uint32_t q = 0; q < na; ++q) if (in.md[ma + q] != in.md[mb + q]) { eq = false; break; }
-      if (eq) return true;
-    }
-  }
+  if (!same_cigar) return false;
+  if (in.mode != TB_MODE_FULL) return true;
+  const uint32_t ma = in.md_off[i], na = in.md_off[i + 1] - ma, mb = in.md_off[o], nb = in.md_off[o + 1] - mb;
+  if (na != nb) return false;
+  for (uint32_t q = 0; q < na; ++q) if (in.md[ma + q] != in.md[mb + q]) return false;
+  return true;
+}
+
+__device__ __forceinline__ bool tile_same_key(const ColIn& in, uint32_t i, uint32_t c0, uint32_t c1, uint32_t o) {
+  if (tile_same_raw(in, i, c0, c1, o, in.cig_off[o], in.cig_off[o + 1])) return true;
+  if (in.mode == TB_MODE_CIGAR) return false;
   return tb_mode_cmp(in, i, o) == 0;
 }
 
@@ -219,7 +223,8 @@ __device__ __forceinline__ bool tile_same_key(const ColIn& in, uint32_t i, uint3
 // of the record parser / verifier / sort key folds away); MODE < 0 reads it from the window descriptor.
 template <int THREADS, int MODE>
 __device__ uint32_t tile_process(const ColIn& in_, const TileParams& tp, TileSmem<THREADS>& sm, uint32_t n_sub, uint32_t rankbase, bool single,
-                                 uint64_t outbase, uint32_t* s_scan, volatile uint32_t* s_flags /*[0]=kept [1]=overflow [2]=ngroups*/) {
+                                 uint64_t outbase, uint32_t* s_scan,
+                                 volatile uint32_t* s_flags /*[0]=kept [1]=overflow [2]=ngroups; whole launch: [4]=records [5]=heads [6]=batches*/) {
   constexpr int NW = THREADS / 32;
   ColIn in = in_;
   if (MODE >= 0) in.mode = MODE;
@@ -282,12 +287,22 @@ __device__ uint32_t tile_process(const ColIn& in_, const TileParams& tp, TileSme
       }
     }
   }
+  // Runs of identical neighbours: a passing record that is the same alignment as the record in the lane before it (same
+  // file, hence record i-1; same position, strand, tag and raw CIGAR words, and in -L the same MD bytes) is a member
+  // of that lane's run; it neither probes nor merges. The run's first record, its head, carries the weight 1 + members,
+  // and keeps its own (E, index), the smallest of the run (the running maximum E is non-decreasing along it). Runs end at
+  // a warp step, so lane 0 is always a head. Heads queue in registers (lane q holds queue entry q) until 32 are pending
+  // and then probe the table as one full warp; the rest is flushed by extra steps past the range's end.
   const uint32_t glimit = E - (E >> 3);
-  for (uint32_t jb = j0; jb < j1; jb += 32) {
+  uint32_t q_i = 0, q_tag = 0, q_rel = 0, q_fw = 0; int q_E = 0;   // this lane's queue entry
+  uint32_t npend = 0;                                                           // queued heads (warp-uniform)
+  uint32_t n_heads = 0, n_batches = 0;                                          // statistics (warp-uniform)
+  uint32_t jb = j0;
+  for (; jb < j1 || npend; jb += 32) {
     if (single && s_flags[2] > glimit) { s_flags[1] = 1; break; }   // warp-uniform (broadcast read)
     const uint32_t j = jb + lane;
     const bool valid = j < j1;
-    uint32_t f = 0xfffffffeu, i = 0, c0 = 0, c1 = 0, h1 = 0, h2 = 0; int pos = INT_MIN + 1 + (int)lane, reflen = 0; bool pass = false; unsigned sc = 0;
+    uint32_t f = 0xfffffffeu, i = 0, c0 = 0, c1 = 0, h1 = 0; int pos = INT_MIN + 1 + (int)lane, reflen = 0; bool pass = false; unsigned sc = 0;
     if (valid) {
       f = f_lo;                                   // slices are contiguous in j: walk forward from the step's first file
       while (sm.soff[f + 1] <= j) ++f;
@@ -296,8 +311,39 @@ __device__ uint32_t tile_process(const ColIn& in_, const TileParams& tp, TileSme
       c0 = in.cig_off[i]; c1 = in.cig_off[i + 1];
       const uint16_t fl = in.flag[i]; const uint8_t mq = in.mapq[i]; const uint16_t nh = in.nh[i];
       sc = tb_strand_code(in.strand[i]);
-      tb_parse_record32(in, i, pos, c0, c1, reflen, h1, h2);
       pass = tb_passes_options(in, fl, mq, nh);
+    }
+    // parse: reference length and key hash. Outside -E the CIGAR walk is one warp-uniform loop, so every word is compared
+    // with the same word of the previous lane's record on the way (same_words: the raw CIGARs are identical).
+    const uint32_t nc = c1 - c0;
+    bool same_words = __shfl_up_sync(0xffffffffu, nc, 1) == nc;
+    if (in.mode == TB_MODE_EXON) {
+      uint32_t h2;
+      if (valid) tb_parse_record32(in, i, pos, c0, c1, reflen, h1, h2);
+    } else {
+      uint32_t a = c0, b = c1;
+      if (in.mode == TB_MODE_CLIP && valid) tb_clip_range(in.cigar, a, b);
+      h1 = 0x9876543u ^ (b - a);
+      const uint32_t nmax = __reduce_max_sync(0xffffffffu, nc);
+      for (uint32_t q = 0; q < nmax; ++q) {
+        const uint32_t c = c0 + q;
+        const uint32_t w = q < nc ? in.cigar[c] : 0u;
+        same_words &= __shfl_up_sync(0xffffffffu, w, 1) == w;
+        if (q < nc && tb_op_ref(w & 0xf)) reflen += (int)(w >> 4);
+        if (c >= a && c < b) { h1 = (h1 ^ w) * 0x9E3779B1u; h1 ^= h1 >> 15; }
+      }
+      if (in.mode == TB_MODE_FULL && valid) {   // the MD tag, as tb_parse_record32 folds it
+        const uint32_t m0 = in.md_off[i], m1 = in.md_off[i + 1];
+        h1 = (h1 ^ (uint32_t)(m1 > m0)) * 0x9E3779B1u; h1 ^= h1 >> 15;
+        uint32_t acc = 0, nb = 0;
+        for (uint32_t q = m0; q < m1; ++q) {
+          const uint32_t ch = in.md[q];
+          if (ch == 0) break;
+          acc = (acc << 8) | ch;
+          if (++nb == 4) { h1 = (h1 ^ acc) * 0x9E3779B1u; h1 ^= h1 >> 15; acc = 0; nb = 0; }
+        }
+        h1 = (h1 ^ (acc ^ (nb << 29))) * 0x9E3779B1u; h1 ^= h1 >> 15;
+      }
     }
     // segmented inclusive max-scan of ref_len over (file,position) runs == the running max that orders the reference's
     // priority queue (SURVEY §9.2); records the filters drop still take part (they delay the records behind them)
@@ -315,43 +361,84 @@ __device__ uint32_t tile_process(const ColIn& in_, const TileParams& tp, TileSme
     carry_f = __shfl_sync(0xffffffffu, f, 31); carry_pos = __shfl_sync(0xffffffffu, pos, 31); carry_max = __shfl_sync(0xffffffffu, Erel, 31);
     f_lo = carry_f;   // only meaningful while lane 31 is valid, i.e. while another step follows
 
+    // ---- run detection: slot-independent hash of the key, compared with the previous lane's as a pre-filter ----
+    const uint32_t tag = (sc << 30) | (tb_mix32(h1 ^ ((uint32_t)reflen * 0x9E3779B1u) ^ (uint32_t)tp.seed) >> 2);
+    const unsigned passm = __ballot_sync(0xffffffffu, pass);
+    my_kept += pass;
+    const uint32_t tag_u = __shfl_up_sync(0xffffffffu, tag, 1), c0_u = __shfl_up_sync(0xffffffffu, c0, 1);
+    bool member = pass && lane > 0 && ((passm >> (lane - 1)) & 1u) && f == f_prev && pos == pos_prev && tag == tag_u && same_words;
+    if (member && in.mode == TB_MODE_EXON)   // the walk above did not compare; record i-1's words end where record i's begin
+      member = tile_same_raw(in, i, c0, c1, i - 1, c0_u, c0);
+    if (member && in.mode == TB_MODE_FULL) {   // -L: the MD bytes as well (record i-1's end where record i's begin)
+      const uint32_t ma = in.md_off[i], na = in.md_off[i + 1] - ma, mb = in.md_off[i - 1];
+      if (ma - mb != na) member = false;
+      for (uint32_t q = 0; member && q < na; ++q) member = in.md[ma + q] == in.md[mb + q];
+    }
+    const unsigned memm = __ballot_sync(0xffffffffu, member);
+    const unsigned headm = passm & ~memm;
+    const uint32_t nh = __popc(headm);
+    // ---- append the heads to the queue: lane q takes the head of rank (q - npend) mod 32 ----
+    const uint32_t r = (lane - npend) & 31u;
+    uint32_t src = 0;   // lane of the r-th set bit of headm (r < nh)
+#pragma unroll
+    for (uint32_t w = 16; w; w >>= 1)
+      if ((uint32_t)__popc(headm & ((1u << (src + w)) - 1u)) <= r) src += w;
+    const uint32_t weight = __ffsll(~((unsigned long long)memm >> (lane + 1)));   // 1 + the members that follow
+    const uint32_t g_i = __shfl_sync(0xffffffffu, i, src), g_tag = __shfl_sync(0xffffffffu, tag, src);
+    const uint32_t g_rel = __shfl_sync(0xffffffffu, (uint32_t)(pos - in.pos_lo), src), g_fw = __shfl_sync(0xffffffffu, f | (weight << 26), src);
+    const int g_E = __shfl_sync(0xffffffffu, Erel, src);
+    if (lane >= npend) { q_i = g_i; q_tag = g_tag; q_rel = g_rel; q_fw = g_fw; q_E = g_E; }
+    const uint32_t tot = npend + nh;
+    if (tot == 0 || (tot < 32 && jb + 32 < j1)) { npend = tot; continue; }   // warp-uniform: not full, and more records follow
+
+    // ---- probe the queued heads as one warp (all 32 lanes unless this is the range's last batch) ----
+    const bool live = lane < tot;
+    const uint32_t qf = q_fw & 0x3ffffffu;
+    n_heads += tot < 32 ? tot : 32u; n_batches += tot >= 32;
     uint32_t s = 0;
-    if (pass) {
-      ++my_kept;
+    bool placed = false;
+    if (live) {
       uint32_t base = 0, size = E;
       if (!single) {
-        const uint32_t rel = (uint32_t)(pos - in.pos_lo);
-        const uint32_t Pa = tp.P[rel] - rankbase, Pb = tp.P[rel + 1] - rankbase;
+        const uint32_t Pa = tp.P[q_rel] - rankbase, Pb = tp.P[q_rel + 1] - rankbase;
         base = (5u * Pa) >> 2; size = ((5u * Pb) >> 2) - base;
       }
-      const uint32_t tag = (sc << 30) | (tb_mix32(h1 ^ ((uint32_t)reflen * 0x9E3779B1u) ^ (uint32_t)tp.seed) >> 2);
-      s = base + __umulhi(tb_mix32(h2 + (uint32_t)reflen), size);
-      const unsigned long long mine = ((unsigned long long)tag << 32) | i;
-      bool placed = false;
+      s = base + __umulhi(q_tag << 2, size);   // the tag's 30 hash bits also pick the first entry
+      const unsigned long long mine = ((unsigned long long)q_tag << 32) | q_i;
       for (uint32_t t = 0; t < size; ++t) {
         unsigned long long w = sm.word[s];
         if (w == EMPTY64) {
           w = atomicCAS(&sm.word[s], EMPTY64, mine);
           if (w == EMPTY64) { sm.rbase[s] = (uint16_t)base; atomicAdd((uint32_t*)&s_flags[2], 1u); placed = true; break; }
         }
-        if ((uint32_t)(w >> 32) == tag) {
+        if ((uint32_t)(w >> 32) == q_tag) {
           const uint32_t o = (uint32_t)w;  // owner: compare the real keys
-          if (o == i || tile_same_key(in, i, c0, c1, o)) { placed = true; break; }
+          if (o == q_i || tile_same_key(in, q_i, in.cig_off[q_i], in.cig_off[q_i + 1], o)) { placed = true; break; }
         }
         if (++s == base + size) s = base;
       }
-      if (!placed) { s_flags[1] = 1; pass = false; }
+      if (!placed) s_flags[1] = 1;
     }
-    // merge the lanes of one file that hit one group: the lowest lane has the smallest (E, index) of them
-    const uint32_t mkey = pass ? (s | (f << 13)) : (0x80000000u | lane);
+    // merge the heads of one file that hit one group: queue order is stream order, so the lowest lane has the smallest
+    // (E, index) of them. Each head adds its own weight to the count (a warp reduction over the match_any groups would
+    // run once per distinct group mask).
+    const uint32_t mkey = placed ? (s | (qf << 13)) : (0x80000000u | lane);
     const unsigned peers = __match_any_sync(0xffffffffu, mkey);
-    if (pass && (int)lane == __ffs(peers) - 1) {
-      atomicAdd(&sm.cnt[s], (uint32_t)__popc(peers));
-      const unsigned long long repkey = ((unsigned long long)(uint32_t)Erel << 32) | i;
+    if (placed) atomicAdd(&sm.cnt[s], q_fw >> 26);
+    if (placed && (int)lane == __ffs(peers) - 1) {
+      const unsigned long long repkey = ((unsigned long long)(uint32_t)q_E << 32) | q_i;
       if (repkey < sm.rep[s]) atomicMin(&sm.rep[s], repkey);
-      const uint32_t bi = s * W + (f >> 5), bit = 1u << (f & 31);
+      const uint32_t bi = s * W + (qf >> 5), bit = 1u << (qf & 31);
       if (!(sm.bits[bi] & bit)) atomicOr(&sm.bits[bi], bit);
     }
+    // heads beyond the batch stay queued: lane q < tot - 32 took rank q + 32 - npend, exactly the first of them
+    q_i = g_i; q_tag = g_tag; q_rel = g_rel; q_fw = g_fw; q_E = g_E;
+    npend = tot > 32 ? tot - 32 : 0u;
+  }
+  if (lane == 0) {
+    atomicAdd((uint32_t*)&s_flags[4], min(jb, j1) - j0);
+    atomicAdd((uint32_t*)&s_flags[5], n_heads);
+    atomicAdd((uint32_t*)&s_flags[6], n_batches);
   }
   if (my_kept) atomicAdd((uint32_t*)&s_flags[0], my_kept);
   __syncthreads();
@@ -402,17 +489,26 @@ __device__ uint32_t tile_process(const ColIn& in_, const TileParams& tp, TileSme
       const uint16_t rb = sm.rbase[e];
       const unsigned long long ki = sm.word[e];
       uint32_t rank = 0, ties = 0;
-      for (uint32_t q = r; q > 0;) {
-        const uint32_t eq = sm.occ[--q];
-        if (!single && sm.rbase[eq] != rb) break;
-        const unsigned long long kq = sm.word[eq];
-        rank += kq < ki; ties += kq == ki;
-      }
-      for (uint32_t q = r + 1; q < G; ++q) {
-        const uint32_t eq = sm.occ[q];
-        if (!single && sm.rbase[eq] != rb) break;
-        const unsigned long long kq = sm.word[eq];
-        rank += kq < ki; ties += kq == ki;
+      if (single) {   // one position: every entry is compared, with no region test
+#pragma unroll 4
+        for (uint32_t q = 0; q < G; ++q) {
+          const unsigned long long kq = sm.word[sm.occ[q]];
+          rank += kq < ki; ties += kq == ki;
+        }
+        --ties;   // the entry itself
+      } else {        // the entries of the position: the neighbours with the same region base
+        for (uint32_t q = r; q > 0;) {
+          const uint32_t eq = sm.occ[--q];
+          if (sm.rbase[eq] != rb) break;
+          const unsigned long long kq = sm.word[eq];
+          rank += kq < ki; ties += kq == ki;
+        }
+        for (uint32_t q = r + 1; q < G; ++q) {
+          const uint32_t eq = sm.occ[q];
+          if (sm.rbase[eq] != rb) break;
+          const unsigned long long kq = sm.word[eq];
+          rank += kq < ki; ties += kq == ki;
+        }
       }
       uint16_t sat = round == 0 ? ((((uint32_t)(ki >> 24) & 0xffu) == 255u) ? 0x4000u : 0u) : (sm.tmp[e] & 0x4000u);
       sm.tmp[e] = (uint16_t)(rank | sat | (ties ? 0x8000u : 0u));
@@ -433,8 +529,8 @@ __device__ uint32_t tile_process(const ColIn& in_, const TileParams& tp, TileSme
     const uint32_t e = sm.occ[r];
     const uint16_t rb = sm.rbase[e];
     const uint32_t t = sm.tmp[e];
-    uint32_t rank = t & 0x1fffu, a = r;
     const bool tied = (t & 0x8000u) != 0;
+    uint32_t rank = t & 0x1fffu, a = (single && !tied) ? 0u : r;   // a: first entry of the position (0 in single mode)
     const unsigned long long ki = sm.word[e];
     const uint32_t oi = (uint32_t)(sm.rep[e] >> 32);
     while (a > 0) {
@@ -466,7 +562,7 @@ template <int THREADS, int MODE>
 __global__ void __launch_bounds__(THREADS, 1024 / THREADS) col_tile_kernel(ColIn in, TileParams tp) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   __shared__ uint32_t s_scan[33];
-  __shared__ uint32_t s_flags[4];
+  __shared__ uint32_t s_flags[8];
   __shared__ SlotMeta s_meta[2];
   __shared__ uint32_t s_pbig;
   const uint32_t E = tp.ecap, W = tp.W, k = (uint32_t)in.k, tid = threadIdx.x;
@@ -491,7 +587,7 @@ __global__ void __launch_bounds__(THREADS, 1024 / THREADS) col_tile_kernel(ColIn
   auto load_bounds = [&](const SlotMeta& d, uint32_t* dst) {   // all threads: per-file slices of a slot
     if (d.m < tp.M) for (uint32_t f = tid; f < k; f += THREADS) { dst[f] = tp.off[(uint64_t)d.m * k + f]; dst[k + f] = tp.off[(uint64_t)(d.m + 1) * k + f]; }
   };
-  if (tid == 0) { fetch_meta(s_meta[0]); fetch_meta(s_meta[1]); }
+  if (tid == 0) { fetch_meta(s_meta[0]); fetch_meta(s_meta[1]); s_flags[4] = 0; s_flags[5] = 0; s_flags[6] = 0; }
   __syncthreads();
   load_bounds(s_meta[0], ab);
   for (uint32_t it = 0;; ++it) {
@@ -563,6 +659,11 @@ __global__ void __launch_bounds__(THREADS, 1024 / THREADS) col_tile_kernel(ColIn
     if (tid == 0) tp.gcount[m] = G;
   }
   if (tid == 0 && kept_total) atomicAdd((unsigned long long*)&tp.status[CS_NKEPT], (unsigned long long)kept_total);
+  if (tid == 0 && s_flags[4]) {
+    atomicAdd((unsigned long long*)&tp.status[CS_TILE_RECORDS], (unsigned long long)s_flags[4]);
+    atomicAdd((unsigned long long*)&tp.status[CS_TILE_HEADS], (unsigned long long)s_flags[5]);
+    atomicAdd((unsigned long long*)&tp.status[CS_TILE_BATCHES], (unsigned long long)s_flags[6]);
+  }
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -718,6 +819,7 @@ int col_front_tile(tb_ctx* ctx, const ColIn& in, const ColGeom& g, ColGroups& ou
     if (cudaEventElapsedTime(&ms, ctx->ev[5], ctx->ev[0]) == cudaSuccess) ctx->last_ms[3] = ms;
     (void)cudaGetLastError();
   }
+  for (int q = 0; q < 3; ++q) ctx->last_tile_runs[q] = h_status[CS_TILE_RECORDS + q];
   if (h_status[CS_ERR] == ERR_UNSORTED) { ctx->set_error("tb_collapse_window: run not coordinate-sorted at record %lld", h_status[CS_ERRIDX]); return 1; }
   if (h_status[CS_TABLE_OVERFLOW]) return 2;
   const int64_t G = h_status[CS_NGROUPS];

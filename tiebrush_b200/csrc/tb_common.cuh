@@ -78,6 +78,7 @@ struct tb_ctx {
   int last_cov_exact = 0;   // last coverage call took the exact ordered-double path (weights that are not multiples of 2^-20)
   int last_tile_gen = 0;    // 1 once a collapse call has run the tile kernel (col_tile_kernel)
   int64_t last_tile_slots = 0;   // slots of the last tile-path call that used the heavy list (256-thread geometry)
+  int64_t last_tile_runs[3] = {0, 0, 0};   // last tile-path call: records streamed, heads probed, full-warp probe batches
   std::string err;
   DevBuf buf[TB_NBUF];   // workspace slots (see the enum in each pipeline)
   DevBuf in_stage[20];   // device copies of host input arrays
