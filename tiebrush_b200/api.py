@@ -287,79 +287,198 @@ class Context:
         return res
 
     # ------------------------------------------------------------------------------------------
+    # tiecov (csrc/coverage.cu, csrc/shard.cu, csrc/bgzf.cu): thin ctypes plumbing, no logic of its own
+    def _check(self, rc):
+        """Raises for a failed tiecov call: ValueError for bad input records (rc 2: an unsupported CIGAR op), TieBrushError
+        for anything else."""
+        if rc == 2:
+            raise ValueError(self._err())
+        if rc != 0:
+            raise TieBrushError(self._err())
+
     def sample_window(self, cols, cap_rows=None):
         """tiecov -s of one window (whole bundles): rows (tid, start0, end0, ival) of the sample-count heat-map; `cols` needs
         tid, pos, yc, strand, cig_off, cigar as for coverage_window plus yx (YX tag, 1 when absent). Host columns only."""
-        n = int(cols["pos"].shape[0])
-        keep = [_host(cols[k], dt) for k, dt in (("tid", np.int32), ("pos", np.int32), ("yc", np.float32), ("strand", np.uint8),
-                                                 ("cig_off", np.uint32), ("cigar", np.uint32), ("yx", np.int32))]
-        tid, pos, yc, strand, cig_off, cigar, yx = keep
-        n_cig = int(cig_off[-1]) if n else 0
-        cin = _lib.CovIn(n, _ptr(tid), _ptr(pos), _ptr(yc), _ptr(strand), _ptr(cig_off), _ptr(cigar), 0, n_cig)
-        cap = cap_rows if cap_rows is not None else 2 * n_cig + 16
-        rt, rs, re, rv = np.empty(cap, np.int32), np.empty(cap, np.int32), np.empty(cap, np.int32), np.empty(cap, np.float64)
-        rows = _lib.RunsOut(cap, 0, _ptr(rt), _ptr(rs), _ptr(re), _ptr(rv), 0)
-        rc = self.lib.tc_sample_window(self.h, C.byref(cin), _ptr(yx), C.byref(rows))
-        if rc == 2:
-            raise ValueError(self._err())
-        if rc != 0:
-            raise TieBrushError(self._err())
-        r = int(rows.n_runs)
-        return rt[:r], rs[:r], re[:r], rv[:r].astype(np.uint64)
+        keep = []
+        cin = _cov_in(cols, keep)
+        yx = _host(cols["yx"], np.int32)
+        out = cov_out_buffers(cap_rows if cap_rows is not None else 2 * int(cin.n_cig) + 16, 1)
+        rows, _ = _out_structs(out)
+        self._check(self.lib.tc_sample_window(self.h, C.byref(cin), _ptr(yx), C.byref(rows)))
+        t, s0, e0, v = _rows(out, int(rows.n_runs), 0)["runs"]
+        return t, s0, e0, v.astype(np.uint64)
 
     def coverage_window(self, cols, want_runs=True, want_juncs=True, cap_runs=None, cap_juncs=None, out=None):
         """One window of tiecov -c/-j. Returns dict(runs=(tid,start0,end0,value), juncs=(tid,start,end,strand,value))."""
-        dev = _is_torch(cols["pos"])
-        n = int(cols["pos"].shape[0])
         keep = []
-
-        def col(name, dt):
-            a = cols[name]
-            if not dev:
-                a = _host(a, dt)
-            keep.append(a)
-            return a
-
-        tid, pos, yc = col("tid", np.int32), col("pos", np.int32), col("yc", np.float32)
-        strand, cig_off, cigar = col("strand", np.uint8), col("cig_off", np.uint32), col("cigar", np.uint32)
-        n_cig = int(cols["n_cig"]) if "n_cig" in cols else (int(cig_off[-1]) if n else 0)
-        end = cols.get("end")
-        if end is not None:
-            end = end if dev else _host(end, np.int32)
-            keep.append(end)
-        cin = _lib.CovIn(n, _ptr(tid), _ptr(pos), _ptr(yc), _ptr(strand), _ptr(cig_off), _ptr(cigar), 1 if dev else 0, n_cig, _ptr(end))
-        capr = cap_runs if cap_runs is not None else 2 * n_cig + 16
-        capj = cap_juncs if cap_juncs is not None else n_cig + 16
+        cin = _cov_in(cols, keep)
         if out is None:
-            if dev:
-                import torch
-                d = cols["pos"].device
-                i32 = lambda m: torch.empty(m, dtype=torch.int32, device=d)
-                out = dict(r_tid=i32(capr), r_start=i32(capr), r_end=i32(capr), r_val=torch.empty(capr, dtype=torch.float64, device=d),
-                           j_tid=i32(capj), j_start=i32(capj), j_end=i32(capj), j_strand=torch.empty(capj, dtype=torch.uint8, device=d),
-                           j_val=torch.empty(capj, dtype=torch.float64, device=d))
-            else:
-                out = dict(r_tid=np.empty(capr, np.int32), r_start=np.empty(capr, np.int32), r_end=np.empty(capr, np.int32), r_val=np.empty(capr, np.float64),
-                           j_tid=np.empty(capj, np.int32), j_start=np.empty(capj, np.int32), j_end=np.empty(capj, np.int32),
-                           j_strand=np.empty(capj, np.uint8), j_val=np.empty(capj, np.float64))
-        odev = 1 if _is_torch(out["r_tid"]) else 0
-        runs = _lib.RunsOut(int(out["r_tid"].shape[0]), 0, _ptr(out["r_tid"]), _ptr(out["r_start"]), _ptr(out["r_end"]), _ptr(out["r_val"]), odev)
-        juncs = _lib.JuncsOut(int(out["j_tid"].shape[0]), 0, _ptr(out["j_tid"]), _ptr(out["j_start"]), _ptr(out["j_end"]), _ptr(out["j_strand"]),
-                              _ptr(out["j_val"]), odev)
-        rc = self.lib.tc_coverage_window(self.h, C.byref(cin), C.byref(runs) if want_runs else None, C.byref(juncs) if want_juncs else None)
-        if rc == 2:
-            raise ValueError(self._err())
-        if rc != 0:
-            raise TieBrushError(self._err())
-        r, j = int(runs.n_runs), int(juncs.n_juncs)
-        return dict(runs=(out["r_tid"][:r], out["r_start"][:r], out["r_end"][:r], out["r_val"][:r]),
-                    juncs=(out["j_tid"][:j], out["j_start"][:j], out["j_end"][:j], out["j_strand"][:j], out["j_val"][:j]),
-                    n_runs=r, n_juncs=j)
+            n_cig = int(cin.n_cig)
+            out = cov_out_buffers(cap_runs if cap_runs is not None else 2 * n_cig + 16, cap_juncs if cap_juncs is not None else n_cig + 16,
+                                  device=cols["pos"].device if _is_torch(cols["pos"]) else None)
+        runs, juncs = _out_structs(out)
+        self._check(self.lib.tc_coverage_window(self.h, C.byref(cin), C.byref(runs) if want_runs else None, C.byref(juncs) if want_juncs else None))
+        return _rows(out, int(runs.n_runs), int(juncs.n_juncs))
+
+    def last_cov_exact(self):
+        return int(self.lib.tc_last_exact(self.h))
+
+    def coverage_stream(self, cols, window, out, next_tid_pos=None):
+        """tc_coverage_stream: one slice in windows cut at bundle heads. Returns the rows and `consumed`."""
+        keep = []
+        cin = _cov_in(cols, keep)
+        runs, juncs = _out_structs(out)
+        nx = None
+        if next_tid_pos is not None:
+            nx = (C.c_int32 * 2)(int(next_tid_pos[0]), int(next_tid_pos[1]))
+        consumed = C.c_int64(0)
+        self._check(self.lib.tc_coverage_stream(self.h, C.byref(cin), int(window), nx, C.byref(runs), C.byref(juncs), C.byref(consumed)))
+        res = _rows(out, int(runs.n_runs), int(juncs.n_juncs))
+        res["consumed"] = int(consumed.value)
+        res["windows"] = int(self.lib.tc_stream_windows(self.h))
+        return res
+
+    def comm_init(self, rank, world, unique_id):
+        buf = (C.c_ubyte * 128).from_buffer_copy(unique_id)
+        self._check(self.lib.tb_comm_init(self.h, int(rank), int(world), buf))
+
+    def shard_coverage(self, segs, window, out):
+        """tc_shard_coverage over this rank's device-resident segments (list of column dicts). Collective."""
+        keep = []
+        arr = (_lib.CovIn * len(segs))(*[_cov_in(s, keep) for s in segs])
+        runs, juncs = _out_structs(out)
+        self._check(self.lib.tc_shard_coverage(self.h, arr, len(segs), int(window), C.byref(runs), C.byref(juncs)))
+        res = _rows(out, int(runs.n_runs), int(juncs.n_juncs))
+        res["windows"] = int(self.lib.tc_stream_windows(self.h))
+        res["stats"] = dict(zip(("lead_received", "lead_sent", "ranks_received_from", "halo_bytes_sent", "seam_records"),
+                                (int(self.lib.tc_shard_stat(self.h, i)) for i in range(5))))
+        return res
+
+    def shard_gather(self, local, all_out, world):
+        """tc_shard_gather: ordered gather of `local` (result of shard_coverage, device rows) into `all_out` on rank 0. Collective."""
+        lr = _lib.RunsOut(int(local["n_runs"]), int(local["n_runs"]), *[_ptr(a) for a in local["runs"]], 1)
+        lj = _lib.JuncsOut(int(local["n_juncs"]), int(local["n_juncs"]), *[_ptr(a) for a in local["juncs"]], 1)
+        base = (C.c_int64 * (world + 1))()
+        if all_out is not None:
+            ar, aj = _out_structs(all_out)
+            rc = self.lib.tc_shard_gather(self.h, C.byref(lr), C.byref(lj), C.byref(ar), C.byref(aj), base)
+        else:
+            rc = self.lib.tc_shard_gather(self.h, C.byref(lr), C.byref(lj), None, None, base)
+        self._check(rc)
+        res = dict(junc_base=[int(x) for x in base], gather_bytes=int(self.lib.tc_shard_stat(self.h, 5)))
+        if all_out is not None:
+            res.update(_rows(all_out, int(ar.n_runs), int(aj.n_juncs)))
+        return res
+
+    def shard_coverage_gather(self, segs, window, out, all_out, cap_runs_all, cap_juncs_all, world):
+        """tc_shard_coverage_gather: this rank's windows with the ordered gather on rank 0 overlapped (one round per window on a
+        second stream). `all_out` = rank 0's arrays (capacity cap_*_all, cut into `world` regions), None elsewhere; every rank
+        passes the same capacities. Returns the local rows, the regions [(runs offset, runs, juncs offset, juncs)] and, on rank 0,
+        the gathered rows per region."""
+        keep = []
+        arr = (_lib.CovIn * len(segs))(*[_cov_in(s, keep) for s in segs])
+        runs, juncs = _out_structs(out)
+        if all_out is not None:
+            ar, aj = _out_structs(all_out)
+            ar.capacity, aj.capacity = int(cap_runs_all), int(cap_juncs_all)
+        else:
+            ar = _lib.RunsOut(int(cap_runs_all), 0, None, None, None, None, 1)
+            aj = _lib.JuncsOut(int(cap_juncs_all), 0, None, None, None, None, None, 1)
+        region = (C.c_int64 * (4 * world))()
+        self._check(self.lib.tc_shard_coverage_gather(self.h, arr, len(segs), int(window), C.byref(runs), C.byref(juncs), C.byref(ar), C.byref(aj), region))
+        res = _rows(out, int(runs.n_runs), int(juncs.n_juncs))
+        res["windows"] = int(self.lib.tc_stream_windows(self.h))
+        res["stats"] = dict(zip(("lead_received", "lead_sent", "ranks_received_from", "halo_bytes_sent", "seam_records", "gather_bytes", "gather_rounds"),
+                                (int(self.lib.tc_shard_stat(self.h, i)) for i in range(7))))
+        res["regions"] = [tuple(int(region[4 * r + q]) for q in range(4)) for r in range(world)]
+        res["total_runs"] = sum(x[1] for x in res["regions"]); res["total_juncs"] = sum(x[3] for x in res["regions"])
+        if all_out is not None:
+            def cat(keys, oi, ci):
+                parts = [[all_out[k][x[oi]:x[oi] + x[ci]] for x in res["regions"]] for k in keys]
+                if _is_torch(all_out[keys[0]]):
+                    import torch
+                    return tuple(torch.cat(p) for p in parts)
+                return tuple(np.concatenate(p) for p in parts)
+            res["gathered_runs"] = lambda: cat(("r_tid", "r_start", "r_end", "r_val"), 0, 1)
+            res["gathered_juncs"] = lambda: cat(("j_tid", "j_start", "j_end", "j_strand", "j_val"), 2, 3)
+        return res
+
+    def bam_columns(self, data, skip=0, last=True):
+        """tc_bam_columns: the tiecov columns of the complete records in `data` (bytes of whole or partial BGZF blocks; the
+        records start `skip` inflated bytes into the first block) as torch tensors on this context's device (copies: the
+        library's buffers are reused by the next call). Returns (cols, stat); stat["resume_byte"] / ["resume_skip"] tell where
+        the next chunk starts."""
+        import torch
+        bi, keep = _bgzf_in(data, skip, 1, last)
+        cin, yx, st = _lib.CovIn(), C.c_void_p(), _lib.BgzfStat()
+        self._check(self.lib.tc_bam_columns(self.h, C.byref(bi), C.byref(cin), C.byref(yx), C.byref(st)))
+        n = int(cin.n)
+        dev = torch.device("cuda", self.device)
+        with torch.cuda.device(dev):
+            t = lambda p, m, ts: torch.as_tensor(_DevArray(p, m, ts), device=dev).clone() if m else torch.empty(0, dtype={"<i4": torch.int32, "<f4": torch.float32, "|u1": torch.uint8}[ts], device=dev)
+            cols = dict(tid=t(cin.tid, n, "<i4"), pos=t(cin.pos, n, "<i4"), end=t(cin.end, n, "<i4"), yc=t(cin.yc, n, "<f4"), yx=t(yx.value, n, "<i4"),
+                        strand=t(cin.strand, n, "|u1"), cig_off=t(cin.cig_off, n + 1, "<i4"), cigar=t(cin.cigar, int(cin.n_cig), "<i4"))
+        cols["n_cig"] = int(cin.n_cig)
+        return cols, _stat(st)
+
+    def coverage_bam(self, path, want_runs=True, want_juncs=True, want_sample=False, chunk_bytes=16 << 20, window=1 << 22):
+        """tiecov -c / -j / -s of a BAM file, read in chunks of `chunk_bytes` and decoded on the device (tc_coverage_bam).
+        Returns dict(runs, juncs, n_runs, n_juncs) like coverage_window, plus sample=(tid, start0, end0, ival) when want_sample
+        (the rows of sample_window), header (read_bam_header) and stat (totals over the chunks)."""
+        hdr = read_bam_header(path)
+        parts = dict(r=[], j=[], s=[])
+        totals = dict(blocks=0, bytes_in=0, bytes_out=0, records=0, unmapped=0, chunks=0)
+        cap = 1 << 16
+        out = srow = None
+        with open(path, "rb") as f:
+            f.seek(hdr["block_offset"])
+            pending, skip, first, eof = b"", hdr["skip"], 1, False
+            while True:
+                new = b"" if eof else f.read(chunk_bytes)
+                eof = eof or len(new) < chunk_bytes
+                data = pending + new
+                last = eof
+                while True:
+                    if out is None:
+                        out = cov_out_buffers(cap, cap)
+                        srow = cov_out_buffers(cap, 1)
+                    runs, juncs = _out_structs(out)
+                    sr, _ = _out_structs(srow)
+                    bi, keep = _bgzf_in(data, skip, first, last)
+                    st = _lib.BgzfStat()
+                    rc = self.lib.tc_coverage_bam(self.h, C.byref(bi), int(window), C.byref(runs) if want_runs else None,
+                                                  C.byref(juncs) if want_juncs else None, C.byref(sr) if want_sample else None, C.byref(st))
+                    if rc == 5:
+                        cap = max(2 * cap, int(st.need_rows))
+                        out = None
+                        continue
+                    self._check(rc)
+                    break
+                r, j, ns = int(runs.n_runs), int(juncs.n_juncs), int(sr.n_runs)
+                if r:
+                    parts["r"].append(tuple(out[k][:r].copy() for k in ("r_tid", "r_start", "r_end", "r_val")))
+                if j:
+                    parts["j"].append(tuple(out[k][:j].copy() for k in ("j_tid", "j_start", "j_end", "j_strand", "j_val")))
+                if ns:
+                    parts["s"].append(tuple(srow[k][:ns].copy() for k in ("r_tid", "r_start", "r_end", "r_val")))
+                s = _stat(st)
+                for k in ("blocks", "bytes_in", "bytes_out", "records", "unmapped"):
+                    totals[k] += s[k]
+                totals["chunks"] += 1
+                first = 0
+                if last:
+                    break
+                pending, skip = data[s["resume_byte"]:], s["resume_skip"]
+        cat = lambda xs, dts: tuple(np.concatenate([x[i] for x in xs]) if xs else np.zeros(0, dt) for i, dt in enumerate(dts))
+        runs = cat(parts["r"], (np.int32, np.int32, np.int32, np.float64))
+        juncs = cat(parts["j"], (np.int32, np.int32, np.int32, np.uint8, np.float64))
+        res = dict(runs=runs, juncs=juncs, n_runs=len(runs[0]), n_juncs=len(juncs[0]), header=hdr, stat=totals)
+        if want_sample:
+            t, s0, e0, v = cat(parts["s"], (np.int32, np.int32, np.int32, np.float64))
+            res["sample"] = (t, s0, e0, v.astype(np.uint64))
+        return res
 
 
-# ---------------------------------------------------------------------------------------------------------------------
-# tiecov over long streams / several GPUs (csrc/shard.cu): thin ctypes plumbing, no logic of its own
-# ---------------------------------------------------------------------------------------------------------------------
 def _cov_in(cols, keep):
     """tc_soa_in for a column dict (numpy or torch); `keep` collects the arrays that must outlive the call."""
     dev = _is_torch(cols["pos"])
@@ -405,27 +524,7 @@ def _rows(out, r, j):
                 juncs=(out["j_tid"][:j], out["j_start"][:j], out["j_end"][:j], out["j_strand"][:j], out["j_val"][:j]), n_runs=r, n_juncs=j)
 
 
-def _coverage_stream(self, cols, window, out, next_tid_pos=None):
-    """tc_coverage_stream: one slice in windows cut at bundle heads. Returns the rows and `consumed`."""
-    keep = []
-    cin = _cov_in(cols, keep)
-    runs, juncs = _out_structs(out)
-    nx = None
-    if next_tid_pos is not None:
-        nx = (C.c_int32 * 2)(int(next_tid_pos[0]), int(next_tid_pos[1]))
-    consumed = C.c_int64(0)
-    rc = self.lib.tc_coverage_stream(self.h, C.byref(cin), int(window), nx, C.byref(runs), C.byref(juncs), C.byref(consumed))
-    if rc == 2:
-        raise ValueError(self._err())
-    if rc != 0:
-        raise TieBrushError(self._err())
-    res = _rows(out, int(runs.n_runs), int(juncs.n_juncs))
-    res["consumed"] = int(consumed.value)
-    res["windows"] = int(self.lib.tc_stream_windows(self.h))
-    return res
-
-
-def _comm_unique_id():
+def comm_unique_id():
     buf = (C.c_ubyte * 128)()
     lib = _lib.load()
     if lib.tb_comm_unique_id(buf) != 0:
@@ -433,88 +532,8 @@ def _comm_unique_id():
     return bytes(buf)
 
 
-def _comm_init(self, rank, world, unique_id):
-    buf = (C.c_ubyte * 128).from_buffer_copy(unique_id)
-    if self.lib.tb_comm_init(self.h, int(rank), int(world), buf) != 0:
-        raise TieBrushError(self._err())
-
-
-def _shard_coverage(self, segs, window, out):
-    """tc_shard_coverage over this rank's device-resident segments (list of column dicts). Collective."""
-    keep = []
-    arr = (_lib.CovIn * len(segs))(*[_cov_in(s, keep) for s in segs])
-    runs, juncs = _out_structs(out)
-    rc = self.lib.tc_shard_coverage(self.h, arr, len(segs), int(window), C.byref(runs), C.byref(juncs))
-    if rc == 2:
-        raise ValueError(self._err())
-    if rc != 0:
-        raise TieBrushError(self._err())
-    res = _rows(out, int(runs.n_runs), int(juncs.n_juncs))
-    res["windows"] = int(self.lib.tc_stream_windows(self.h))
-    res["stats"] = dict(zip(("lead_received", "lead_sent", "ranks_received_from", "halo_bytes_sent", "seam_records"),
-                            (int(self.lib.tc_shard_stat(self.h, i)) for i in range(5))))
-    return res
-
-
-def _shard_gather(self, local, all_out, world):
-    """tc_shard_gather: ordered gather of `local` (result of shard_coverage, device rows) into `all_out` on rank 0. Collective."""
-    lr = _lib.RunsOut(int(local["n_runs"]), int(local["n_runs"]), *[_ptr(a) for a in local["runs"]], 1)
-    lj = _lib.JuncsOut(int(local["n_juncs"]), int(local["n_juncs"]), *[_ptr(a) for a in local["juncs"]], 1)
-    base = (C.c_int64 * (world + 1))()
-    if all_out is not None:
-        ar, aj = _out_structs(all_out)
-        rc = self.lib.tc_shard_gather(self.h, C.byref(lr), C.byref(lj), C.byref(ar), C.byref(aj), base)
-    else:
-        rc = self.lib.tc_shard_gather(self.h, C.byref(lr), C.byref(lj), None, None, base)
-    if rc != 0:
-        raise TieBrushError(self._err())
-    res = dict(junc_base=[int(x) for x in base], gather_bytes=int(self.lib.tc_shard_stat(self.h, 5)))
-    if all_out is not None:
-        res.update(_rows(all_out, int(ar.n_runs), int(aj.n_juncs)))
-    return res
-
-
-def _shard_coverage_gather(self, segs, window, out, all_out, cap_runs_all, cap_juncs_all, world):
-    """tc_shard_coverage_gather: this rank's windows with the ordered gather on rank 0 overlapped (one round per window on a
-    second stream). `all_out` = rank 0's arrays (capacity cap_*_all, cut into `world` regions), None elsewhere; every rank
-    passes the same capacities. Returns the local rows, the regions [(runs offset, runs, juncs offset, juncs)] and, on rank 0,
-    the gathered rows per region."""
-    keep = []
-    arr = (_lib.CovIn * len(segs))(*[_cov_in(s, keep) for s in segs])
-    runs, juncs = _out_structs(out)
-    if all_out is not None:
-        ar, aj = _out_structs(all_out)
-        ar.capacity, aj.capacity = int(cap_runs_all), int(cap_juncs_all)
-    else:
-        ar = _lib.RunsOut(int(cap_runs_all), 0, None, None, None, None, 1)
-        aj = _lib.JuncsOut(int(cap_juncs_all), 0, None, None, None, None, None, 1)
-    region = (C.c_int64 * (4 * world))()
-    rc = self.lib.tc_shard_coverage_gather(self.h, arr, len(segs), int(window), C.byref(runs), C.byref(juncs), C.byref(ar), C.byref(aj), region)
-    if rc == 2:
-        raise ValueError(self._err())
-    if rc != 0:
-        raise TieBrushError(self._err())
-    res = _rows(out, int(runs.n_runs), int(juncs.n_juncs))
-    res["windows"] = int(self.lib.tc_stream_windows(self.h))
-    res["stats"] = dict(zip(("lead_received", "lead_sent", "ranks_received_from", "halo_bytes_sent", "seam_records", "gather_bytes", "gather_rounds"),
-                            (int(self.lib.tc_shard_stat(self.h, i)) for i in range(7))))
-    res["regions"] = [tuple(int(region[4 * r + q]) for q in range(4)) for r in range(world)]
-    res["total_runs"] = sum(x[1] for x in res["regions"]); res["total_juncs"] = sum(x[3] for x in res["regions"])
-    if all_out is not None:
-        cat = lambda keys, oi, ci: tuple((torch_cat if _is_torch(all_out[keys[0]]) else np.concatenate)([all_out[kk][x[oi]:x[oi] + x[ci]] for x in res["regions"]]) for kk in keys)
-        import functools
-        try:
-            import torch
-            torch_cat = torch.cat
-        except Exception:   # pragma: no cover
-            torch_cat = None
-        res["gathered_runs"] = lambda: cat(("r_tid", "r_start", "r_end", "r_val"), 0, 1)
-        res["gathered_juncs"] = lambda: cat(("j_tid", "j_start", "j_end", "j_strand", "j_val"), 2, 3)
-    return res
-
-
 # ---------------------------------------------------------------------------------------------------------------------
-# tiecov straight from BAM bytes (csrc/bgzf.cu): BGZF inflate and record parse on the device
+# tiecov straight from BAM bytes (csrc/bgzf.cu): host helpers
 # ---------------------------------------------------------------------------------------------------------------------
 def _bgzf_blocks(f):
     """(byte offset, inflated bytes) of every BGZF block of an open binary file, from its current position (host zlib)."""
@@ -596,95 +615,3 @@ def _stat(st):
 class _DevArray:   # a device pointer as a torch-importable array (zero copy; cloned at once)
     def __init__(self, ptr, n, typestr):
         self.__cuda_array_interface__ = dict(shape=(n,), typestr=typestr, data=(ptr or 0, False), version=2)
-
-
-def _bam_columns(self, data, skip=0, last=True):
-    """tc_bam_columns: the tiecov columns of the complete records in `data` (bytes of whole or partial BGZF blocks; the
-    records start `skip` inflated bytes into the first block) as torch tensors on this context's device (copies: the
-    library's buffers are reused by the next call). Returns (cols, stat); stat["resume_byte"] / ["resume_skip"] tell where
-    the next chunk starts."""
-    import torch
-    bi, keep = _bgzf_in(data, skip, 1, last)
-    cin, yx, st = _lib.CovIn(), C.c_void_p(), _lib.BgzfStat()
-    if self.lib.tc_bam_columns(self.h, C.byref(bi), C.byref(cin), C.byref(yx), C.byref(st)) != 0:
-        raise TieBrushError(self._err())
-    n = int(cin.n)
-    dev = torch.device("cuda", self.device)
-    with torch.cuda.device(dev):
-        t = lambda p, m, ts: torch.as_tensor(_DevArray(p, m, ts), device=dev).clone() if m else torch.empty(0, dtype={"<i4": torch.int32, "<f4": torch.float32, "|u1": torch.uint8}[ts], device=dev)
-        cols = dict(tid=t(cin.tid, n, "<i4"), pos=t(cin.pos, n, "<i4"), end=t(cin.end, n, "<i4"), yc=t(cin.yc, n, "<f4"), yx=t(yx.value, n, "<i4"),
-                    strand=t(cin.strand, n, "|u1"), cig_off=t(cin.cig_off, n + 1, "<i4"), cigar=t(cin.cigar, int(cin.n_cig), "<i4"))
-    cols["n_cig"] = int(cin.n_cig)
-    return cols, _stat(st)
-
-
-def _coverage_bam(self, path, want_runs=True, want_juncs=True, want_sample=False, chunk_bytes=16 << 20, window=1 << 22):
-    """tiecov -c / -j / -s of a BAM file, read in chunks of `chunk_bytes` and decoded on the device (tc_coverage_bam).
-    Returns dict(runs, juncs, n_runs, n_juncs) like coverage_window, plus sample=(tid, start0, end0, ival) when want_sample
-    (the rows of sample_window), header (read_bam_header) and stat (totals over the chunks)."""
-    hdr = read_bam_header(path)
-    parts = dict(r=[], j=[], s=[])
-    totals = dict(blocks=0, bytes_in=0, bytes_out=0, records=0, unmapped=0, chunks=0)
-    cap = 1 << 16
-    out = srow = None
-    with open(path, "rb") as f:
-        f.seek(hdr["block_offset"])
-        pending, skip, first, eof = b"", hdr["skip"], 1, False
-        while True:
-            new = b"" if eof else f.read(chunk_bytes)
-            eof = eof or len(new) < chunk_bytes
-            data = pending + new
-            last = eof
-            while True:
-                if out is None:
-                    out = cov_out_buffers(cap, cap)
-                    srow = cov_out_buffers(cap, 1)
-                runs, juncs = _out_structs(out)
-                sr, _ = _out_structs(srow)
-                bi, keep = _bgzf_in(data, skip, first, last)
-                st = _lib.BgzfStat()
-                rc = self.lib.tc_coverage_bam(self.h, C.byref(bi), int(window), C.byref(runs) if want_runs else None,
-                                              C.byref(juncs) if want_juncs else None, C.byref(sr) if want_sample else None, C.byref(st))
-                if rc == 5:
-                    cap = max(2 * cap, int(st.need_rows))
-                    out = None
-                    continue
-                if rc == 2:
-                    raise ValueError(self._err())
-                if rc != 0:
-                    raise TieBrushError(self._err())
-                break
-            r, j, ns = int(runs.n_runs), int(juncs.n_juncs), int(sr.n_runs)
-            if r:
-                parts["r"].append(tuple(out[k][:r].copy() for k in ("r_tid", "r_start", "r_end", "r_val")))
-            if j:
-                parts["j"].append(tuple(out[k][:j].copy() for k in ("j_tid", "j_start", "j_end", "j_strand", "j_val")))
-            if ns:
-                parts["s"].append(tuple(srow[k][:ns].copy() for k in ("r_tid", "r_start", "r_end", "r_val")))
-            s = _stat(st)
-            for k in ("blocks", "bytes_in", "bytes_out", "records", "unmapped"):
-                totals[k] += s[k]
-            totals["chunks"] += 1
-            first = 0
-            if last:
-                break
-            pending, skip = data[s["resume_byte"]:], s["resume_skip"]
-    cat = lambda xs, dts: tuple(np.concatenate([x[i] for x in xs]) if xs else np.zeros(0, dt) for i, dt in enumerate(dts))
-    runs = cat(parts["r"], (np.int32, np.int32, np.int32, np.float64))
-    juncs = cat(parts["j"], (np.int32, np.int32, np.int32, np.uint8, np.float64))
-    res = dict(runs=runs, juncs=juncs, n_runs=len(runs[0]), n_juncs=len(juncs[0]), header=hdr, stat=totals)
-    if want_sample:
-        t, s0, e0, v = cat(parts["s"], (np.int32, np.int32, np.int32, np.float64))
-        res["sample"] = (t, s0, e0, v.astype(np.uint64))
-    return res
-
-
-Context.bam_columns = _bam_columns
-Context.coverage_bam = _coverage_bam
-Context.coverage_stream = _coverage_stream
-Context.shard_coverage_gather = _shard_coverage_gather
-Context.comm_init = _comm_init
-Context.shard_coverage = _shard_coverage
-Context.shard_gather = _shard_gather
-Context.last_cov_exact = lambda self: int(self.lib.tc_last_exact(self.h))
-comm_unique_id = _comm_unique_id

@@ -19,7 +19,7 @@
 // every read and write against their buffers whatever the bytes say, and never trap.
 #include <functional>
 #include <algorithm>
-#include "tb_common.cuh"
+#include "tc_columns.cuh"
 
 int tc_stream_impl(tb_ctx* ctx, const tc_soa_in* in, int64_t skip, int64_t window, const int32_t* next, tc_runs_out* runs, tc_juncs_out* juncs,
                    int64_t* consumed, const std::function<int()>* after_window, const int32_t* yx);
@@ -36,11 +36,10 @@ enum {   // ctx->bam_buf slots
   BZ_ROFF,       // i64 [records] uncompressed offset of every record
   BZ_REC,        // Rec [records]
   BZ_STATUS,     // u64 [8]
-  BZ_COLS,       // two column sets (ping-pong for tc_coverage_bam's held bundle): 8 slots each from here
+  BZ_COLS,       // two record sets (ping-pong for tc_coverage_bam's held bundle): 8 slots each from here (tc_alloc_records)
   BZ_COUNT_ = BZ_COLS + 16
 };
 static_assert((int)BZ_COUNT_ <= (int)TB_NBAMBUF, "bam_buf too small");
-enum { C_TID = 0, C_POS, C_END, C_YC, C_YX, C_STRAND, C_CIGOFF, C_CIGAR };
 // status words
 enum { S_INFLATE = 0, S_WALK, S_PARSE, S_BREAK, S_TAIL, S_UNMAPPED, S_N_ };
 // inflate error codes
@@ -447,11 +446,9 @@ __global__ void __launch_bounds__(256) parse_kernel(const uint8_t* __restrict__ 
   rec[i] = o;
 }
 
-struct Cols { int32_t *tid, *pos, *end, *yx; float* yc; uint8_t* strand; uint32_t *cig_off, *cigar; };
-
 struct KeepIn { const Rec* rec; __device__ long long operator()(int64_t i) const { return rec[i].kept ? (1LL << 32) | (long long)rec[i].ncig : 0LL; } };
 struct KeepOut {   // places record i's columns and CIGAR words after the `held` records already in the set
-  const Rec* rec; const uint8_t* u; Cols c; int64_t held; uint32_t held_cig; int64_t n;
+  const Rec* rec; const uint8_t* u; TcRecords c; int64_t held; uint32_t held_cig; int64_t n;
   __device__ void operator()(int64_t i, long long exc, long long inc) const {
     const Rec& x = rec[i];
     if (x.kept) {
@@ -463,19 +460,6 @@ struct KeepOut {   // places record i's columns and CIGAR words after the `held`
     if (i == n - 1) c.cig_off[held + (inc >> 32)] = held_cig + (uint32_t)(inc & 0xffffffffLL);
   }
 };
-
-// the held bundle: records [from, n) of set `a` to the front of set `b`, CIGAR offsets rebased
-__global__ void carry_kernel(Cols a, Cols b, int64_t from, int64_t m, uint32_t cbase, uint32_t ncig) {
-  for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < m || k < (int64_t)ncig; k += (int64_t)gridDim.x * blockDim.x) {
-    if (k < m) {
-      const int64_t s = from + k;
-      b.tid[k] = a.tid[s]; b.pos[k] = a.pos[s]; b.end[k] = a.end[s]; b.yc[k] = a.yc[s]; b.yx[k] = a.yx[s]; b.strand[k] = a.strand[s];
-      b.cig_off[k] = a.cig_off[s] - cbase;
-    }
-    if (k < (int64_t)ncig) b.cigar[k] = a.cigar[cbase + k];
-    if (k == 0) b.cig_off[m] = ncig;
-  }
-}
 
 const char* inflate_msg(int code) {
   switch (code) {
@@ -499,7 +483,12 @@ const char* parse_msg(int code) {
   }
 }
 
-static inline unsigned grid_of(int64_t n, int t) { return (unsigned)((n + t - 1) / t); }
+// record set k of ctx->bam_buf, as sized by the last bam_decode that wrote it
+TcRecords column_set(tb_ctx* ctx, int k) {
+  TcRecords c;
+  tc_alloc_records(ctx->bam_buf + BZ_COLS + 8 * k, 0, 0, true, &c);
+  return c;
+}
 
 }  // namespace
 
@@ -579,7 +568,7 @@ static int bam_decode(tb_ctx* ctx, const tb_bgzf_in* in, int64_t held, const cha
     h_st[S_INFLATE] = h_st[S_WALK] = h_st[S_PARSE] = h_st[S_BREAK] = ~0ull;
     TB_CUDA(cudaMemcpyAsync(d_st, h_st, sizeof(unsigned long long) * 8, cudaMemcpyHostToDevice, s));
     if (ctx->profiling) TB_CUDA(cudaEventRecord(ctx->ev[14], s));
-    bgzf_inflate_kernel<<<grid_of(nb, INF_WARPS), INF_THREADS, 0, s>>>(B[BZ_COMP].as<uint8_t>(), B[BZ_BLK].as<BlkDesc>(), nb, B[BZ_U].as<uint8_t>(), d_st);
+    bgzf_inflate_kernel<<<tb_grid_for(nb, INF_WARPS), INF_THREADS, 0, s>>>(B[BZ_COMP].as<uint8_t>(), B[BZ_BLK].as<BlkDesc>(), nb, B[BZ_U].as<uint8_t>(), d_st);
     ctx->launches++;
     TB_CUDA(cudaGetLastError());
     if (ctx->profiling) TB_CUDA(cudaEventRecord(ctx->ev[15], s));
@@ -595,7 +584,7 @@ static int bam_decode(tb_ctx* ctx, const tb_bgzf_in* in, int64_t held, const cha
     TB_CUDA(B[BZ_WALK].ensure(sizeof(Walk) * nb));
     TB_CUDA(B[BZ_RBASE].ensure(sizeof(uint32_t) * (nb + 1)));
     Walk* walk = B[BZ_WALK].as<Walk>();
-    walk_guess_kernel<<<grid_of(nb, 128), 128, 0, s>>>(du, U, B[BZ_BLK].as<BlkDesc>(), nb, in->skip, walk, d_st);
+    walk_guess_kernel<<<tb_grid_for(nb, 128), 128, 0, s>>>(du, U, B[BZ_BLK].as<BlkDesc>(), nb, in->skip, walk, d_st);
     walk_fix_kernel<<<1, 1, 0, s>>>(du, U, B[BZ_BLK].as<BlkDesc>(), nb, walk, d_st);
     ctx->launches += 2;
     TB_CUDA(B[BZ_AGG].ensure(sizeof(long long) * (tb_scan_blocks(nb) + 8)));
@@ -626,8 +615,8 @@ static int bam_decode(tb_ctx* ctx, const tb_bgzf_in* in, int64_t held, const cha
   if (nrec > 0) {
     TB_CUDA(B[BZ_ROFF].ensure(sizeof(int64_t) * nrec));
     TB_CUDA(B[BZ_REC].ensure(sizeof(Rec) * nrec));
-    record_offsets_kernel<<<grid_of(nb, 128), 128, 0, s>>>(du, B[BZ_WALK].as<Walk>(), B[BZ_RBASE].as<uint32_t>(), nb, B[BZ_ROFF].as<int64_t>());
-    parse_kernel<<<grid_of(nrec, 256), 256, 0, s>>>(du, B[BZ_ROFF].as<int64_t>(), nrec, B[BZ_REC].as<Rec>(), d_st);
+    record_offsets_kernel<<<tb_grid_for(nb, 128), 128, 0, s>>>(du, B[BZ_WALK].as<Walk>(), B[BZ_RBASE].as<uint32_t>(), nb, B[BZ_ROFF].as<int64_t>());
+    parse_kernel<<<tb_grid_for(nrec, 256), 256, 0, s>>>(du, B[BZ_ROFF].as<int64_t>(), nrec, B[BZ_REC].as<Rec>(), d_st);
     ctx->launches += 2;
     TB_CUDA(cudaGetLastError());
     TB_CUDA(cudaMemcpyAsync(h_st, d_st, sizeof(unsigned long long) * 8, cudaMemcpyDeviceToHost, s));
@@ -648,21 +637,9 @@ static int bam_decode(tb_ctx* ctx, const tb_bgzf_in* in, int64_t held, const cha
   const uint32_t held_cig = held > 0 ? ctx->bam_hcig : 0;
   const int64_t cap_cig = (int64_t)held_cig + U / 4 + 1;
   if (cap_cig >= (1LL << 32)) { ctx->set_error("%s: %lld CIGAR words exceed the 32-bit offsets of one column set (pass smaller chunks)", fn, (long long)cap_cig); return 1; }
-  DevBuf* S = B + BZ_COLS + 8 * set;
-  const size_t cap = (size_t)(held + nrec) + 1;
-  TB_CUDA(S[C_TID].ensure(4 * cap)); TB_CUDA(S[C_POS].ensure(4 * cap)); TB_CUDA(S[C_END].ensure(4 * cap)); TB_CUDA(S[C_YC].ensure(4 * cap));
-  TB_CUDA(S[C_YX].ensure(4 * cap)); TB_CUDA(S[C_STRAND].ensure(cap)); TB_CUDA(S[C_CIGOFF].ensure(4 * cap)); TB_CUDA(S[C_CIGAR].ensure(4 * (size_t)cap_cig));
-  auto cols_of = [&](int k) {
-    DevBuf* X = B + BZ_COLS + 8 * k;
-    return Cols{X[C_TID].as<int32_t>(), X[C_POS].as<int32_t>(), X[C_END].as<int32_t>(), X[C_YX].as<int32_t>(), X[C_YC].as<float>(), X[C_STRAND].as<uint8_t>(),
-                X[C_CIGOFF].as<uint32_t>(), X[C_CIGAR].as<uint32_t>()};
-  };
-  const Cols c = cols_of(set);
-  if (held > 0) {
-    const int64_t work = std::max<int64_t>(held, held_cig);
-    carry_kernel<<<(unsigned)std::min<int64_t>((work + 255) / 256, 4096), 256, 0, s>>>(cols_of(ctx->bam_set), c, ctx->bam_from, held, ctx->bam_cbase, held_cig);
-    ctx->launches++;
-  }
+  TcRecords c;
+  TB_CUDA(tc_alloc_records(B + BZ_COLS + 8 * set, held + nrec + 1, cap_cig, true, &c));
+  if (held > 0) tc_copy_records(ctx, s, column_set(ctx, ctx->bam_set), ctx->bam_from, held, c, 0, 0, held_cig);
   long long tot = 0;
   if (nrec > 0) {
     TB_CUDA(B[BZ_AGG].ensure(sizeof(long long) * (tb_scan_blocks(nrec) + 8)));
@@ -681,11 +658,9 @@ static int bam_decode(tb_ctx* ctx, const tb_bgzf_in* in, int64_t held, const cha
 }
 
 static void set_columns(tb_ctx* ctx, int set, int64_t n, uint32_t ncig, tc_soa_in* cols, const int32_t** yx) {
-  DevBuf* X = ctx->bam_buf + BZ_COLS + 8 * set;
-  memset(cols, 0, sizeof(*cols));
-  cols->n = n; cols->tid = X[C_TID].as<int32_t>(); cols->pos = X[C_POS].as<int32_t>(); cols->yc = X[C_YC].as<float>(); cols->strand = X[C_STRAND].as<uint8_t>();
-  cols->cig_off = X[C_CIGOFF].as<uint32_t>(); cols->cigar = X[C_CIGAR].as<uint32_t>(); cols->on_device = 1; cols->n_cig = ncig; cols->end = X[C_END].as<int32_t>();
-  if (yx) *yx = X[C_YX].as<int32_t>();
+  const TcRecords c = column_set(ctx, set);
+  *cols = tc_window(c, n, ncig);
+  if (yx) *yx = c.yx;
 }
 
 extern "C" {

@@ -18,7 +18,7 @@
 // Weights: YC is float32 on disk (SURVEY §9.5); the reference accumulates doubles. Here every weight is
 // converted once to 2^-20 fixed point (exact for all integer-valued YC and for dyadic fractions) and
 // summed in int64, which equals the reference's double sum whenever that sum is exact.
-#include "tb_common.cuh"
+#include "tc_columns.cuh"
 
 namespace {
 
@@ -883,17 +883,6 @@ __global__ void __launch_bounds__(128) junc_exact_kernel(CovIn in, int64_t NB, c
   o_val[k] = sum;
 }
 
-static inline unsigned grid_for(int64_t n, int threads) { return (unsigned)((n + threads - 1) / threads); }
-
-template <class T>
-static int stage_in(tb_ctx* ctx, DevBuf& b, const T* src, size_t count, int on_device, const T** out) {
-  if (on_device || src == nullptr) { *out = src; return 0; }
-  TB_CUDA(b.ensure(count * sizeof(T) + 16));
-  TB_CUDA(cudaMemcpyAsync(b.p, src, count * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));
-  *out = (const T*)b.p;
-  return 0;
-}
-
 }  // namespace
 
 int tc_coverage_impl(tb_ctx* ctx, const tc_soa_in* hin, tc_runs_out* runs, tc_juncs_out* juncs, const int32_t* yx_in, CovExt* ext) {
@@ -908,25 +897,11 @@ int tc_coverage_impl(tb_ctx* ctx, const tc_soa_in* hin, tc_runs_out* runs, tc_ju
   cudaStream_t st = ctx->stream;
 
   // ---- inputs on the device ----
-  CovIn in; in.n = n;
-  int64_t ncig = hin->n_cig;
-  if (stage_in(ctx, ctx->in_stage[0], hin->tid, (size_t)n, hin->on_device, &in.tid)) return 1;
-  if (stage_in(ctx, ctx->in_stage[1], hin->pos, (size_t)n, hin->on_device, &in.pos)) return 1;
-  if (stage_in(ctx, ctx->in_stage[2], hin->yc, (size_t)n, hin->on_device, &in.yc)) return 1;
-  if (stage_in(ctx, ctx->in_stage[3], hin->strand, (size_t)n, hin->on_device, &in.strand)) return 1;
-  if (stage_in(ctx, ctx->in_stage[4], hin->cig_off, (size_t)n + 1, hin->on_device, &in.cig_off)) return 1;
-  {
-    // host arrays: a window of a longer stream keeps its absolute CIGAR offsets (tc_coverage_stream): copy the window's
-    // words only and bias the device pointer so that cigar[cig_off[i]] still lands on them
-    const uint32_t cbase = (!hin->on_device && n > 0) ? hin->cig_off[0] : 0u;
-    const uint32_t* staged = nullptr;
-    if (stage_in(ctx, ctx->in_stage[5], hin->cigar ? hin->cigar + cbase : nullptr, (size_t)ncig, hin->on_device, &staged)) return 1;
-    in.cigar = staged - cbase;
-  }
-  in.end = nullptr;
-  if (hin->end) { if (stage_in(ctx, ctx->in_stage[7], hin->end, (size_t)n, hin->on_device, &in.end)) return 1; }
+  tc_soa_in win;
   const int32_t* d_yx = nullptr;
-  if (sample) { if (stage_in(ctx, ctx->in_stage[6], yx_in, (size_t)n, hin->on_device, &d_yx)) return 1; }
+  if (tc_stage_window(ctx, ctx->in_stage, *hin, yx_in, &win, &d_yx)) return 1;
+  CovIn in{n, win.tid, win.pos, win.yc, win.strand, win.cig_off, win.cigar, win.end};
+  const int64_t ncig = hin->n_cig;
 
   DevBuf* B = ctx->buf;
   TB_CUDA(B[CB_RFIRST].ensure(sizeof(uint32_t) * n));
@@ -1057,7 +1032,7 @@ int tc_coverage_impl(tb_ctx* ctx, const tc_soa_in* hin, tc_runs_out* runs, tc_ju
     if (L >= (1LL << 32)) { ctx->set_error("tc_coverage_window: %lld cells do not fit the 32-bit item lists (smaller windows)", (long long)L); return 1; }
     TB_CUDA(B[CB_IOFF].ensure(sizeof(uint32_t) * (n + 2)));
     uint32_t* ioff = B[CB_IOFF].as<uint32_t>();
-    ow_items_kernel<false><<<grid_for(n, 256), 256, 0, st>>>(in, B[CB_BID].as<uint32_t>(), B[CB_BSTART].as<int32_t>(), B[CB_BBASE].as<long long>(), ioff,
+    ow_items_kernel<false><<<tb_grid_for(n, 256), 256, 0, st>>>(in, B[CB_BID].as<uint32_t>(), B[CB_BSTART].as<int32_t>(), B[CB_BBASE].as<long long>(), ioff,
                                                             nullptr, nullptr, nullptr, nullptr, nullptr);
     TB_CUDA(B[CB_AGG].ensure((size_t)(tb_scan_blocks(n) + 8) * sizeof(SumNz)));
     TB_CUDA((tb_device_scan<OpSumU32>(ctx, IcntIn{ioff}, n, B[CB_AGG].as<uint32_t>(), IoffOut{ioff, n})));
@@ -1069,7 +1044,7 @@ int tc_coverage_impl(tb_ctx* ctx, const tc_soa_in* hin, tc_runs_out* runs, tc_ju
     TB_CUDA(B[CB_IKEY].ensure(sizeof(uint64_t) * nalloc)); TB_CUDA(B[CB_IKEY2].ensure(sizeof(uint64_t) * nalloc));
     TB_CUDA(B[CB_IVAL].ensure(sizeof(uint32_t) * nalloc)); TB_CUDA(B[CB_IVAL2].ensure(sizeof(uint32_t) * nalloc));
     TB_CUDA(B[CB_ILO].ensure(sizeof(uint32_t) * nalloc)); TB_CUDA(B[CB_IHI].ensure(sizeof(uint32_t) * nalloc)); TB_CUDA(B[CB_IREC].ensure(sizeof(uint32_t) * nalloc));
-    ow_items_kernel<true><<<grid_for(n, 256), 256, 0, st>>>(in, B[CB_BID].as<uint32_t>(), B[CB_BSTART].as<int32_t>(), B[CB_BBASE].as<long long>(), ioff,
+    ow_items_kernel<true><<<tb_grid_for(n, 256), 256, 0, st>>>(in, B[CB_BID].as<uint32_t>(), B[CB_BSTART].as<int32_t>(), B[CB_BBASE].as<long long>(), ioff,
                                                            B[CB_IKEY].as<unsigned long long>(), B[CB_IVAL].as<uint32_t>(), B[CB_ILO].as<uint32_t>(),
                                                            B[CB_IHI].as<uint32_t>(), B[CB_IREC].as<uint32_t>());
     ctx->launches += 2;
@@ -1100,7 +1075,7 @@ int tc_coverage_impl(tb_ctx* ctx, const tc_soa_in* hin, tc_runs_out* runs, tc_ju
       TB_CUDA(B[CB_JVAL].ensure(sizeof(int64_t) * jcap));
       jt.key = B[CB_JTAG].as<unsigned long long>(); jt.tid = B[CB_JTID].as<int32_t>(); jt.val = B[CB_JVAL].as<long long>();
       jt.mask = jcap - 1; jt.seed = seed;
-      junc_init_kernel<<<grid_for(jcap, 256), 256, 0, st>>>(jt, jcap);
+      junc_init_kernel<<<tb_grid_for(jcap, 256), 256, 0, st>>>(jt, jcap);
       ctx->launches++;
     }
     if (acc_cov) {
@@ -1109,7 +1084,7 @@ int tc_coverage_impl(tb_ctx* ctx, const tc_soa_in* hin, tc_runs_out* runs, tc_ju
     }
     // ---- K7 (+K9 insert): the dominant kernel ----
     if (ctx->profiling && !cells) TB_CUDA(cudaEventRecord(ctx->ev[0], st));
-    cov_accumulate_kernel<<<grid_for(n, COV_THREADS * COV_RPT), COV_THREADS, 0, st>>>(in, B[CB_BID].as<uint32_t>(), B[CB_BSTART].as<int32_t>(), B[CB_BBASE].as<long long>(),
+    cov_accumulate_kernel<<<tb_grid_for(n, COV_THREADS * COV_RPT), COV_THREADS, 0, st>>>(in, B[CB_BID].as<uint32_t>(), B[CB_BSTART].as<int32_t>(), B[CB_BBASE].as<long long>(),
                                                            B[CB_DIFF].as<long long>(), acc_cov, do_junc, jt, d_status, (has_end && do_cov) ? 1 : 0);
     ctx->launches++;
     if (ctx->profiling && !cells) TB_CUDA(cudaEventRecord(ctx->ev[1], st));
@@ -1126,6 +1101,7 @@ int tc_coverage_impl(tb_ctx* ctx, const tc_soa_in* hin, tc_runs_out* runs, tc_ju
   }
 
   // ---- K8 ----
+  tc_runs_out d_runs = runs ? *runs : tc_runs_out{};   // where the rows are written: the caller's device arrays or out_stage
   if (ctx->profiling) TB_CUDA(cudaEventRecord(ctx->ev[10], st));
   if (do_cov) {
     // change points: at most one per non-zero difference cell, and no more than two per M block
@@ -1152,18 +1128,11 @@ int tc_coverage_impl(tb_ctx* ctx, const tc_soa_in* hin, tc_runs_out* runs, tc_ju
     }
     const int64_t K = h_status[ST_NCHANGE];
     // output staging
-    int64_t cap = runs->capacity;
-    int32_t *o_tid = runs->tid, *o_start = runs->start0, *o_end = runs->end0; double* o_val = runs->value;
-    int64_t stage_cap = cap < K ? cap : K;
+    int64_t stage_cap = runs->capacity < K ? runs->capacity : K;
     if (stage_cap < 1) stage_cap = 1;
-    if (!runs->on_device) {
-      TB_CUDA(ctx->out_stage[0].ensure(sizeof(int32_t) * stage_cap)); TB_CUDA(ctx->out_stage[1].ensure(sizeof(int32_t) * stage_cap));
-      TB_CUDA(ctx->out_stage[2].ensure(sizeof(int32_t) * stage_cap)); TB_CUDA(ctx->out_stage[3].ensure(sizeof(double) * stage_cap));
-      o_tid = ctx->out_stage[0].as<int32_t>(); o_start = ctx->out_stage[1].as<int32_t>(); o_end = ctx->out_stage[2].as<int32_t>();
-      o_val = ctx->out_stage[3].as<double>();
-    }
+    if (!runs->on_device) TB_CUDA(tc_alloc_rows(ctx->out_stage, d_runs, stage_cap));
     RunOut ro{cppos, cpdepth, d_status, B[CB_BBASE].as<long long>(), B[CB_BSTART].as<int32_t>(), B[CB_BTID].as<int32_t>(),
-              o_tid, o_start, o_end, o_val, stage_cap, sample ? 1.0 : (cells ? 0.0 : COV_FX_SCALE)};
+              d_runs.tid, d_runs.start0, d_runs.end0, d_runs.value, stage_cap, sample ? 1.0 : (cells ? 0.0 : COV_FX_SCALE)};
     TB_CUDA((tb_device_scan<OpSumU32>(ctx, RunValidIn{cpdepth, d_status}, K, B[CB_AGG].as<uint32_t>(), ro)));
     cov_store_total_kernel<<<1, 1, 0, st>>>(nullptr, B[CB_AGG].as<uint32_t>() + tb_scan_blocks(K), d_status);
     ctx->launches++;
@@ -1183,13 +1152,7 @@ int tc_coverage_impl(tb_ctx* ctx, const tc_soa_in* hin, tc_runs_out* runs, tc_ju
       return 1;
     }
     runs->n_runs = h_status[ST_NRUNS];
-    if (!runs->on_device && runs->n_runs > 0) {
-      size_t r = (size_t)runs->n_runs;
-      TB_CUDA(cudaMemcpyAsync(runs->tid, ctx->out_stage[0].p, sizeof(int32_t) * r, cudaMemcpyDeviceToHost, st));
-      TB_CUDA(cudaMemcpyAsync(runs->start0, ctx->out_stage[1].p, sizeof(int32_t) * r, cudaMemcpyDeviceToHost, st));
-      TB_CUDA(cudaMemcpyAsync(runs->end0, ctx->out_stage[2].p, sizeof(int32_t) * r, cudaMemcpyDeviceToHost, st));
-      TB_CUDA(cudaMemcpyAsync(runs->value, ctx->out_stage[3].p, sizeof(double) * r, cudaMemcpyDeviceToHost, st));
-    }
+    TB_CUDA(tc_copy_rows(*runs, d_runs, runs->n_runs, cudaMemcpyDeviceToHost, st));
   }
   // ---- K9 extraction: compact, verify, sort (start,end,strand) then stable by tid ----
   if (do_junc) {
@@ -1203,37 +1166,28 @@ int tc_coverage_impl(tb_ctx* ctx, const tc_soa_in* hin, tc_runs_out* runs, tc_ju
       TB_CUDA(B[CB_RSAGG].ensure(sizeof(uint32_t) * tb_radix_agg_elems(J)));
       unsigned long long* counter = (unsigned long long*)(d_status + ST_N_);
       TB_CUDA(cudaMemsetAsync(counter, 0, sizeof(unsigned long long), st));
-      junc_compact_kernel<<<grid_for(jcap, 256), 256, 0, st>>>(jt, jcap, B[CB_JKEYS].as<unsigned long long>(), B[CB_JIDX].as<uint32_t>(), counter, d_status);
+      junc_compact_kernel<<<tb_grid_for(jcap, 256), 256, 0, st>>>(jt, jcap, B[CB_JKEYS].as<unsigned long long>(), B[CB_JIDX].as<uint32_t>(), counter, d_status);
       ctx->launches++;
       uint64_t* rk; uint32_t* rv;
       TB_CUDA(tb_radix_sort(ctx, B[CB_JKEYS].as<uint64_t>(), B[CB_JIDX].as<uint32_t>(), B[CB_JKEYS2].as<uint64_t>(), B[CB_JIDX2].as<uint32_t>(), J, 0, 64,
                             B[CB_RSTABLE].as<uint32_t>(), B[CB_RSAGG].as<uint32_t>(), &rk, &rv));
       // stable second sort by tid (31 significant bits)
       uint32_t* other_v = (rv == B[CB_JIDX].as<uint32_t>()) ? B[CB_JIDX2].as<uint32_t>() : B[CB_JIDX].as<uint32_t>();
-      junc_tidkey_kernel<<<grid_for(J, 256), 256, 0, st>>>(jt, rv, J, B[CB_TIDKEYS].as<unsigned long long>());
+      junc_tidkey_kernel<<<tb_grid_for(J, 256), 256, 0, st>>>(jt, rv, J, B[CB_TIDKEYS].as<unsigned long long>());
       ctx->launches++;
       uint64_t* rk2; uint32_t* rv2;
       TB_CUDA(tb_radix_sort(ctx, B[CB_TIDKEYS].as<uint64_t>(), rv, B[CB_TIDKEYS2].as<uint64_t>(), other_v, J, 0, 32,
                             B[CB_RSTABLE].as<uint32_t>(), B[CB_RSAGG].as<uint32_t>(), &rk2, &rv2));
-      int32_t *o_tid = juncs->tid, *o_start = juncs->start, *o_end = juncs->end; uint8_t* o_strand = juncs->strand; double* o_val = juncs->value;
-      if (!juncs->on_device) {
-        TB_CUDA(ctx->out_stage[4].ensure(sizeof(int32_t) * 3 * J)); TB_CUDA(ctx->out_stage[5].ensure(J)); TB_CUDA(ctx->out_stage[6].ensure(sizeof(double) * J));
-        o_tid = ctx->out_stage[4].as<int32_t>(); o_start = o_tid + J; o_end = o_start + J; o_strand = ctx->out_stage[5].as<uint8_t>(); o_val = ctx->out_stage[6].as<double>();
-      }
-      junc_emit_kernel<<<grid_for(J, 256), 256, 0, st>>>(jt, rv2, J, o_tid, o_start, o_end, o_strand, o_val);
+      tc_juncs_out o = *juncs;
+      if (!juncs->on_device) TB_CUDA(tc_alloc_rows(ctx->out_stage + 4, o, J));
+      junc_emit_kernel<<<tb_grid_for(J, 256), 256, 0, st>>>(jt, rv2, J, o.tid, o.start, o.end, o.strand, o.value);
       ctx->launches++;
       if (exact) {   // ordered double sums replace the fixed-point values
-        junc_exact_kernel<<<grid_for(J, 128), 128, 0, st>>>(in, NB, B[CB_BTID].as<int32_t>(), B[CB_BSTART].as<int32_t>(), d_rfirst, d_pmend, J,
-                                                           o_tid, o_start, o_end, o_strand, o_val);
+        junc_exact_kernel<<<tb_grid_for(J, 128), 128, 0, st>>>(in, NB, B[CB_BTID].as<int32_t>(), B[CB_BSTART].as<int32_t>(), d_rfirst, d_pmend, J,
+                                                           o.tid, o.start, o.end, o.strand, o.value);
         ctx->launches++;
       }
-      if (!juncs->on_device) {
-        TB_CUDA(cudaMemcpyAsync(juncs->tid, o_tid, sizeof(int32_t) * J, cudaMemcpyDeviceToHost, st));
-        TB_CUDA(cudaMemcpyAsync(juncs->start, o_start, sizeof(int32_t) * J, cudaMemcpyDeviceToHost, st));
-        TB_CUDA(cudaMemcpyAsync(juncs->end, o_end, sizeof(int32_t) * J, cudaMemcpyDeviceToHost, st));
-        TB_CUDA(cudaMemcpyAsync(juncs->strand, o_strand, (size_t)J, cudaMemcpyDeviceToHost, st));
-        TB_CUDA(cudaMemcpyAsync(juncs->value, o_val, sizeof(double) * J, cudaMemcpyDeviceToHost, st));
-      }
+      TB_CUDA(tc_copy_rows(*juncs, o, J, cudaMemcpyDeviceToHost, st));
       TB_CUDA(cudaMemcpyAsync(h_status, d_status, sizeof(int64_t) * 16, cudaMemcpyDeviceToHost, st));
     }
     TB_CUDA(cudaStreamSynchronize(st));

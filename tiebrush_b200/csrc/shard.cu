@@ -21,7 +21,7 @@
 #include <nccl.h>
 #include <algorithm>
 #include <functional>
-#include "tb_common.cuh"
+#include "tc_columns.cuh"
 
 int tc_coverage_impl(tb_ctx* ctx, const tc_soa_in* in, tc_runs_out* runs, tc_juncs_out* juncs, const int32_t* yx, CovExt* ext);
 
@@ -60,10 +60,10 @@ NcclApi g_nccl;
     if (r__ != ncclSuccess) { ctx->set_error("NCCL error %s at %s:%d: %s", #call, __FILE__, __LINE__, g_nccl.GetErrorString(r__)); return 1; } \
   } while (0)
 
-// workspace slots of this file in ctx->shard_buf
-enum { SB_GATHER = 0, SB_SEND, SB_TAIL_TID, SB_TAIL_POS, SB_TAIL_YC, SB_TAIL_STRAND, SB_TAIL_OFF, SB_TAIL_CIG, SB_SEAM_TID, SB_SEAM_POS, SB_SEAM_YC,
-       SB_SEAM_STRAND, SB_SEAM_OFF, SB_SEAM_CIG, SB_GROUND, SB_COUNT_ };
-static_assert(SB_COUNT_ <= 16, "raise tb_ctx::shard_buf");
+// workspace slots of this file in ctx->shard_buf: SB_TAIL (the leads received from the right) and SB_SEAM (the seam window)
+// are record sets of 8 slots each (tc_alloc_records)
+enum { SB_GATHER = 0, SB_SEND, SB_GROUND, SB_TAIL, SB_SEAM = SB_TAIL + 8, SB_COUNT_ = SB_SEAM + 8 };
+static_assert(SB_COUNT_ <= (int)(sizeof(tb_ctx::shard_buf) / sizeof(DevBuf)), "raise tb_ctx::shard_buf");
 
 // ---- open-bundle state of a slice: maximum (tid << 32 | end) key over its records. Only the records of the LAST reference
 // id can hold it (tids never decrease), so a one-thread binary search finds where they start and the reduction reads
@@ -136,22 +136,48 @@ __global__ void __launch_bounds__(1024) shard_lead_head_kernel(int64_t base, int
   }
 }
 
-// offsets src[0..count) of a piece (absolute offsets of whoever filled it) -> dst[i] = src[i] - src[0] + dst0
-__global__ void __launch_bounds__(256) shard_copy_off_kernel(const uint32_t* __restrict__ src, int64_t count, uint32_t dst0, uint32_t* __restrict__ dst) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < count) dst[i] = src[i] - src[0] + dst0;
+// see tc_copy_records. The source's first offset is read here, so a piece whose offsets arrived from another rank needs no
+// host round trip.
+__global__ void __launch_bounds__(256) tc_copy_records_kernel(TcRecords src, int64_t from, int64_t m, TcRecords dst, int64_t r, uint32_t w, uint32_t words) {
+  const uint32_t c0 = src.cig_off[from];
+  for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k <= m || k < (int64_t)words; k += (int64_t)gridDim.x * blockDim.x) {
+    if (k <= m) dst.cig_off[r + k] = src.cig_off[from + k] - c0 + w;
+    if (k < m) {
+      const int64_t s = from + k, d = r + k;
+      if (src.tid && dst.tid) dst.tid[d] = src.tid[s];
+      if (src.pos && dst.pos) dst.pos[d] = src.pos[s];
+      if (src.yc && dst.yc) dst.yc[d] = src.yc[s];
+      if (src.strand && dst.strand) dst.strand[d] = src.strand[s];
+      if (src.end && dst.end) dst.end[d] = src.end[s];
+      if (src.yx && dst.yx) dst.yx[d] = src.yx[s];
+    }
+    if (k < (int64_t)words) dst.cigar[w + k] = src.cigar[c0 + k];
+  }
 }
 
-static inline unsigned grid_for(int64_t n, int threads) { return (unsigned)((n + threads - 1) / threads); }
+// n rows of a column set to (send) or from a peer, one ncclSend / ncclRecv per column the set has; inside the caller's group
+static int nccl_rows(tb_ctx* ctx, const TcCols& c, int64_t n, bool send, int peer, cudaStream_t st) {
+  ncclComm_t comm = (ncclComm_t)ctx->comm;
+  for (int i = 0; i < c.n; ++i) {
+    if (!c.p[i]) continue;
+    if (send) TB_NCCL(g_nccl.Send(c.p[i], (size_t)n * c.size[i], ncclUint8, peer, comm, st));
+    else TB_NCCL(g_nccl.Recv(c.p[i], (size_t)n * c.size[i], ncclUint8, peer, comm, st));
+  }
+  return 0;
+}
 
-// sub-window [w0, w0 + len) of a slice as its own tc_soa_in (absolute CIGAR offsets are kept)
-static tc_soa_in sub_window(const tc_soa_in& in, int64_t w0, int64_t len, int64_t words) {
-  tc_soa_in s = in;
-  s.n = len;
-  s.tid = in.tid + w0; s.pos = in.pos + w0; s.yc = in.yc + w0; s.strand = in.strand + w0; s.cig_off = in.cig_off + w0;
-  s.end = in.end ? in.end + w0 : nullptr;
-  s.n_cig = words;
-  return s;
+// n records to or from a peer: the row columns, the n + 1 offsets at c.cig_off, then `words` CIGAR words at c.cigar
+static int nccl_records(tb_ctx* ctx, const TcRecords& c, int64_t n, int64_t words, bool send, int peer, cudaStream_t st) {
+  if (nccl_rows(ctx, tc_cols(c), n, send, peer, st)) return 1;
+  ncclComm_t comm = (ncclComm_t)ctx->comm;
+  if (send) {
+    TB_NCCL(g_nccl.Send(c.cig_off, (size_t)(n + 1) * 4, ncclUint8, peer, comm, st));
+    TB_NCCL(g_nccl.Send(c.cigar, (size_t)words * 4, ncclUint8, peer, comm, st));
+  } else {
+    TB_NCCL(g_nccl.Recv(c.cig_off, (size_t)(n + 1) * 4, ncclUint8, peer, comm, st));
+    TB_NCCL(g_nccl.Recv(c.cigar, (size_t)words * 4, ncclUint8, peer, comm, st));
+  }
+  return 0;
 }
 
 // ---- ordered gather overlapped with the windows (tc_shard_coverage_gather) ------------------------------------------------
@@ -169,6 +195,40 @@ struct GatherState {
   int rounds = 0;
   int64_t bytes = 0;
 };
+
+// One ordered transfer of rows to rank 0, cr[r] / cj[r] from rank r (this rank's start at gs.sent_*). Rank 0 places them
+// by layout: `regions` puts rank r's at r * cap + got[r] (tc_shard_coverage_gather), otherwise they follow each other in rank
+// order (tc_shard_gather). Rank 0 copies its own rows (unless they are already in place) and receives the others'; every
+// other rank sends. Adds the bytes that crossed NCCL to gs.bytes and the rows to gs.got_* / gs.sent_*.
+static int gather_rows(tb_ctx* ctx, GatherState& gs, const tc_runs_out* runs, const tc_juncs_out* juncs, const std::vector<int64_t>& cr,
+                       const std::vector<int64_t>& cj, bool regions, cudaStream_t st) {
+  const int W = ctx->comm ? ctx->world : 1, R = ctx->comm ? ctx->rank : 0;
+  std::vector<int64_t> br(W), bj(W);   // first row of rank r on rank 0
+  for (int r = 0; r < W; ++r) {
+    br[r] = regions ? r * gs.cap_r + gs.got_r[r] : (r ? br[r - 1] + cr[r - 1] : 0);
+    bj[r] = regions ? r * gs.cap_j + gs.got_j[r] : (r ? bj[r - 1] + cj[r - 1] : 0);
+  }
+  if (R == 0) {
+    if (gs.all_runs && runs) TB_CUDA(tc_copy_rows(tc_at(*gs.all_runs, br[0]), tc_at(*runs, gs.sent_r), cr[0], cudaMemcpyDeviceToDevice, st));
+    if (gs.all_juncs && juncs) TB_CUDA(tc_copy_rows(tc_at(*gs.all_juncs, bj[0]), tc_at(*juncs, gs.sent_j), cj[0], cudaMemcpyDeviceToDevice, st));
+  }
+  if (W > 1) {
+    TB_NCCL(g_nccl.GroupStart());
+    for (int r = 1; r < W; ++r) {
+      if (R != 0 && r != R) continue;   // rank 0 receives from every rank, the others send their own rows
+      const tc_runs_out* rs = R ? runs : gs.all_runs;
+      const tc_juncs_out* js = R ? juncs : gs.all_juncs;
+      const int64_t ro = R ? gs.sent_r : br[r], jo = R ? gs.sent_j : bj[r];
+      if (rs && cr[r] > 0 && nccl_rows(ctx, tc_cols(tc_at(*rs, ro)), cr[r], R != 0, R ? 0 : r, st)) return 1;
+      if (js && cj[r] > 0 && nccl_rows(ctx, tc_cols(tc_at(*js, jo)), cj[r], R != 0, R ? 0 : r, st)) return 1;
+      gs.bytes += cr[r] * 20 + cj[r] * 21;
+    }
+    TB_NCCL(g_nccl.GroupEnd());
+  }
+  for (int r = 0; r < W; ++r) { gs.got_r[r] += cr[r]; gs.got_j[r] += cj[r]; }
+  gs.sent_r += cr[R]; gs.sent_j += cj[R];
+  return 0;
+}
 
 static int gather_round(tb_ctx* ctx, GatherState& gs, const tc_runs_out* runs, const tc_juncs_out* juncs, bool done) {
   const int W = ctx->comm ? ctx->world : 1, R = ctx->comm ? ctx->rank : 0;
@@ -200,54 +260,9 @@ static int gather_round(tb_ctx* ctx, GatherState& gs, const tc_runs_out* runs, c
       return 1;
     }
   }
-  auto d2d = [&](void* dst, const void* src, size_t bytes) { return (bytes && dst != src) ? cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, gst) : cudaSuccess; };
-  if (R == 0 && gs.all_runs && runs && new_r > 0) {
-    const int64_t o = gs.got_r[0];
-    TB_CUDA(d2d(gs.all_runs->tid + o, runs->tid + gs.sent_r, sizeof(int32_t) * new_r)); TB_CUDA(d2d(gs.all_runs->start0 + o, runs->start0 + gs.sent_r, sizeof(int32_t) * new_r));
-    TB_CUDA(d2d(gs.all_runs->end0 + o, runs->end0 + gs.sent_r, sizeof(int32_t) * new_r)); TB_CUDA(d2d(gs.all_runs->value + o, runs->value + gs.sent_r, sizeof(double) * new_r));
-  }
-  if (R == 0 && gs.all_juncs && juncs && new_j > 0) {
-    const int64_t o = gs.got_j[0];
-    TB_CUDA(d2d(gs.all_juncs->tid + o, juncs->tid + gs.sent_j, sizeof(int32_t) * new_j)); TB_CUDA(d2d(gs.all_juncs->start + o, juncs->start + gs.sent_j, sizeof(int32_t) * new_j));
-    TB_CUDA(d2d(gs.all_juncs->end + o, juncs->end + gs.sent_j, sizeof(int32_t) * new_j)); TB_CUDA(d2d(gs.all_juncs->strand + o, juncs->strand + gs.sent_j, (size_t)new_j));
-    TB_CUDA(d2d(gs.all_juncs->value + o, juncs->value + gs.sent_j, sizeof(double) * new_j));
-  }
-  if (W > 1) {
-    ncclComm_t comm = (ncclComm_t)ctx->comm;
-    TB_NCCL(g_nccl.GroupStart());
-    if (R == 0) {
-      for (int r = 1; r < W; ++r) {
-        const int64_t cr = (int64_t)h[4 * r], cj = (int64_t)h[4 * r + 1];
-        const int64_t ro = r * gs.cap_r + gs.got_r[r], jo = r * gs.cap_j + gs.got_j[r];
-        if (gs.all_runs && cr > 0) {
-          TB_NCCL(g_nccl.Recv(gs.all_runs->tid + ro, (size_t)cr * 4, ncclUint8, r, comm, gst)); TB_NCCL(g_nccl.Recv(gs.all_runs->start0 + ro, (size_t)cr * 4, ncclUint8, r, comm, gst));
-          TB_NCCL(g_nccl.Recv(gs.all_runs->end0 + ro, (size_t)cr * 4, ncclUint8, r, comm, gst)); TB_NCCL(g_nccl.Recv(gs.all_runs->value + ro, (size_t)cr * 8, ncclUint8, r, comm, gst));
-          gs.bytes += cr * 20;
-        }
-        if (gs.all_juncs && cj > 0) {
-          TB_NCCL(g_nccl.Recv(gs.all_juncs->tid + jo, (size_t)cj * 4, ncclUint8, r, comm, gst)); TB_NCCL(g_nccl.Recv(gs.all_juncs->start + jo, (size_t)cj * 4, ncclUint8, r, comm, gst));
-          TB_NCCL(g_nccl.Recv(gs.all_juncs->end + jo, (size_t)cj * 4, ncclUint8, r, comm, gst)); TB_NCCL(g_nccl.Recv(gs.all_juncs->strand + jo, (size_t)cj, ncclUint8, r, comm, gst));
-          TB_NCCL(g_nccl.Recv(gs.all_juncs->value + jo, (size_t)cj * 8, ncclUint8, r, comm, gst));
-          gs.bytes += cj * 21;
-        }
-      }
-    } else {
-      if (runs && new_r > 0) {
-        TB_NCCL(g_nccl.Send(runs->tid + gs.sent_r, (size_t)new_r * 4, ncclUint8, 0, comm, gst)); TB_NCCL(g_nccl.Send(runs->start0 + gs.sent_r, (size_t)new_r * 4, ncclUint8, 0, comm, gst));
-        TB_NCCL(g_nccl.Send(runs->end0 + gs.sent_r, (size_t)new_r * 4, ncclUint8, 0, comm, gst)); TB_NCCL(g_nccl.Send(runs->value + gs.sent_r, (size_t)new_r * 8, ncclUint8, 0, comm, gst));
-        gs.bytes += new_r * 20;
-      }
-      if (juncs && new_j > 0) {
-        TB_NCCL(g_nccl.Send(juncs->tid + gs.sent_j, (size_t)new_j * 4, ncclUint8, 0, comm, gst)); TB_NCCL(g_nccl.Send(juncs->start + gs.sent_j, (size_t)new_j * 4, ncclUint8, 0, comm, gst));
-        TB_NCCL(g_nccl.Send(juncs->end + gs.sent_j, (size_t)new_j * 4, ncclUint8, 0, comm, gst)); TB_NCCL(g_nccl.Send(juncs->strand + gs.sent_j, (size_t)new_j, ncclUint8, 0, comm, gst));
-        TB_NCCL(g_nccl.Send(juncs->value + gs.sent_j, (size_t)new_j * 8, ncclUint8, 0, comm, gst));
-        gs.bytes += new_j * 21;
-      }
-    }
-    TB_NCCL(g_nccl.GroupEnd());
-  }
-  for (int r = 0; r < W; ++r) { gs.got_r[r] += (int64_t)h[4 * r]; gs.got_j[r] += (int64_t)h[4 * r + 1]; }
-  gs.sent_r += new_r; gs.sent_j += new_j;
+  std::vector<int64_t> cr(W), cj(W);
+  for (int r = 0; r < W; ++r) { cr[r] = (int64_t)h[4 * r]; cj[r] = (int64_t)h[4 * r + 1]; }
+  if (gather_rows(ctx, gs, runs, juncs, cr, cj, true, gst)) return 1;
   gs.all_done = all;
   gs.rounds++;
   return 0;
@@ -288,18 +303,12 @@ int tc_stream_impl(tb_ctx* ctx, const tc_soa_in* in, int64_t skip, int64_t windo
       }
       if (w1 < n) { ext.has_next = 1; ext.next_tid = nx[0]; ext.next_pos = nx[1]; }
       else if (next) { ext.has_next = 1; ext.next_tid = next[0]; ext.next_pos = next[1]; }
-      tc_soa_in sub = sub_window(*in, w0, wlen, (int64_t)(c01[1] - c01[0]));
-      tc_runs_out r; tc_juncs_out j;
-      if (runs) {
-        r = *runs; r.capacity = runs->capacity - runs->n_runs; r.n_runs = 0;
-        r.tid = runs->tid + runs->n_runs; r.start0 = runs->start0 + runs->n_runs; r.end0 = runs->end0 + runs->n_runs; r.value = runs->value + runs->n_runs;
-      }
-      if (juncs) {
-        j = *juncs; j.capacity = juncs->capacity - juncs->n_juncs; j.n_juncs = 0;
-        j.tid = juncs->tid + juncs->n_juncs; j.start = juncs->start + juncs->n_juncs; j.end = juncs->end + juncs->n_juncs;
-        j.strand = juncs->strand + juncs->n_juncs; j.value = juncs->value + juncs->n_juncs;
-      }
-      const int rc = tc_coverage_impl(ctx, &sub, runs ? &r : nullptr, juncs ? &j : nullptr, yx ? yx + w0 : nullptr, &ext);
+      const TcRecords wc = tc_at(tc_records(*in, yx), w0);
+      const tc_soa_in sub = tc_window(wc, wlen, (int64_t)(c01[1] - c01[0]), in->on_device);
+      tc_runs_out r; tc_juncs_out j;   // the rows after those already in runs / juncs
+      if (runs) { r = tc_at(*runs, runs->n_runs); r.capacity -= runs->n_runs; r.n_runs = 0; }
+      if (juncs) { j = tc_at(*juncs, juncs->n_juncs); j.capacity -= juncs->n_juncs; j.n_juncs = 0; }
+      const int rc = tc_coverage_impl(ctx, &sub, runs ? &r : nullptr, juncs ? &j : nullptr, wc.yx, &ext);
       if (rc == 3) {   // one bundle spans the window
         if (w1 >= n) { *consumed = w0; goto done; }   // ... and the slice: the caller joins it with what follows
         wlen = std::min(wlen * 2, n - w0);
@@ -320,6 +329,13 @@ int tc_stream_impl(tb_ctx* ctx, const tc_soa_in* in, int64_t skip, int64_t windo
 done:
   ctx->last_ms[6] = ms_acc[0]; ctx->last_ms[1] = ms_acc[1]; ctx->last_ms[7] = ms_acc[2];   // sums over the windows of this call
   return 0;
+}
+
+void tc_copy_records(tb_ctx* ctx, cudaStream_t st, const TcRecords& src, int64_t from, int64_t m, const TcRecords& dst, int64_t r, uint32_t w,
+                     uint32_t words) {
+  const int64_t work = std::max<int64_t>(m + 1, words);
+  tc_copy_records_kernel<<<(unsigned)std::min<int64_t>((work + 255) / 256, 4096), 256, 0, st>>>(src, from, m, dst, r, w, words);
+  ctx->launches++;
 }
 
 extern "C" {
@@ -377,24 +393,11 @@ static int shard_coverage_impl(tb_ctx* ctx, const tc_soa_in* segs, int n_segs, i
   tc_soa_in dseg;
   if (!segs[0].on_device) {
     if (n_segs != 1) { ctx->set_error("tc_shard_coverage: host arrays are accepted as ONE segment; several segments must be device resident"); return 1; }
-    const tc_soa_in& h = segs[0];
+    tc_soa_in h = segs[0];
     dseg = h; dseg.on_device = 1;
-    if (h.n > 0) {
-      const uint32_t c0 = h.cig_off[0], c1 = h.cig_off[h.n];
-      DevBuf* IS = ctx->in_stage;
-      auto up = [&](DevBuf& b, const void* src, size_t bytes, const void** out) -> cudaError_t {
-        cudaError_t e = b.ensure(bytes + 16); if (e != cudaSuccess) return e;
-        e = cudaMemcpyAsync(b.p, src, bytes, cudaMemcpyHostToDevice, st); *out = b.p; return e;
-      };
-      const void* q;
-      TB_CUDA(up(IS[8], h.tid, sizeof(int32_t) * h.n, &q)); dseg.tid = (const int32_t*)q;
-      TB_CUDA(up(IS[9], h.pos, sizeof(int32_t) * h.n, &q)); dseg.pos = (const int32_t*)q;
-      TB_CUDA(up(IS[10], h.yc, sizeof(float) * h.n, &q)); dseg.yc = (const float*)q;
-      TB_CUDA(up(IS[11], h.strand, (size_t)h.n, &q)); dseg.strand = (const uint8_t*)q;
-      TB_CUDA(up(IS[12], h.cig_off, sizeof(uint32_t) * (h.n + 1), &q)); dseg.cig_off = (const uint32_t*)q;
-      TB_CUDA(up(IS[13], h.cigar + c0, sizeof(uint32_t) * (size_t)(c1 - c0), &q)); dseg.cigar = (const uint32_t*)q - c0;   // offsets stay absolute
-      if (h.end) { TB_CUDA(up(IS[14], h.end, sizeof(int32_t) * h.n, &q)); dseg.end = (const int32_t*)q; }
-      dseg.n_cig = (int64_t)(c1 - c0);
+    if (h.n > 0) {   // staged in in_stage[8..16): tc_coverage_impl stages its windows in [0, 8)
+      h.n_cig = (int64_t)(h.cig_off[h.n] - h.cig_off[0]);
+      if (tc_stage_window(ctx, ctx->in_stage + 8, h, nullptr, &dseg, nullptr)) return 1;
       TB_CUDA(cudaStreamSynchronize(st));
     }
     segs = &dseg;
@@ -410,6 +413,7 @@ static int shard_coverage_impl(tb_ctx* ctx, const tc_soa_in* segs, int n_segs, i
   int64_t n_local = 0;
   for (int s = 0; s < n_segs; ++s) n_local += segs[s].n;
   int64_t lead = 0, tail_n = 0, tail_words = 0;
+  TcRecords tail{};   // the leads received from the ranks on the right, in rank order
   int32_t tail_next[2] = {0, 0};
   DevBuf* SB = ctx->shard_buf;
   cudaEvent_t e0 = ctx->ev[12], e1 = ctx->ev[13];
@@ -498,45 +502,39 @@ static int shard_coverage_impl(tb_ctx* ctx, const tc_soa_in* segs, int n_segs, i
     if (!from.empty()) { const unsigned long long fk = firstkey[from[0]]; tail_next[0] = (int32_t)(fk >> 32); tail_next[1] = (int32_t)(uint32_t)fk; }
     if (tail_words >= (1LL << 32) || tail_n >= (1LL << 31)) { ctx->set_error("tc_shard_coverage: %lld lead records do not fit one window", (long long)tail_n); return 1; }
     if (tail_n > 0) {
-      TB_CUDA(SB[SB_TAIL_TID].ensure(sizeof(int32_t) * tail_n)); TB_CUDA(SB[SB_TAIL_POS].ensure(sizeof(int32_t) * tail_n));
-      TB_CUDA(SB[SB_TAIL_YC].ensure(sizeof(float) * tail_n)); TB_CUDA(SB[SB_TAIL_STRAND].ensure((size_t)tail_n));
-      TB_CUDA(SB[SB_TAIL_OFF].ensure(sizeof(uint32_t) * (tail_n + 1))); TB_CUDA(SB[SB_SEND].ensure(sizeof(uint32_t) * (tail_n + from.size() + 1)));
-      TB_CUDA(SB[SB_TAIL_CIG].ensure(sizeof(uint32_t) * (tail_words + 4)));
+      TB_CUDA(tc_alloc_records(SB + SB_TAIL, tail_n, tail_words + 4, false, &tail));
+      TB_CUDA(SB[SB_SEND].ensure(sizeof(uint32_t) * (tail_n + from.size() + 1)));
     }
-    // ---- 4. the halo exchange proper: one grouped send / receive of the lead records' columns ----
+    // ---- 4. the halo exchange proper: one grouped send / receive of the lead records' columns. No `end` column: the
+    // seam window that takes the leads is processed from the CIGARs ----
     TB_NCCL(g_nccl.GroupStart());
     if (lead > 0) {
-      TB_NCCL(g_nccl.Send(first.tid, (size_t)lead * 4, ncclUint8, owner, comm, st));
-      TB_NCCL(g_nccl.Send(first.pos, (size_t)lead * 4, ncclUint8, owner, comm, st));
-      TB_NCCL(g_nccl.Send(first.yc, (size_t)lead * 4, ncclUint8, owner, comm, st));
-      TB_NCCL(g_nccl.Send(first.strand, (size_t)lead, ncclUint8, owner, comm, st));
-      TB_NCCL(g_nccl.Send(first.cig_off, (size_t)(lead + 1) * 4, ncclUint8, owner, comm, st));
-      TB_NCCL(g_nccl.Send(first.cigar + lead_c[0], (size_t)(lead_c[1] - lead_c[0]) * 4, ncclUint8, owner, comm, st));
+      TcRecords lr = tc_records(first);
+      lr.end = nullptr;
+      lr.cigar += lead_c[0];
+      if (nccl_records(ctx, lr, lead, lead_c[1] - lead_c[0], true, owner, st)) return 1;
       ctx->shard_stat[1] = lead; ctx->shard_stat[3] = (int64_t)lead * 17 + 4 + (int64_t)(lead_c[1] - lead_c[0]) * 4;
     }
     {
       int64_t ro = 0, wo = 0; size_t piece = 0;
       for (int r : from) {
-        TB_NCCL(g_nccl.Recv(SB[SB_TAIL_TID].as<int32_t>() + ro, (size_t)leads[r] * 4, ncclUint8, r, comm, st));
-        TB_NCCL(g_nccl.Recv(SB[SB_TAIL_POS].as<int32_t>() + ro, (size_t)leads[r] * 4, ncclUint8, r, comm, st));
-        TB_NCCL(g_nccl.Recv(SB[SB_TAIL_YC].as<float>() + ro, (size_t)leads[r] * 4, ncclUint8, r, comm, st));
-        TB_NCCL(g_nccl.Recv(SB[SB_TAIL_STRAND].as<uint8_t>() + ro, (size_t)leads[r], ncclUint8, r, comm, st));
         // the leads + 1 offsets of piece p land in a scratch area at [ro + p, ...) and are rebased into the tail below
-        TB_NCCL(g_nccl.Recv(SB[SB_SEND].as<uint32_t>() + ro + piece, (size_t)(leads[r] + 1) * 4, ncclUint8, r, comm, st));
-        TB_NCCL(g_nccl.Recv(SB[SB_TAIL_CIG].as<uint32_t>() + wo, (size_t)lwords[r] * 4, ncclUint8, r, comm, st));
+        TcRecords dst = tc_at(tail, ro);
+        dst.cig_off = SB[SB_SEND].as<uint32_t>() + ro + piece;
+        dst.cigar = tail.cigar + wo;
+        if (nccl_records(ctx, dst, leads[r], lwords[r], false, r, st)) return 1;
         ro += leads[r]; wo += lwords[r]; ++piece;
       }
     }
     TB_NCCL(g_nccl.GroupEnd());
     ctx->shard_stat[0] = tail_n; ctx->shard_stat[2] = (int64_t)from.size();
     // ---- 5. received offsets -> offsets into the tail arena, piece by piece ----
-    if (tail_n > 0) {
-      int64_t ro = 0, wo = 0; size_t piece = 0;
-      for (int r : from) {
-        shard_copy_off_kernel<<<grid_for(leads[r] + 1, 256), 256, 0, st>>>(SB[SB_SEND].as<uint32_t>() + ro + piece, leads[r] + 1, (uint32_t)wo, SB[SB_TAIL_OFF].as<uint32_t>() + ro);
-        ctx->launches++;
-        ro += leads[r]; wo += lwords[r]; ++piece;
-      }
+    int64_t ro = 0, wo = 0; size_t piece = 0;
+    for (int r : from) {
+      TcRecords src{};
+      src.cig_off = SB[SB_SEND].as<uint32_t>() + ro + piece;
+      tc_copy_records(ctx, st, src, 0, leads[r], tail, ro, (uint32_t)wo, 0);
+      ro += leads[r]; wo += lwords[r]; ++piece;
     }
   }
   if (ctx->profiling) TB_CUDA(cudaEventRecord(e1, st));
@@ -570,26 +568,11 @@ static int shard_coverage_impl(tb_ctx* ctx, const tc_soa_in* segs, int n_segs, i
       TB_CUDA(cudaStreamSynchronize(st));
     }
     const int64_t ow = (int64_t)(oc[1] - oc[0]), sw = ow + tail_words;
-    TB_CUDA(SB[SB_SEAM_TID].ensure(sizeof(int32_t) * sn)); TB_CUDA(SB[SB_SEAM_POS].ensure(sizeof(int32_t) * sn)); TB_CUDA(SB[SB_SEAM_YC].ensure(sizeof(float) * sn));
-    TB_CUDA(SB[SB_SEAM_STRAND].ensure((size_t)sn)); TB_CUDA(SB[SB_SEAM_OFF].ensure(sizeof(uint32_t) * (sn + 1))); TB_CUDA(SB[SB_SEAM_CIG].ensure(sizeof(uint32_t) * (sw + 4)));
-    auto d2d = [&](void* dst, const void* src, size_t bytes) { return bytes ? cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, st) : cudaSuccess; };
-    TB_CUDA(d2d(SB[SB_SEAM_TID].p, last.tid + consumed_last, sizeof(int32_t) * open_n));
-    TB_CUDA(d2d(SB[SB_SEAM_POS].p, last.pos + consumed_last, sizeof(int32_t) * open_n));
-    TB_CUDA(d2d(SB[SB_SEAM_YC].p, last.yc + consumed_last, sizeof(float) * open_n));
-    TB_CUDA(d2d(SB[SB_SEAM_STRAND].p, last.strand + consumed_last, (size_t)open_n));
-    TB_CUDA(d2d(SB[SB_SEAM_CIG].p, last.cigar + oc[0], sizeof(uint32_t) * ow));
-    TB_CUDA(d2d(SB[SB_SEAM_TID].as<int32_t>() + open_n, SB[SB_TAIL_TID].p, sizeof(int32_t) * tail_n));
-    TB_CUDA(d2d(SB[SB_SEAM_POS].as<int32_t>() + open_n, SB[SB_TAIL_POS].p, sizeof(int32_t) * tail_n));
-    TB_CUDA(d2d(SB[SB_SEAM_YC].as<float>() + open_n, SB[SB_TAIL_YC].p, sizeof(float) * tail_n));
-    TB_CUDA(d2d(SB[SB_SEAM_STRAND].as<uint8_t>() + open_n, SB[SB_TAIL_STRAND].p, (size_t)tail_n));
-    TB_CUDA(d2d(SB[SB_SEAM_CIG].as<uint32_t>() + ow, SB[SB_TAIL_CIG].p, sizeof(uint32_t) * tail_words));
-    if (open_n > 0) { shard_copy_off_kernel<<<grid_for(open_n, 256), 256, 0, st>>>(last.cig_off + consumed_last, open_n, 0u, SB[SB_SEAM_OFF].as<uint32_t>()); ctx->launches++; }
-    shard_copy_off_kernel<<<grid_for(tail_n + 1, 256), 256, 0, st>>>(SB[SB_TAIL_OFF].as<uint32_t>(), tail_n + 1, (uint32_t)ow, SB[SB_SEAM_OFF].as<uint32_t>() + open_n);
-    ctx->launches++;
-    tc_soa_in seam; memset(&seam, 0, sizeof(seam));
-    seam.n = sn; seam.tid = SB[SB_SEAM_TID].as<int32_t>(); seam.pos = SB[SB_SEAM_POS].as<int32_t>(); seam.yc = SB[SB_SEAM_YC].as<float>();
-    seam.strand = SB[SB_SEAM_STRAND].as<uint8_t>(); seam.cig_off = SB[SB_SEAM_OFF].as<uint32_t>(); seam.cigar = SB[SB_SEAM_CIG].as<uint32_t>();
-    seam.on_device = 1; seam.n_cig = sw;
+    TcRecords sc;   // like the tail, without `end`
+    TB_CUDA(tc_alloc_records(SB + SB_SEAM, sn, sw + 4, false, &sc));
+    if (open_n > 0) tc_copy_records(ctx, st, tc_records(last), consumed_last, open_n, sc, 0, 0, (uint32_t)ow);
+    tc_copy_records(ctx, st, tail, 0, tail_n, sc, open_n, (uint32_t)ow, (uint32_t)tail_words);
+    const tc_soa_in seam = tc_window(sc, sn, sw);
     int64_t consumed = 0;
     const int rc = tc_stream_impl(ctx, &seam, 0, std::max<int64_t>(window, sn), nullptr, runs, juncs, &consumed, cb);
     if (rc) return rc;
@@ -682,48 +665,11 @@ int tc_shard_gather(tb_ctx* ctx, const tc_runs_out* runs, const tc_juncs_out* ju
     if (all_runs) { if (all_runs->capacity < tr) { ctx->set_error("tc_shard_gather: runs capacity %lld < %lld", (long long)all_runs->capacity, (long long)tr); return 1; } all_runs->n_runs = tr; }
     if (all_juncs) { if (all_juncs->capacity < tj) { ctx->set_error("tc_shard_gather: junction capacity %lld < %lld", (long long)all_juncs->capacity, (long long)tj); return 1; } all_juncs->n_juncs = tj; }
   }
-  auto d2d = [&](void* dst, const void* src, size_t bytes) { return (bytes && dst != src) ? cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, st) : cudaSuccess; };
-  if (R == 0) {
-    if (all_runs && runs) {
-      TB_CUDA(d2d(all_runs->tid, runs->tid, sizeof(int32_t) * nr)); TB_CUDA(d2d(all_runs->start0, runs->start0, sizeof(int32_t) * nr));
-      TB_CUDA(d2d(all_runs->end0, runs->end0, sizeof(int32_t) * nr)); TB_CUDA(d2d(all_runs->value, runs->value, sizeof(double) * nr));
-    }
-    if (all_juncs && juncs) {
-      TB_CUDA(d2d(all_juncs->tid, juncs->tid, sizeof(int32_t) * nj)); TB_CUDA(d2d(all_juncs->start, juncs->start, sizeof(int32_t) * nj));
-      TB_CUDA(d2d(all_juncs->end, juncs->end, sizeof(int32_t) * nj)); TB_CUDA(d2d(all_juncs->strand, juncs->strand, (size_t)nj));
-      TB_CUDA(d2d(all_juncs->value, juncs->value, sizeof(double) * nj));
-    }
-  }
-  if (W > 1) {
-    TB_NCCL(g_nccl.GroupStart());
-    if (R == 0) {
-      int64_t ro = cr[0], jo = cj[0];
-      for (int r = 1; r < W; ++r) {
-        if (all_runs && cr[r] > 0) {
-          TB_NCCL(g_nccl.Recv(all_runs->tid + ro, (size_t)cr[r] * 4, ncclUint8, r, comm, st)); TB_NCCL(g_nccl.Recv(all_runs->start0 + ro, (size_t)cr[r] * 4, ncclUint8, r, comm, st));
-          TB_NCCL(g_nccl.Recv(all_runs->end0 + ro, (size_t)cr[r] * 4, ncclUint8, r, comm, st)); TB_NCCL(g_nccl.Recv(all_runs->value + ro, (size_t)cr[r] * 8, ncclUint8, r, comm, st));
-        }
-        if (all_juncs && cj[r] > 0) {
-          TB_NCCL(g_nccl.Recv(all_juncs->tid + jo, (size_t)cj[r] * 4, ncclUint8, r, comm, st)); TB_NCCL(g_nccl.Recv(all_juncs->start + jo, (size_t)cj[r] * 4, ncclUint8, r, comm, st));
-          TB_NCCL(g_nccl.Recv(all_juncs->end + jo, (size_t)cj[r] * 4, ncclUint8, r, comm, st)); TB_NCCL(g_nccl.Recv(all_juncs->strand + jo, (size_t)cj[r], ncclUint8, r, comm, st));
-          TB_NCCL(g_nccl.Recv(all_juncs->value + jo, (size_t)cj[r] * 8, ncclUint8, r, comm, st));
-        }
-        ro += cr[r]; jo += cj[r];
-      }
-    } else {
-      if (runs && nr > 0) {
-        TB_NCCL(g_nccl.Send(runs->tid, (size_t)nr * 4, ncclUint8, 0, comm, st)); TB_NCCL(g_nccl.Send(runs->start0, (size_t)nr * 4, ncclUint8, 0, comm, st));
-        TB_NCCL(g_nccl.Send(runs->end0, (size_t)nr * 4, ncclUint8, 0, comm, st)); TB_NCCL(g_nccl.Send(runs->value, (size_t)nr * 8, ncclUint8, 0, comm, st));
-      }
-      if (juncs && nj > 0) {
-        TB_NCCL(g_nccl.Send(juncs->tid, (size_t)nj * 4, ncclUint8, 0, comm, st)); TB_NCCL(g_nccl.Send(juncs->start, (size_t)nj * 4, ncclUint8, 0, comm, st));
-        TB_NCCL(g_nccl.Send(juncs->end, (size_t)nj * 4, ncclUint8, 0, comm, st)); TB_NCCL(g_nccl.Send(juncs->strand, (size_t)nj, ncclUint8, 0, comm, st));
-        TB_NCCL(g_nccl.Send(juncs->value, (size_t)nj * 8, ncclUint8, 0, comm, st));
-      }
-    }
-    TB_NCCL(g_nccl.GroupEnd());
-    ctx->shard_stat[5] = R == 0 ? (tr - cr[0]) * 20 + (tj - cj[0]) * 21 : nr * 20 + nj * 21;   // bytes over NVLink in the gather
-  }
+  GatherState gs;
+  gs.all_runs = all_runs; gs.all_juncs = all_juncs;
+  gs.got_r.assign(W, 0); gs.got_j.assign(W, 0);
+  if (gather_rows(ctx, gs, runs, juncs, cr, cj, false, st)) return 1;
+  if (W > 1) ctx->shard_stat[5] = gs.bytes;   // bytes over NVLink in the gather
   TB_CUDA(cudaStreamSynchronize(st));
   return 0;
 }

@@ -82,12 +82,12 @@ struct tb_ctx {
   std::string err;
   DevBuf buf[TB_NBUF];   // workspace slots (see the enum in each pipeline)
   DevBuf in_stage[20];   // device copies of host input arrays
-  DevBuf out_stage[8];   // device output arrays when the caller wants host results
+  DevBuf out_stage[9];   // device output arrays when the caller wants host results: runs in 0..3, junction rows in 4..8
   HostBuf pinned[2];     // small pinned readback areas
   // multi-GPU (shard.cu): NCCL communicator of this context's rank, workspace, statistics of the last sharded call
   void* comm = nullptr; int rank = 0; int world = 1;
   cudaStream_t gather_stream = nullptr;   // second stream: ordered gather overlapped with the windows
-  DevBuf shard_buf[16];
+  DevBuf shard_buf[19];
   int64_t shard_stat[8] = {};   // lead records received | sent | ranks received from | bytes sent (halo) | seam records | bytes moved by the gather
   int64_t stream_windows = 0;   // windows of the last tc_coverage_stream / tc_shard_coverage call
   // BAM decode (bgzf.cu): workspace, and the bundle tc_coverage_bam holds for its next call: records [bam_from, bam_from +
@@ -101,6 +101,18 @@ struct tb_ctx {
 };
 
 extern std::string g_tb_global_error;
+
+static inline unsigned tb_grid_for(int64_t n, int threads) { return (unsigned)((n + threads - 1) / threads); }
+
+// a host input array on the device (device arrays and NULL pass through)
+template <class T>
+static int tb_stage_in(tb_ctx* ctx, DevBuf& b, const T* src, size_t count, int on_device, const T** out) {
+  if (on_device || src == nullptr) { *out = src; return 0; }
+  TB_CUDA(b.ensure(count * sizeof(T) + 16));
+  TB_CUDA(cudaMemcpyAsync(b.p, src, count * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));
+  *out = (const T*)b.p;
+  return 0;
+}
 
 // tc_coverage_stream's view of one window (coverage.cu): the record that follows the window in the stream, and how many
 // records of the window were processed (all but the last bundle when that record continues it)

@@ -213,14 +213,3 @@ static_assert(XB_COUNT_ <= TB_NBUF, "raise TB_NBUF");
 enum { CS_ERR = 0, CS_ERRIDX, CS_NKEPT, CS_NGROUPS, CS_TABLE_OVERFLOW, CS_NBUNDLES, CS_YD_OVERFLOW, CS_NHEAVY, CS_N_ };   // 8-10: YD (YS_*)
 enum { CS_TILE_RECORDS = 11, CS_TILE_HEADS, CS_TILE_BATCHES };   // tile kernel statistics of the collapse call
 enum { ERR_POS_RANGE = 1, ERR_UNSORTED = 2 };
-
-static inline unsigned tb_grid_for(int64_t n, int threads) { return (unsigned)((n + threads - 1) / threads); }
-
-template <class T>
-static int tb_stage_in(tb_ctx* ctx, DevBuf& b, const T* src, size_t count, int on_device, const T** out) {
-  if (on_device || src == nullptr) { *out = src; return 0; }
-  TB_CUDA(b.ensure(count * sizeof(T) + 16));
-  TB_CUDA(cudaMemcpyAsync(b.p, src, count * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));
-  *out = (const T*)b.p;
-  return 0;
-}
